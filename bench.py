@@ -1,12 +1,16 @@
 """Benchmark of the north-star metric: batched RRT* plans/s (512x512 worlds, n=5000, r_rewire=50).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--plans P] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--plans P] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch: P independent RRT* plans per GPU (world w
 seeded 1000+w, one start/goal pair per world, sample stream of plan p = default_rng(p)), i.e. the
 sampler kernel + the persistent plan kernel.  N > 1 is launched by torchrun, one rank per GPU;
 plans are independent so every rank runs its own P plans (the headline: weak scaling, no data-path
-collective; only per-plan statistics are gathered at the end of each step).
+collective; only per-plan statistics are gathered at the end of each step).  Every timed loop that averages over repeated
+launches or calls, in every leg below, runs exactly K of them.
+
+`--dump-outputs DIR` writes what the last timed step of the headline computed (dump_outputs): the inputs are fixed by the
+seeds above, so two builds run with the same arguments can be compared output for output.
 
 The JSON line carries, besides the contract keys:
   roofline             plan kernel: algorithmic bytes / CUDA-event time against the shared-memory read bandwidth MEASURED in the
@@ -233,7 +237,7 @@ def collision_microbench(local: int, steps: int, warmup: int, cpu: bool, sm_mhz:
         launch()
     torch.cuda.synchronize(dev)
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    reps = max(steps, 10)
+    reps = steps
     e0.record(stream)
     for _ in range(reps):
         launch()
@@ -459,7 +463,7 @@ def informed_bench(local: int, steps: int, cpu: bool, peaks: dict, plans: int = 
     for _ in range(2):
         db.run()
     torch.cuda.synchronize(dev)
-    reps = max(2, min(steps, 4))
+    reps = steps
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record(stream)
     for _ in range(reps):
@@ -521,15 +525,15 @@ def informed_bench(local: int, steps: int, cpu: bool, peaks: dict, plans: int = 
 # ------------------------------------------------------------------------------------------------
 # cfg1: one RRTStar plan through the drop-in class (BASELINE.json configs[0], the reference's own CPU-runnable case)
 # ------------------------------------------------------------------------------------------------
-def class_api_bench(cpu: bool):
-    """RRTStar(og, n=1000, r_rewire=50, seed=0).plan() on a 256x256 world, timed around the public call including the
-    networkx graph it returns -- the latency a user of the reference's API sees (the reference: about 0.6 s, SURVEY.md 6)."""
+def class_api_bench(steps: int, cpu: bool):
+    """RRTStar(og, n=1000, r_rewire=50, seed=0).plan() on a 256x256 world, `steps` calls timed around the public call including
+    the networkx graph it returns -- the latency a user of the reference's API sees (the reference: about 0.6 s, SURVEY.md 6)."""
     from rrtplanner_b200 import rrt, worlds
     og = worlds.perlin_occupancygrid(256, 256, seed=worlds.world_seed(0))
     xs, xg = worlds.start_goal(og, 0)
     pl = rrt.RRTStar(og, 1000, 50.0, pbar=False, seed=0)
     pl.plan(xs, xg)
-    reps = 5
+    reps = steps
     t0 = time.perf_counter()
     for _ in range(reps):
         pl = rrt.RRTStar(og, 1000, 50.0, pbar=False, seed=0)
@@ -601,7 +605,7 @@ def dubins_bench(local: int, steps: int, cpu: bool, plans: int = DUB_PLANS, thre
             db.run()
         torch.cuda.synchronize(dev)
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        reps = max(2, min(steps, 5))
+        reps = steps
         e0.record(stream)
         for _ in range(reps):
             db.run()
@@ -797,6 +801,44 @@ def strong_leg(local: int, rank: int, world: int, steps: int, warmup: int, barri
 
 
 # ------------------------------------------------------------------------------------------------
+# --dump-outputs: what the last timed step computed, for comparing two builds output for output
+# ------------------------------------------------------------------------------------------------
+DUMP_PLANS = 256          # trees of 256 plans at n = 5000: 25.6 MB
+# statistics that are results of a plan; checks / cells depend on how the warps of a block interleave in the goal search and
+# nn_pairs on which form of the plan kernel answers the nearest query, so they are left out
+DUMP_STATS = ("j", "vgoal", "found", "first_solution_iter", "ellipse_iters", "accepted", "ring_members")
+
+
+def dump_outputs(out_dir: str, out: dict):
+    """Write the trees of a fixed sample of plans (default_rng(0), at most DUMP_PLANS, ascending plan index) and the result
+    statistics of every plan as DIR/<name>.npy: plan_index, pts (float32), cost (float64), parent (float32; ids < 2**24),
+    stat_<name> (float64).  Every value written is finite: the unfilled rows of a tree (row >= j + found) keep the fill values
+    of pts (-32768) and parent (-1), and their cost, inf in the library's layout, is written as -1 (a real cost is >= 0)."""
+    import torch
+
+    from rrtplanner_b200 import _lib
+    P = out["stats"].shape[0]
+    sel = np.sort(np.random.default_rng(0).choice(P, size=min(P, DUMP_PLANS), replace=False))
+    idx = torch.from_numpy(sel).to(out["pts"].device)
+    stats = out["stats"].cpu().numpy()
+    cost = out["cost"].index_select(0, idx).cpu().numpy()
+    top = stats[sel, _lib.STAT_NAMES.index("j")] + (stats[sel, _lib.STAT_NAMES.index("found")] != 0)
+    cost[np.arange(cost.shape[1])[None, :] >= top[:, None]] = -1.0
+    arrays = {"plan_index": sel.astype(np.float64),
+              "pts": out["pts"].index_select(0, idx).cpu().numpy().astype(np.float32),
+              "cost": cost,
+              "parent": out["parent"].index_select(0, idx).cpu().numpy().astype(np.float32)}
+    for name in DUMP_STATS:
+        arrays["stat_" + name] = stats[:, _lib.STAT_NAMES.index(name)].astype(np.float64)
+    for name, a in arrays.items():
+        if not np.isfinite(a).all():
+            raise RuntimeError(f"--dump-outputs: {name} of the last timed step holds a non-finite value")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+# ------------------------------------------------------------------------------------------------
 # GPU arm
 # ------------------------------------------------------------------------------------------------
 def gpu_arm(args):
@@ -874,6 +916,8 @@ def gpu_arm(args):
     ms_total = float(t.item())
 
     stats = db.out["stats"].cpu().numpy()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, db.out)
     S = {n: stats[:, i] for i, n in enumerate(_lib.STAT_NAMES)}
     if world > 1 and rank == 0:
         all_stats = torch.stack(gathered).cpu().numpy().reshape(-1, _lib.STAT_COUNT)
@@ -995,7 +1039,7 @@ def gpu_arm(args):
         ctx.close()
 
     # ---- strong scaling: the same 4096 plans in total whatever N, with the final gather of the paths ----
-    strong = None if args.no_strong else strong_leg(local, rank, world, max(2, min(args.steps, 10)), args.warmup, barrier)
+    strong = None if args.no_strong else strong_leg(local, rank, world, args.steps, args.warmup, barrier)
 
     # cfg5 on every rank (weak scaling like the headline; K8 plans shard by index exactly like K7's)
     dub_multi = dubins_bench(local, args.steps, False, rank=rank, world=world) if (world > 1 and not args.no_dubins) else None
@@ -1081,7 +1125,7 @@ def gpu_arm(args):
     if world == 1 and not args.no_informed:
         line["informed_bench"] = informed_bench(local, args.steps, not args.no_cpu, measured)
     if world == 1 and not args.no_class_api:
-        line["class_api_bench"] = class_api_bench(not args.no_cpu)
+        line["class_api_bench"] = class_api_bench(args.steps, not args.no_cpu)
     if world == 1 and not args.no_dubins:
         line["dubins_bench"] = dubins_bench(local, args.steps, not args.no_cpu)
     if dub_multi is not None:
@@ -1114,7 +1158,14 @@ def main():
     ap.add_argument("--informed-only", action="store_true", help="run only the cfg4 RRTStarInformed leg (profiling aid)")
     ap.add_argument("--dubins-plans", type=int, default=DUB_PLANS)
     ap.add_argument("--plan-only", action="store_true", help="device arm of the headline only (experiments): implies every --no-* flag")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps of the headline, write the trees of its last step (a fixed sample of plans) and the "
+                         "result statistics of every plan as DIR/<name>.npy (rank 0's plans)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "native" or args.collision_only or args.informed_only or args.dubins_only):
+        ap.error("--dump-outputs writes the outputs of the native headline; it does not combine with --impl reference or --*-only")
     if args.plan_only:
         args.no_e2e = args.no_cpu = args.no_strong = args.no_collision = args.no_dubins = args.no_informed = args.no_class_api = True
     if args.warmup < 3 and args.impl == "native":
