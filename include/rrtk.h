@@ -209,6 +209,24 @@ int rrtk_sample_streams_carry(const uint32_t *d_bits, const int32_t *d_rowcum, i
                               const rrtk_plan_desc *d_plans, int nplans, uint64_t *d_state, uint32_t *d_carry,
                               int n, int16_t *d_samples, void *stream);
 
+/* The unit-disc stream of the ellipse phase of RRTStarInformed.plan (rrt.py:240, 579-587, 694-701), from the same
+ * generator: the reference draws free[choice(nfree)] in iterations 0 .. f (f = the first solution iteration) and then
+ * unitball() = two uniform(0, 1) draws per iteration.  Per plan p (world d_plans[p].world, nfree = d_rowcum[world*(W+1)+W]):
+ *   d_state    PCG64 start state as for rrtk_sample_streams; d_carry (optional, NULL = zero) has_uint32 / uinteger
+ *   d_first    f = d_first[p * first_stride] (int64; -1 = no solution): the probe's statistics work directly, e.g. K7 stats
+ *              + RRTK_STAT_FIRST_SOL_ITER or K8 stats + RRTK_STAT2_FIRST_SOL with stride RRTK_STAT_COUNT
+ *   d_balls    nplans x n x 2 doubles: row i > f = (sqrt(u1) cos(2 pi u2), sqrt(u1) sin(2 pi u2)) of the i-th iteration's two
+ *              uniforms after the min(f + 1, n) bounded draws; rows <= f and every row when f < 0 are 0.0.  The uniforms,
+ *              sqrt and products are bit-exact, cos / sin are the device's (<= 2 ulp from numpy's)
+ *   d_state_out, d_carry_out (optional) the generator as the planner object holds it after plan(), for a next plan():
+ *              state after the bounded draws and 2 * (n - 1 - f) 64-bit outputs, carry as the bounded draws left it.
+ *              May alias d_state / d_carry.
+ * This replaces the host side of RRTStarInformed.plan (rrtplanner_b200/rrt.py: generator advance + unitball() loop), so
+ * a probe launch (d_balls == NULL in rrtk_plan_batch), this call and the full launch reproduce a seeded planner object. */
+int rrtk_ball_streams(const int32_t *d_rowcum, int W, const rrtk_plan_desc *d_plans, int nplans, int n,
+                      const uint64_t *d_state, const uint32_t *d_carry, const int64_t *d_first, int first_stride,
+                      double *d_balls, uint64_t *d_state_out, uint32_t *d_carry_out, void *stream);
+
 /* ---- K7: the plan() loops (rrt.py:418-437, 498-548, 690-748) + go2goal (rrt.py:284-332) ---------- */
 /*
  * Runs nplans independent plans, one thread block each, tree and bit grid resident on chip.
@@ -394,10 +412,19 @@ int rrtk_ctx_plan_worlds(rrtk_ctx *ctx, int kind, const uint8_t *h_og, int nworl
  *                   plan in h_path / h_xy, h_len, h_path_cost): ~2 KB per plan instead of 16 B per tree row
  * h_stats always comes back.  Output pointers of a mode that is not requested may be NULL.  On an error after the first
  * copy was enqueued the call drains every stream before it returns, so no transfer is still writing into the caller's
- * buffers.  RRTK_PIPE_TRACE=1 in the environment prints the device time stamps of every chunk's stages to stderr. */
+ * buffers.  RRTK_PIPE_TRACE=1 in the environment prints the device time stamps of every chunk's stages to stderr.
+ *   RRTK_SEED_BALLS informed plans in seed mode draw their ellipse phase from the plan's own generator, as a seeded
+ *                   RRTStarInformed object does (rrt.py:85, 240, 579-587): per chunk, sample streams -> probe launch ->
+ *                   rrtk_ball_streams on the probe's statistics -> full launch.  Needs h_state, kind RRTK_INFORMED and
+ *                   h_balls == NULL (RRTK_ERR_INVALID otherwise, before any device work); nothing per iteration is uploaded.
+ *                   The descriptors carry the rotation as before; a plan whose rotation is not finite (start == goal)
+ *                   and that reaches the ellipse phase makes the call fail with RRTK_ERR_INVALID naming it (found on the
+ *                   device, so reported when the call returns).  rrtk_ctx_plan2_worlds takes the flag with cfg->informed
+ *                   and cfg->balls == NULL. */
 #define RRTK_IN_BITS 1
 #define RRTK_OUT_TREES 2
 #define RRTK_OUT_PATHS 4
+#define RRTK_SEED_BALLS 8
 int rrtk_ctx_plan_worlds2(rrtk_ctx *ctx, int kind, const void *h_grids, int nworlds, int W, int H,
                           const rrtk_plan_desc *h_plans, int nplans, int n, double r_rewire, double r_goal,
                           const int16_t *h_samples, const uint64_t *h_state, const double *h_balls, int flags,

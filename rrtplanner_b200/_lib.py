@@ -19,6 +19,8 @@ STAT_NAMES = ("j", "vgoal", "found", "checks", "cells", "first_solution_iter", "
 STAT_COUNT = len(STAT_NAMES)
 
 MODEL_EUCLID, MODEL_DUBINS = 0, 1
+# flags of rrtk_ctx_plan_worlds2 / rrtk_ctx_plan2_worlds
+IN_BITS, OUT_TREES, OUT_PATHS, SEED_BALLS = 1, 2, 4, 8
 STAT2_NAMES = ("j", "vgoal", "found", "checks", "accepted", "rewires", "propagated", "ring_members", "len_evals", "overflow",
                "ell_iters", "first_solution_iter")
 DUBINS_WORDS = ("LSL", "RSR", "LSR", "RSL", "RLR", "LRL")
@@ -83,6 +85,7 @@ SIGNATURES = {
     "rrtk_argsort_scratch_bytes": (_sz, [_i]),
     "rrtk_sample_streams": (_i, [_vp, _vp, _i, _i, _vp, _i, _vp, _i, _vp, _vp]),
     "rrtk_sample_streams_carry": (_i, [_vp, _vp, _i, _i, _vp, _i, _vp, _vp, _i, _vp, _vp]),
+    "rrtk_ball_streams": (_i, [_vp, _i, _vp, _i, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp]),
     "rrtk_plan_batch": (_i, [_i, _vp, _i, _i, _vp, _i, _i, _d, _d, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp]),
     "rrtk_plan_kernel": (C.c_char_p, [_i, _i, _i, _i, _i]),
     "rrtk_plan_footprint": (_i, [_i, _i, _i, _i, _i, _vp, _vp]),
@@ -266,11 +269,12 @@ class Context:
         return pts, cost, parent, stats, ell
 
     def plan_worlds2(self, kind, grids, W, H, desc, n, r_rewire=0.0, r_goal=0.0, samples=None, states=None, balls=None,
-                     bits=False, trees=False, paths=True, path_cap=256, out=None, chunk=0):
+                     bits=False, trees=False, paths=True, path_cap=256, out=None, chunk=0, seed_balls=False):
         """rrtk_ctx_plan_worlds2: ``grids`` is (nworlds, W, H) uint8, or with ``bits=True`` the (nworlds, words) uint32 tiled
         bit grids of pack_grids_host.  Returns a dict with ``stats`` and, as requested, the trees (``pts``, ``cost``,
         ``parent``, ``ell``) and / or the path records (``path``, ``xy``, ``len``, ``path_cost``).  ``out``: optional dict of
-        preallocated (e.g. pinned) host arrays under the same names."""
+        preallocated (e.g. pinned) host arrays under the same names.  ``seed_balls`` (informed, with ``states``, no ``balls``):
+        the ellipse phase draws from each plan's own generator, as a seeded RRTStarInformed object does (RRTK_SEED_BALLS)."""
         grids = np.ascontiguousarray(grids, dtype=np.uint32 if bits else np.uint8)
         nw = grids.shape[0]
         nplans = desc.shape[0]
@@ -281,7 +285,7 @@ class Context:
                 out[name] = np.empty(shape, dtype=dtype)
             return out[name]
         buf("stats", (nplans, STAT_COUNT), np.int64)
-        flags = (1 if bits else 0) | (2 if trees else 0) | (4 if paths else 0)
+        flags = (1 if bits else 0) | (2 if trees else 0) | (4 if paths else 0) | (SEED_BALLS if seed_balls else 0)
         if trees:
             buf("pts", (nplans, n + 1, 2), np.int16); buf("cost", (nplans, n + 1), np.float64); buf("parent", (nplans, n + 1), np.int32)
             if kind == KIND_INFORMED:
@@ -360,11 +364,11 @@ class Context:
         return pts, head, cost, elen, parent, stats
 
     def plan2_worlds(self, cfg, grids, W, H, desc, n, samples=None, states=None, heads=None, bits=False, trees=False, paths=True,
-                     path_cap=256, out=None, chunk=0, balls=None):
+                     path_cap=256, out=None, chunk=0, balls=None, seed_balls=False):
         """rrtk_ctx_plan2_worlds: K8 plans with their worlds in one pipelined call.  ``grids`` as for plan_worlds2.  Returns a
         dict with ``stats`` and, as requested, the trees (``pts``, ``head``, ``cost``, ``elen``, ``parent``) and / or the path
         records (``path``, ``xy``, ``path_head``, ``len``, ``path_cost``); informed plans (``cfg["informed"]``, ``balls`` as for
-        plan2) also return ``ell``."""
+        plan2) also return ``ell``.  ``seed_balls`` as for plan_worlds2 (informed, with ``states``, no ``balls``)."""
         grids = np.ascontiguousarray(grids, dtype=np.uint32 if bits else np.uint8)
         nw = grids.shape[0]
         nplans = desc.shape[0]
@@ -381,7 +385,7 @@ class Context:
                 balls = np.ascontiguousarray(balls, dtype=np.float64)
                 assert balls.shape == (nplans, n, 2), balls.shape
             cfg["balls"], cfg["ell_c"] = (0 if balls is None else balls.ctypes.data), buf("ell", (nplans, n + 1), np.float64).ctypes.data
-        flags = (1 if bits else 0) | (2 if trees else 0) | (4 if paths else 0)
+        flags = (1 if bits else 0) | (2 if trees else 0) | (4 if paths else 0) | (SEED_BALLS if seed_balls else 0)
         if trees:
             buf("pts", (nplans, n + 1, 2), np.int16); buf("head", (nplans, n + 1), np.uint8); buf("cost", (nplans, n + 1), np.float64)
             buf("elen", (nplans, n + 1), np.float64); buf("parent", (nplans, n + 1), np.int32)

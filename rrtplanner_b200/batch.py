@@ -39,6 +39,26 @@ def make_desc(world_ids, starts, goals, rots=None) -> np.ndarray:
     return d
 
 
+def informed_rotations(starts, goals) -> np.ndarray:
+    """(P, 2, 2) ``RRTStarInformed.rotation_to_world_frame`` of every start / goal pair (rrt.py:601-613), stacked: the same
+    numpy calls (unit axis, outer product with [1, 0], SVD, determinants) on a stack of matrices, which gives the per-pair
+    results bit for bit.  Rows where start == goal, whose axis is undefined and where the reference raises, are NaN."""
+    starts = np.asarray(starts).reshape(-1, 2)
+    goals = np.asarray(goals).reshape(-1, 2)
+    span = goals - starts
+    out = np.full((span.shape[0], 2, 2), np.nan)
+    ok = (span != 0).any(axis=1)
+    if ok.any():
+        s = span[ok].astype(np.float64)
+        axis = s / np.sqrt(s[:, 0] * s[:, 0] + s[:, 1] * s[:, 1])[:, None]     # squares and sum are exact integers
+        outer = axis[:, :, None] * np.array([1, 0])[None, None, :]                # np.outer(axis, [1, 0])
+        U, _, V = np.linalg.svd(outer)
+        D = np.zeros_like(U)
+        D[:, 0, 0], D[:, 1, 1] = np.linalg.det(U), np.linalg.det(V)
+        out[ok] = U @ D @ np.swapaxes(V, 1, 2)
+    return out
+
+
 _M32 = np.uint64(0xFFFFFFFF)
 
 
@@ -162,21 +182,38 @@ def plan_batch(kind, ogs, n, starts, goals, world_ids=None, r_rewire=0.0, r_goal
     sample streams -- or ``seeds`` (P,) -- plan p's free-space stream is what a planner built with
     seed=seeds[p] draws (``default_rng(seed).integers(0, nfree, n)``, rrt.py:85,240).
 
-    Informed plans take their ellipse phase from pre-generated streams: ``balls`` (P, n, 2), the unit-disc
+    Informed plans take their ellipse phase either from pre-generated streams: ``balls`` (P, n, 2), the unit-disc
     point iteration i would use (rrt.py:579-587), and ``rots`` (P, 2, 2), ``rotation_to_world_frame`` of each
     pair (rrt.py:601-613).  Both are required: without ``balls`` the kernel runs as a probe that stops at the
     first solution vertex, and without ``rots`` every ellipse sample collapses onto the centre, so neither is
-    accepted silently.  (RRTStarInformed.plan() composes the two launches that reproduce the reference's single
-    interleaved generator; a batch has no such generator.)
+    accepted silently.
+
+    Or, with ``seeds`` and ``balls="seed"``, from each plan's own generator, as a seeded planner object interleaves
+    its free-space and unit-disc draws on one generator (rrt.py:85,240,579-587): plan p is then what
+    ``RRTStarInformed(ogs[world_ids[p]], n, r_rewire, r_goal, seed=seeds[p]).plan(starts[p], goals[p])`` computes.  The
+    device runs a probe to each plan's first solution vertex and draws the unit-disc stream past it (RRTK_SEED_BALLS of
+    ``rrtk_ctx_plan_worlds2``), so nothing per iteration is uploaded.  ``rots`` defaults to ``informed_rotations``; a plan
+    with start == goal that reaches the ellipse phase raises ``np.linalg.LinAlgError``, as the class does.
     """
     k = KINDS[kind] if isinstance(kind, str) else int(kind)
-    if k == _lib.KIND_INFORMED and (balls is None or rots is None):
-        raise ValueError("plan_batch('informed', ...) needs both balls (P, n, 2) and rots (P, 2, 2); see the docstring")
+    seed_balls = isinstance(balls, str)
+    if seed_balls:
+        if balls != "seed" or k != _lib.KIND_INFORMED:
+            raise ValueError("balls='seed' is the only string option, and it is for informed plans")
+        if seeds is None or samples is not None:
+            raise ValueError("balls='seed' draws the ellipse phase from the plans' generators: pass seeds, not samples")
+        if rots is None:
+            rots = informed_rotations(starts, goals)
+    elif k == _lib.KIND_INFORMED and (balls is None or rots is None):
+        raise ValueError("plan_batch('informed', ...) needs both balls (P, n, 2) and rots (P, 2, 2), or seeds with "
+                         "balls='seed'; see the docstring")
     ogs = np.asarray(ogs)
     if ogs.ndim == 2:
         ogs = ogs[None]
     starts = np.asarray(starts).reshape(-1, 2)
     nplans = starts.shape[0]
+    if seed_balls and len(seeds) != nplans:
+        raise ValueError("balls='seed' needs one seed per plan")
     if world_ids is None:
         world_ids = np.arange(nplans) % ogs.shape[0]
     own = ctx is None
@@ -186,15 +223,33 @@ def plan_batch(kind, ogs, n, starts, goals, world_ids=None, r_rewire=0.0, r_goal
         desc = make_desc(world_ids, starts, goals, rots)
         states = None if seeds is None else seed_states(seeds)
         order = np.argsort(desc["world"], kind="stable")          # the pipelined call wants plans grouped by world
-        if (np.diff(desc["world"]) >= 0).all():
-            pts, cost, parent, stats, ell = ctx.plan_worlds(k, og_u8, desc, n, r_rewire, r_goal, samples=samples,
-                                                            states=states, balls=balls)
+        sorted_ = bool((np.diff(desc["world"]) >= 0).all())
+        if sorted_:
+            order = np.arange(nplans)
+        if seed_balls:
+            d = desc[order]
+            stats = np.empty((nplans, _lib.STAT_COUNT), dtype=np.int64)
+            try:
+                o = ctx.plan_worlds2(k, og_u8, og_u8.shape[1], og_u8.shape[2], d, n, r_rewire, r_goal, states=states[order],
+                                     trees=True, paths=False, seed_balls=True, out={"stats": stats})
+            except ValueError as e:
+                bad = (stats[:, 5] >= 0) & ~np.isfinite(d["rot"]).all(axis=1)
+                if "start == goal" not in str(e) or not bad.any():
+                    raise
+                raise np.linalg.LinAlgError(f"plan {int(order[np.argmax(bad)])}: start == goal, so the ellipse of the informed phase "
+                                            "has no axis (rotation_to_world_frame, rrt.py:601-613)") from None
+            res = (o["pts"], o["cost"], o["parent"], o["stats"], o["ell"])
+        elif sorted_:
+            res = ctx.plan_worlds(k, og_u8, desc, n, r_rewire, r_goal, samples=samples, states=states, balls=balls)
         else:
-            inv = np.empty_like(order)
-            inv[order] = np.arange(order.size)
             take = lambda a: None if a is None else np.asarray(a)[order]          # noqa: E731
             res = ctx.plan_worlds(k, og_u8, desc[order], n, r_rewire, r_goal, samples=take(samples), states=take(states),
                                   balls=take(balls))
+        if sorted_:
+            pts, cost, parent, stats, ell = res
+        else:
+            inv = np.empty_like(order)
+            inv[order] = np.arange(order.size)
             pts, cost, parent, stats, ell = (None if a is None else a[inv] for a in res)
     finally:
         if own:
@@ -219,6 +274,7 @@ class DeviceBatch:
         self.words = int(self.L.rrtk_grid_words(W, H))
         self.og = self.bits = self.rowcum = None
         self.desc = self.samples = self.balls = None
+        self.state_out = self.carry_out = None     # seed_informed: the generators after plan()
         self.nplans = 0
         self.out = None
 
@@ -309,6 +365,59 @@ class DeviceBatch:
             _lib.check(self.L.rrtk_sample_streams(self._p(self.bits), self._p(self.rowcum), self.W, self.H, self._p(self.desc),
                                                   self.nplans, self._p(st), self.n, self._p(self.samples), self._stream()),
                        "sample_streams")
+        return self
+
+    def _words(self, a, cols, dtype, name):
+        """(nplans, cols) generator words as a fresh device tensor: a numpy array (uint64 / uint32) or a torch tensor."""
+        t = self.torch
+        if isinstance(a, t.Tensor):
+            w = a.to(self.dev, dtype).clone()
+        else:
+            a = np.ascontiguousarray(a)
+            w = t.from_numpy(a.view(np.int64 if dtype == t.int64 else np.int32).copy()).to(self.dev)
+        if tuple(w.shape) != (self.nplans, cols):
+            raise ValueError(f"{name} must have shape ({self.nplans}, {cols})")
+        return w.contiguous()
+
+    def _is_informed(self) -> bool:
+        return self.kind == _lib.KIND_INFORMED
+
+    def _first_sol_col(self) -> int:
+        return _lib.STAT_NAMES.index("first_solution_iter")
+
+    def _use_balls(self, balls):
+        self.balls = balls
+
+    def seed_informed(self, states, carry=None):
+        """Informed plans from each plan's own generator, as a seeded RRTStarInformed object draws them (rrt.py:85,240,
+        579-587): ``states`` (nplans, 4) PCG64 words (``seed_states(seeds)``, or the ``state_out`` of an earlier batch) and
+        ``carry`` (nplans, 2) numpy's has_uint32 / uinteger (None = a fresh generator).  Enqueues the sample streams, the
+        probe launch (stops at each plan's first solution vertex) and rrtk_ball_streams, which fills the unit-disc stream
+        from the generator past that iteration; ``run()`` then plans.  ``state_out`` / ``carry_out`` (device tensors) hold
+        the generators as the planner objects hold them after plan(), for a next batch.  The descriptors carry the rotation
+        (``make_desc(..., rots=informed_rotations(starts, goals))``)."""
+        t = self.torch
+        if not self._is_informed():
+            raise ValueError("seed_informed is for informed batches")
+        self._require_free_cells()
+        P, n = self.nplans, self.n
+        st = self._words(states, 4, t.int64, "states")
+        cr = t.zeros((P, 2), dtype=t.int32, device=self.dev) if carry is None else self._words(carry, 2, t.int32, "carry")
+        st_s, cr_s = st.clone(), cr.clone()                # the sampler advances its copy past the n free-space draws
+        self.samples = self._empty((P, n, 2), t.int16)
+        balls = self._empty((P, n, 2), t.float64)
+        self.state_out, self.carry_out = t.empty_like(st), t.empty_like(cr)
+        with t.cuda.device(self.dev):
+            _lib.check(self.L.rrtk_sample_streams_carry(self._p(self.bits), self._p(self.rowcum), self.W, self.H, self._p(self.desc), P,
+                                                        self._p(st_s), self._p(cr_s), n, self._p(self.samples), self._stream()),
+                       "sample_streams_carry")
+            self._use_balls(None)
+            self.run()                                      # probe
+            first = self.out["stats"][:, self._first_sol_col()]
+            _lib.check(self.L.rrtk_ball_streams(self._p(self.rowcum), self.W, self._p(self.desc), P, n, self._p(st), self._p(cr),
+                                                first.data_ptr(), _lib.STAT_COUNT, self._p(balls), self._p(self.state_out),
+                                                self._p(self.carry_out), self._stream()), "ball_streams")
+        self._use_balls(balls)
         return self
 
     def run(self):
@@ -428,9 +537,18 @@ class DeviceBatch2(DeviceBatch):
         rotation (make_desc(..., rots=...)).  Without this call an informed batch runs as the probe (stops at the first solution)."""
         b = np.ascontiguousarray(balls, dtype=np.float64)
         assert self.informed and b.shape == (self.nplans, self.n, 2), b.shape
-        self.balls2 = self.torch.from_numpy(b).to(self.dev)
-        self.cfg["balls"] = self.balls2.data_ptr()
+        self._use_balls(self.torch.from_numpy(b).to(self.dev))
         return self
+
+    def _is_informed(self) -> bool:
+        return self.informed
+
+    def _first_sol_col(self) -> int:
+        return _lib.STAT2_NAMES.index("first_solution_iter")
+
+    def _use_balls(self, balls):
+        self.balls2 = balls
+        self.cfg["balls"] = 0 if balls is None else balls.data_ptr()
 
     def set_heads_host(self, heads: np.ndarray):
         h = np.ascontiguousarray(heads, dtype=np.uint8)

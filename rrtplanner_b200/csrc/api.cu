@@ -1,5 +1,6 @@
 // extern "C" surface of librrtk.so (declared in include/rrtk.h): argument checks, device info,
 // the host-buffer context, and thin forwards to the kernel launchers.
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
@@ -47,6 +48,8 @@ int argsort_launch(const int64_t *, int, int32_t *, void *, size_t, cudaStream_t
 size_t argsort_scratch(int);
 int sample_streams_launch(const uint32_t *, const int32_t *, int, int, const rrtk_plan_desc *, int, const uint64_t *, int,
                           int16_t *, int, cudaStream_t, uint64_t * = nullptr, uint32_t * = nullptr);
+int ball_streams_launch(const int32_t *, int, const rrtk_plan_desc *, int, int, const uint64_t *, const uint32_t *, const int64_t *, int,
+                        double *, uint64_t *, uint32_t *, cudaStream_t);
 int plan_launch(int, const uint32_t *, int, int, const rrtk_plan_desc *, int, int, double, double, const int16_t *,
                 const double *, int16_t *, double *, int32_t *, int64_t *, double *, int, int, int, cudaStream_t);
 int plan_footprint(int, int, int, int, int, int, int, int *, int *);
@@ -366,6 +369,17 @@ int rrtk_sample_streams_carry(const uint32_t *d_bits, const int32_t *d_rowcum, i
                                  d_state, d_carry);
 }
 
+int rrtk_ball_streams(const int32_t *d_rowcum, int W, const rrtk_plan_desc *d_plans, int nplans, int n, const uint64_t *d_state,
+                      const uint32_t *d_carry, const int64_t *d_first, int first_stride, double *d_balls, uint64_t *d_state_out,
+                      uint32_t *d_carry_out, void *stream)
+{
+    RRTK_REQUIRE(d_rowcum && d_plans && d_state && d_first && d_balls && nplans >= 0 && n >= 1 && first_stride >= 1,
+                 "rrtk_ball_streams: bad argument (null pointer, nplans < 0, n < 1 or first_stride < 1)");
+    RRTK_TRY(check_grid_dims(W, 1, 16384));
+    return ball_streams_launch(d_rowcum, W, d_plans, nplans, n, d_state, d_carry, d_first, first_stride, d_balls, d_state_out, d_carry_out,
+                               (cudaStream_t)stream);
+}
+
 int rrtk_plan_batch(int kind, const uint32_t *d_bits, int W, int H, const rrtk_plan_desc *d_plans, int nplans, int n,
                     double r_rewire, double r_goal, const int16_t *d_samples, const double *d_balls, int16_t *d_pts,
                     double *d_cost, int32_t *d_parent, int64_t *d_stats, double *d_ell_c, int threads, void *stream)
@@ -647,6 +661,21 @@ static int pipe_require_free_cells(const rrtk_ctx *c, const rrtk_plan_desc *h_pl
     return RRTK_OK;
 }
 
+// RRTK_SEED_BALLS: with start == goal the ellipse has no orientation (rotation_to_world_frame raises, rrt.py:601-613), which
+// the reference meets only once the plan reaches the ellipse phase, i.e. once it has a first solution vertex
+static int pipe_require_rotations(const rrtk_plan_desc *h_plans, const int64_t *h_stats, int nplans, int first_col, const char *who)
+{
+    for (int p = 0; p < nplans; ++p) {
+        const double *r = h_plans[p].rot;
+        if (h_stats[(size_t)p * RRTK_STAT_COUNT + first_col] >= 0 &&
+            !(std::isfinite(r[0]) && std::isfinite(r[1]) && std::isfinite(r[2]) && std::isfinite(r[3]))) {
+            set_error("%s: plan %d reaches the ellipse phase but its rotation is not finite (start == goal)", who, p);
+            return RRTK_ERR_INVALID;
+        }
+    }
+    return RRTK_OK;
+}
+
 static void pipe_drain(rrtk_ctx *c, int *status)
 {
     auto sync = [&](cudaStream_t st) {
@@ -666,6 +695,10 @@ int rrtk_ctx_plan_worlds2(rrtk_ctx *c, int kind, const void *h_grids, int nworld
                           int chunk_plans)
 {
     const bool in_bits = flags & RRTK_IN_BITS, out_trees = flags & RRTK_OUT_TREES, out_paths = flags & RRTK_OUT_PATHS;
+    const bool seed_balls = flags & RRTK_SEED_BALLS;
+    RRTK_REQUIRE(!seed_balls || h_state, "rrtk_ctx_plan_worlds2: RRTK_SEED_BALLS needs seed mode (h_state)");
+    RRTK_REQUIRE(!seed_balls || kind == RRTK_INFORMED, "rrtk_ctx_plan_worlds2: RRTK_SEED_BALLS needs kind RRTK_INFORMED");
+    RRTK_REQUIRE(!seed_balls || !h_balls, "rrtk_ctx_plan_worlds2: RRTK_SEED_BALLS draws the unit-disc stream itself (pass h_balls = NULL)");
     RRTK_REQUIRE(c && h_grids && h_plans && h_stats, "rrtk_ctx_plan_worlds2: null pointer");
     RRTK_REQUIRE(!out_trees || (h_pts && h_cost && h_parent), "rrtk_ctx_plan_worlds2: RRTK_OUT_TREES needs h_pts, h_cost, h_parent");
     RRTK_REQUIRE(!out_paths || (h_path && h_xy && h_len && h_path_cost && path_cap >= 1),
@@ -758,7 +791,8 @@ int rrtk_ctx_plan_worlds2(rrtk_ctx *c, int kind, const void *h_grids, int nworld
                   rrtk_ok(s.cost.reserve(rows1 * max_m * 8)) && rrtk_ok(s.parent.reserve(rows1 * max_m * 4)) &&
                   rrtk_ok(s.stats.reserve(max_m * RRTK_STAT_COUNT * 8));
         if (ok && !in_bits) ok = rrtk_ok(s.og.reserve(cells * max_nw));
-        if (ok && kind == RRTK_INFORMED) ok = rrtk_ok(s.ell.reserve(rows1 * max_m * 8)) && (!h_balls || rrtk_ok(s.balls.reserve(max_m * n * 16)));
+        if (ok && kind == RRTK_INFORMED)
+            ok = rrtk_ok(s.ell.reserve(rows1 * max_m * 8)) && ((!h_balls && !seed_balls) || rrtk_ok(s.balls.reserve(max_m * n * 16)));
         if (ok && out_paths)
             ok = rrtk_ok(s.path.reserve(max_m * path_cap * 4)) && rrtk_ok(s.xy.reserve(max_m * path_cap * 4)) &&
                  rrtk_ok(s.len.reserve(max_m * 4)) && rrtk_ok(s.pcost.reserve(max_m * 8));
@@ -810,8 +844,17 @@ int rrtk_ctx_plan_worlds2(rrtk_ctx *c, int kind, const void *h_grids, int nworld
         st = s.stream;
         if (!cuda_ok(cudaStreamWaitEvent(st, s.ready, 0), "cudaStreamWaitEvent")) break;
         stamp(st);                                                                // [2] plan stream free and inputs ready
+        if (seed_balls) {
+            // probe (stops at the first solution vertex), then the unit-disc stream from the generator past that iteration
+            if (!rrtk_ok(rrtk_plan_batch(kind, s.bits.as<uint32_t>(), W, H, s.plans.as<rrtk_plan_desc>(), m, n, r_rewire, r_goal,
+                                         s.samples.as<int16_t>(), nullptr, s.pts.as<int16_t>(), s.cost.as<double>(), s.parent.as<int32_t>(),
+                                         s.stats.as<int64_t>(), s.ell.as<double>(), 0, st))) break;
+            if (!rrtk_ok(ball_streams_launch(s.rowcum.as<int32_t>(), W, s.plans.as<rrtk_plan_desc>(), m, n, s.state.as<uint64_t>(), nullptr,
+                                             s.stats.as<int64_t>() + RRTK_STAT_FIRST_SOL_ITER, RRTK_STAT_COUNT, s.balls.as<double>(), nullptr,
+                                             nullptr, st))) break;
+        }
         if (!rrtk_ok(rrtk_plan_batch(kind, s.bits.as<uint32_t>(), W, H, s.plans.as<rrtk_plan_desc>(), m, n, r_rewire, r_goal,
-                                     s.samples.as<int16_t>(), (kind == RRTK_INFORMED && h_balls) ? s.balls.as<double>() : nullptr,
+                                     s.samples.as<int16_t>(), (kind == RRTK_INFORMED && (h_balls || seed_balls)) ? s.balls.as<double>() : nullptr,
                                      s.pts.as<int16_t>(), s.cost.as<double>(), s.parent.as<int32_t>(), s.stats.as<int64_t>(),
                                      s.ell.as<double>(), 0, st))) break;
         stamp(st);                                                                // [3] plan kernel done
@@ -851,6 +894,7 @@ int rrtk_ctx_plan_worlds2(rrtk_ctx *c, int kind, const void *h_grids, int nworld
     }
     for (cudaEvent_t e : tev) cudaEventDestroy(e);
     if (status == RRTK_OK && h_state) status = pipe_require_free_cells(c, h_plans, nplans, "rrtk_ctx_plan_worlds2");
+    if (status == RRTK_OK && seed_balls) status = pipe_require_rotations(h_plans, h_stats, nplans, RRTK_STAT_FIRST_SOL_ITER, "rrtk_ctx_plan_worlds2");
     return status;
 }
 
@@ -1291,7 +1335,11 @@ int rrtk_ctx_plan2_worlds(rrtk_ctx *c, const rrtk_plan2_cfg *cfg, const void *h_
                           int16_t *h_xy, uint8_t *h_path_head, int32_t *h_len, double *h_path_cost, int chunk_plans)
 {
     const bool in_bits = flags & RRTK_IN_BITS, out_trees = flags & RRTK_OUT_TREES, out_paths = flags & RRTK_OUT_PATHS;
+    const bool seed_balls = flags & RRTK_SEED_BALLS;
     RRTK_TRY(check_plan2_cfg(cfg));
+    RRTK_REQUIRE(!seed_balls || h_state, "rrtk_ctx_plan2_worlds: RRTK_SEED_BALLS needs seed mode (h_state)");
+    RRTK_REQUIRE(!seed_balls || cfg->informed, "rrtk_ctx_plan2_worlds: RRTK_SEED_BALLS needs cfg->informed");
+    RRTK_REQUIRE(!seed_balls || !cfg->balls, "rrtk_ctx_plan2_worlds: RRTK_SEED_BALLS draws the unit-disc stream itself (pass cfg->balls = NULL)");
     RRTK_REQUIRE(c && h_grids && h_plans && h_stats, "rrtk_ctx_plan2_worlds: null pointer");
     RRTK_REQUIRE(!out_trees || (h_pts && h_head && h_cost && h_elen && h_parent),
                  "rrtk_ctx_plan2_worlds: RRTK_OUT_TREES needs h_pts, h_head, h_cost, h_elen, h_parent");
@@ -1378,7 +1426,7 @@ int rrtk_ctx_plan2_worlds(rrtk_ctx *c, const rrtk_plan2_cfg *cfg, const void *h_
                   rrtk_ok(s.elen.reserve(rows1 * max_m * 8)) && rrtk_ok(s.parent.reserve(rows1 * max_m * 4)) &&
                   rrtk_ok(s.stats.reserve(max_m * RRTK_STAT_COUNT * 8)) && rrtk_ok(s.scratch2.reserve(plan2_scratch_bytes((int)max_m, n)));
         if (ok && !in_bits) ok = rrtk_ok(s.og.reserve(cells * max_nw));
-        if (ok && h_balls) ok = rrtk_ok(s.balls.reserve(max_m * n * 16));
+        if (ok && (h_balls || seed_balls)) ok = rrtk_ok(s.balls.reserve(max_m * n * 16));
         if (ok && h_ell) ok = rrtk_ok(s.ell.reserve(rows1 * max_m * 8));
         if (ok && out_paths)
             ok = rrtk_ok(s.path.reserve(max_m * path_cap * 4)) && rrtk_ok(s.xy.reserve(max_m * path_cap * 4)) &&
@@ -1415,8 +1463,18 @@ int rrtk_ctx_plan2_worlds(rrtk_ctx *c, const rrtk_plan2_cfg *cfg, const void *h_
         if (!cuda_ok(cudaEventRecord(s.ready, st), "cudaEventRecord")) break;
         st = s.stream;
         if (!cuda_ok(cudaStreamWaitEvent(st, s.ready, 0), "cudaStreamWaitEvent")) break;
-        use.balls = h_balls ? s.balls.as<double>() : nullptr;
         use.ell_c = h_ell ? s.ell.as<double>() : nullptr;
+        if (seed_balls) {
+            // probe (stops at the first solution vertex), then the unit-disc stream from the generator past that iteration
+            use.balls = nullptr;
+            if (!rrtk_ok(rrtk_plan2_batch(&use, s.bits.as<uint32_t>(), W, H, s.plans.as<rrtk_plan_desc>(), m, n, s.samples.as<int16_t>(),
+                                          h_heads ? s.heads.as<uint8_t>() : nullptr, s.pts.as<int16_t>(), s.head_out.as<uint8_t>(), s.cost.as<double>(),
+                                          s.elen.as<double>(), s.parent.as<int32_t>(), s.stats.as<int64_t>(), s.scratch2.p, 0, st))) break;
+            if (!rrtk_ok(ball_streams_launch(s.rowcum.as<int32_t>(), W, s.plans.as<rrtk_plan_desc>(), m, n, s.state.as<uint64_t>(), nullptr,
+                                             s.stats.as<int64_t>() + RRTK_STAT2_FIRST_SOL, RRTK_STAT_COUNT, s.balls.as<double>(), nullptr,
+                                             nullptr, st))) break;
+        }
+        use.balls = (h_balls || seed_balls) ? s.balls.as<double>() : nullptr;
         if (!rrtk_ok(rrtk_plan2_batch(&use, s.bits.as<uint32_t>(), W, H, s.plans.as<rrtk_plan_desc>(), m, n, s.samples.as<int16_t>(),
                                       h_heads ? s.heads.as<uint8_t>() : nullptr, s.pts.as<int16_t>(), s.head_out.as<uint8_t>(), s.cost.as<double>(),
                                       s.elen.as<double>(), s.parent.as<int32_t>(), s.stats.as<int64_t>(), s.scratch2.p, 0, st))) break;
@@ -1448,6 +1506,7 @@ int rrtk_ctx_plan2_worlds(rrtk_ctx *c, const rrtk_plan2_cfg *cfg, const void *h_
     pipe_drain(c, &status);
     if (status != RRTK_OK) return status;
     if (h_state) RRTK_TRY(pipe_require_free_cells(c, h_plans, nplans, "rrtk_ctx_plan2_worlds"));
+    if (seed_balls) RRTK_TRY(pipe_require_rotations(h_plans, h_stats, nplans, RRTK_STAT2_FIRST_SOL, "rrtk_ctx_plan2_worlds"));
     for (int p = 0; p < nplans; ++p)
         if (h_stats[(size_t)p * RRTK_STAT_COUNT + RRTK_STAT2_OVERFLOW]) {
             set_error("plan %d: a rewire-radius set exceeded the kernel's list (1024 vertices); reduce r_rewire", p);

@@ -109,9 +109,11 @@ __device__ __forceinline__ U128 add128(U128 a, U128 b)
     r.hi = a.hi + b.hi + (r.lo < a.lo ? 1ull : 0ull);
     return r;
 }
-__device__ __forceinline__ void pcg_jump(Pcg64 &g, unsigned long long delta)
+// delta steps of the LCG as one affine map: state -> state * mult + plus
+struct PcgAffine { U128 mult, plus; };
+__device__ __forceinline__ PcgAffine pcg_affine(unsigned long long inc_hi, unsigned long long inc_lo, unsigned long long delta)
 {
-    U128 cur_mult = {0x2360ED051FC65DA4ull, 0x4385DF649FCCF645ull}, cur_plus = {g.inc_hi, g.inc_lo};
+    U128 cur_mult = {0x2360ED051FC65DA4ull, 0x4385DF649FCCF645ull}, cur_plus = {inc_hi, inc_lo};
     U128 acc_mult = {0ull, 1ull}, acc_plus = {0ull, 0ull};
     while (delta) {
         if (delta & 1ull) {
@@ -122,9 +124,14 @@ __device__ __forceinline__ void pcg_jump(Pcg64 &g, unsigned long long delta)
         cur_mult = mul128(cur_mult, cur_mult);
         delta >>= 1;
     }
-    const U128 st = add128(mul128(acc_mult, U128{g.hi, g.lo}), acc_plus);
+    return PcgAffine{acc_mult, acc_plus};
+}
+__device__ __forceinline__ void pcg_apply(Pcg64 &g, const PcgAffine &a)
+{
+    const U128 st = add128(mul128(a.mult, U128{g.hi, g.lo}), a.plus);
     g.hi = st.hi; g.lo = st.lo;
 }
+__device__ __forceinline__ void pcg_jump(Pcg64 &g, unsigned long long delta) { pcg_apply(g, pcg_affine(g.inc_hi, g.inc_lo, delta)); }
 
 #ifndef RRTK_SAMPLE_THREADS
 #define RRTK_SAMPLE_THREADS 256
@@ -287,6 +294,85 @@ int sample_streams_launch(const uint32_t *d_bits, const int32_t *d_rowcum, int W
         set_error("sample stream of n=%d does not fit shared memory", n);
         return RRTK_ERR_CAPACITY;
     }
+    RRTK_CUDA(cudaGetLastError());
+    return RRTK_OK;
+}
+
+// ---- the ellipse-phase unit-disc stream of RRTStarInformed.plan (rrt.py:579-587, 694-701) -------------------------
+// The reference draws from ONE generator: free[choice(nfree)] in every iteration up to and including the first solution
+// vertex f (rrt.py:240), then unitball() = two uniform(0, 1) draws per iteration (rrt.py:582-583).  Given f from a probe
+// launch, plan p's generator is replayed past its m = f + 1 bounded draws (m = n when f < 0) by thread 0 -- rejections
+// are rare, so that is about m / 2 PCG steps -- and the ellipse phase, a fixed two 64-bit outputs per row, is split over
+// the block: thread t writes rows f+1+t, f+1+t+T, ... (coalesced), jumping 2T - 2 steps between its rows.
+//   uniform(0, 1) = (next64 >> 11) * 2^-53 (numpy's next_double: no use of the buffered 32-bit half)
+//   ball = (sqrt(u1) cos(a), sqrt(u1) sin(a)),  a = 6.283185307179586 * u2  (Python's 2 * np.pi * u)
+// sqrt and the products are correctly rounded; cos / sin are CUDA's (<= 2 ulp), so a ball may differ from numpy's in its
+// last bits.  Rows <= f (every row when f < 0) are 0.0, as RRTStarInformed.plan hands them to the plan kernel.
+constexpr int kBallThreads = 256;
+
+__global__ void __launch_bounds__(kBallThreads)
+ball_stream_kernel(const int *__restrict__ rowcum, int W, const rrtk_plan_desc *__restrict__ plans, int n,
+                   const unsigned long long *state, const uint32_t *carry, const long long *__restrict__ first, int first_stride,
+                   double2 *__restrict__ balls, unsigned long long *state_out, uint32_t *carry_out)
+{
+    __shared__ unsigned long long s_st[4];       // generator after the bounded draws
+    __shared__ int s_first;
+    const int plan = blockIdx.x, tid = threadIdx.x;
+    if (tid == 0) {
+        // only this thread reads the plan's inputs before the barrier, so state_out / carry_out may alias state / carry
+        Pcg64 g;
+        g.hi = state[4 * plan]; g.lo = state[4 * plan + 1];
+        g.inc_hi = state[4 * plan + 2]; g.inc_lo = state[4 * plan + 3];
+        g.has32 = false; g.buf32 = 0;
+        if (carry) { g.has32 = carry[2 * plan] != 0; g.buf32 = carry[2 * plan + 1]; }
+        long long f = first[(size_t)plan * first_stride];
+        if (f < 0 || f >= n) f = -1;             // f = n - 1 and "none" consume the same draws and write the same rows
+        const int fi = (int)f;
+        const uint32_t nfree = (uint32_t)__ldg(rowcum + (size_t)plans[plan].world * (W + 1) + W);
+        if (nfree > 1u) {                        // numpy returns the single value without touching the generator
+            const int m = fi < 0 ? n : fi + 1;
+            for (int i = 0; i < m; ++i) g.bounded(nfree);
+        }
+        s_st[0] = g.hi; s_st[1] = g.lo; s_st[2] = g.inc_hi; s_st[3] = g.inc_lo;
+        s_first = fi;
+        if (carry_out) { carry_out[2 * plan] = g.has32 ? 1u : 0u; carry_out[2 * plan + 1] = g.buf32; }
+        if (state_out) {                         // the generator as the planner object holds it after plan()
+            if (fi >= 0) pcg_jump(g, 2ull * (unsigned long long)(n - 1 - fi));
+            state_out[4 * plan] = g.hi; state_out[4 * plan + 1] = g.lo; state_out[4 * plan + 2] = g.inc_hi; state_out[4 * plan + 3] = g.inc_lo;
+        }
+    }
+    __syncthreads();
+    const int fi = s_first;
+    const int r0 = fi < 0 ? n : fi + 1;          // first ellipse-phase row
+    double2 *out = balls + (size_t)plan * n;
+    for (int i = tid; i < r0; i += kBallThreads) out[i] = make_double2(0.0, 0.0);
+    if (r0 >= n) return;
+    Pcg64 g;
+    g.hi = s_st[0]; g.lo = s_st[1]; g.inc_hi = s_st[2]; g.inc_lo = s_st[3];
+    g.has32 = false; g.buf32 = 0;
+    pcg_jump(g, 2ull * (unsigned long long)tid);
+    const PcgAffine skip = pcg_affine(g.inc_hi, g.inc_lo, 2ull * kBallThreads - 2ull);
+    for (int i = r0 + tid; i < n; i += kBallThreads) {
+        const double u1 = __dmul_rn((double)(g.next64() >> 11), 1.0 / 9007199254740992.0);
+        const double u2 = __dmul_rn((double)(g.next64() >> 11), 1.0 / 9007199254740992.0);
+        const double a = __dmul_rn(6.283185307179586, u2);
+        double s, c;
+        sincos(a, &s, &c);
+        const double r = __dsqrt_rn(u1);
+        out[i] = make_double2(__dmul_rn(r, c), __dmul_rn(r, s));
+        pcg_apply(g, skip);
+    }
+}
+
+int ball_streams_launch(const int32_t *d_rowcum, int W, const rrtk_plan_desc *d_plans, int nplans, int n, const uint64_t *d_state,
+                        const uint32_t *d_carry, const int64_t *d_first, int first_stride, double *d_balls, uint64_t *d_state_out,
+                        uint32_t *d_carry_out, cudaStream_t st)
+{
+    if (nplans == 0) return RRTK_OK;
+    ball_stream_kernel<<<nplans, kBallThreads, 0, st>>>(d_rowcum, W, d_plans, n, reinterpret_cast<const unsigned long long *>(d_state), d_carry,
+                                                        reinterpret_cast<const long long *>(d_first), first_stride,
+                                                        reinterpret_cast<double2 *>(d_balls),
+                                                        reinterpret_cast<unsigned long long *>(d_state_out), d_carry_out);
     RRTK_CUDA(cudaGetLastError());
     return RRTK_OK;
 }
