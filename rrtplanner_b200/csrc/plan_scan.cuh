@@ -20,8 +20,8 @@
 //            sample), then  key < 0  <=>  d2 < r^2  (one funnel shift appends the sign bit to the
 //            thread's membership word) and  min key  <=>  (min d2, lowest row)  (half a 3-input
 //            minimum per pair).  Everything is exact integer arithmetic: |key| < 2^31 is checked
-//            on the host (grids up to 4096 / 2896 / 2048 cells a side for 1 / 2 / 4 membership
-//            words); larger grids use the 32-bit-distance kernel of plan_wide.cu.
+//            on the host as (2 side^2) << sbits <= 2^29 (grids up to 2896 / 2048 / 1448 cells a side
+//            for 1 / 2 / 3-4 membership words); larger grids use the 32-bit-distance kernel of plan_wide.cu.
 //   barrier
 //   owner    the warps take the samples one at a time, first come first served (a sample costs
 //            anything between a duplicate test and several walks), and evaluate each against the

@@ -61,9 +61,7 @@ int RRTK_SCAN_OCC_FN(int T, int K, int two_per_sm, size_t smem)
     switch (K) {
         case 4: return scan_occupancy_k<4>(T, two_per_sm, smem);
         case 8: return scan_occupancy_k<8>(T, two_per_sm, smem);
-#ifdef RRTK_SCAN_K16
         case 16: return scan_occupancy_k<16>(T, two_per_sm, smem);
-#endif
     }
     return 0;
 }
@@ -73,9 +71,7 @@ int RRTK_SCAN_FN(const PlanParams &P, int nplans, int T, int K, int two_per_sm, 
     switch (K) {
         case 4: return scan_launch_k<4>(P, nplans, T, two_per_sm, smem, st);
         case 8: return scan_launch_k<8>(P, nplans, T, two_per_sm, smem, st);
-#ifdef RRTK_SCAN_K16
         case 16: return scan_launch_k<16>(P, nplans, T, two_per_sm, smem, st);
-#endif
     }
     set_error("packed-key plan kernel: unsupported samples per round %d", K);
     return RRTK_ERR_INVALID;

@@ -595,39 +595,54 @@ def small_case(ctx, kind, og, n, xs, xg, samples, r=0.0, rg=0.0, balls=None):
     return res
 
 
-@pytest.mark.parametrize("kind", ["standard", "star", "informed"])
-def test_edge_cases(ctx, kind):
+def edge_cases():
+    """(name, og, n, xs, xg, samples, r, rg, balls) of the small worlds the edge-case tests run, in a fixed draw order."""
     rng = np.random.default_rng(8)
     balls = lambda n: np.stack([O.unitball_from_uniform(*rng.uniform(0, 1, 2)) for _ in range(n)])  # noqa: E731
     empty = np.zeros((30, 20), dtype=np.uint8)
+    cases = []
     # n = 1: a single iteration, tree can never grow (j != n gate), goal connects to the root
-    small_case(ctx, kind, empty, 1, [2, 2], [25, 15], [[5, 5]], 10, 5, balls(1))
+    cases.append(("n1", empty, 1, [2, 2], [25, 15], [[5, 5]], 10, 5, balls(1)))
     # n = 2
-    small_case(ctx, kind, empty, 2, [2, 2], [25, 15], [[5, 5], [6, 6]], 10, 5, balls(2))
+    cases.append(("n2", empty, 2, [2, 2], [25, 15], [[5, 5], [6, 6]], 10, 5, balls(2)))
     # every sample identical; sample equal to the start; sample equal to the goal
-    small_case(ctx, kind, empty, 20, [2, 2], [25, 15], [[7, 7]] * 20, 10, 5, balls(20))
-    small_case(ctx, kind, empty, 20, [2, 2], [25, 15], [[2, 2]] * 10 + [[25, 15]] * 10, 10, 5, balls(20))
+    cases.append(("same_sample", empty, 20, [2, 2], [25, 15], [[7, 7]] * 20, 10, 5, balls(20)))
+    cases.append(("start_goal_samples", empty, 20, [2, 2], [25, 15], [[2, 2]] * 10 + [[25, 15]] * 10, 10, 5, balls(20)))
     # start == goal (probe of the informed phase uses the identity rotation here)
-    small_case(ctx, kind, empty, 30, [9, 9], [9, 9], rng.integers(0, 20, (30, 2)), 8, 3, balls(30))
+    cases.append(("start_is_goal", empty, 30, [9, 9], [9, 9], rng.integers(0, 20, (30, 2)), 8, 3, balls(30)))
     # wall: goal unreachable, vgoal = 0
     wall = np.zeros((40, 30), dtype=np.uint8)
     wall[20] = 1
     left = np.argwhere(wall[:20] == 0)
-    res = small_case(ctx, kind, wall, 50, [3, 3], [35, 20], left[rng.integers(0, len(left), 50)], 10, 4, balls(50))
-    assert int(res.stats[0, 1]) == 0 and int(res.stats[0, 2]) == 0
+    cases.append(("wall", wall, 50, [3, 3], [35, 20], left[rng.integers(0, len(left), 50)], 10, 4, balls(50)))
     # start inside an obstacle: nothing is ever visible from it
     blocked = np.zeros((16, 16), dtype=np.uint8)
     blocked[4, 4] = 1
-    small_case(ctx, kind, blocked, 25, [4, 4], [12, 12], rng.integers(0, 16, (25, 2)), 6, 3, balls(25))
+    cases.append(("blocked_start", blocked, 25, [4, 4], [12, 12], rng.integers(0, 16, (25, 2)), 6, 3, balls(25)))
     # huge radius on a tiny grid: the radius set is the whole tree every time
-    small_case(ctx, kind, empty, 120, [0, 0], [29, 19], rng.integers(0, 20, (120, 2)), 1e6, 4, balls(120))
+    cases.append(("huge_radius", empty, 120, [0, 0], [29, 19], rng.integers(0, 20, (120, 2)), 1e6, 4, balls(120)))
     # radius 0 and non-integer radius
-    small_case(ctx, kind, empty, 60, [0, 0], [29, 19], rng.integers(0, 20, (60, 2)), 0.0, 0.0, balls(60))
-    small_case(ctx, kind, empty, 60, [0, 0], [29, 19], rng.integers(0, 20, (60, 2)), 7.5, 2.5, balls(60))
+    cases.append(("radius0", empty, 60, [0, 0], [29, 19], rng.integers(0, 20, (60, 2)), 0.0, 0.0, balls(60)))
+    cases.append(("radius7.5", empty, 60, [0, 0], [29, 19], rng.integers(0, 20, (60, 2)), 7.5, 2.5, balls(60)))
     # 1-wide grids
     line = np.zeros((1, 64), dtype=np.uint8)
     line[0, 40] = 1
-    small_case(ctx, kind, line, 40, [0, 1], [0, 60], np.stack([np.zeros(40, int), rng.integers(0, 64, 40)], 1), 9, 3, balls(40))
+    cases.append(("one_wide", line, 40, [0, 1], [0, 60], np.stack([np.zeros(40, int), rng.integers(0, 64, 40)], 1), 9, 3, balls(40)))
+    return cases
+
+
+def run_edge_case(ctx, kind, case):
+    name, og, n, xs, xg, samples, r, rg, balls = case
+    res = small_case(ctx, kind, og, n, xs, xg, samples, r, rg, balls)
+    if name == "wall":
+        assert int(res.stats[0, 1]) == 0 and int(res.stats[0, 2]) == 0
+    return res
+
+
+@pytest.mark.parametrize("kind", ["standard", "star", "informed"])
+def test_edge_cases(ctx, kind):
+    for case in edge_cases():
+        run_edge_case(ctx, kind, case)
 
 
 def test_plan_rejects_bad_inputs(ctx):
