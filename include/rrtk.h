@@ -275,6 +275,25 @@ int rrtk_extract_paths_xy(const int32_t *d_parent, const int16_t *d_pts, const d
                           int nplans, int n, int cap, int32_t *d_path, int16_t *d_xy, int32_t *d_len,
                           double *d_path_cost, void *stream);
 
+/* Greedy line-of-sight shortcut of path records, in place (rows as rrtk_extract_paths_xy writes them): the pruning a caller
+ * applies before following or drawing a tree path.  Row p holds m = d_len[p] points q_0 .. q_{m-1} (root first) of world
+ * d_world[p] (NULL = world 0):
+ *     keep = [0]; i = 0
+ *     while i < m - 1:  k = max({k in (i, m-1] : collisionfree(q_i, q_k)} u {i + 1});  keep.append(k); i = k
+ *     cost = sum over consecutive kept (a, b) of sqrt(double(|b - a|^2)), left to right from 0.0
+ * collisionfree is rrt.py:183-229 walked from the earlier point to the later one (the walk rounds halves away from its start,
+ * so the direction matters).  A path nothing can prune keeps its points and gets a cost bit-equal to the tree's vcosts[vgoal].
+ *   d_xy / d_path  kept entries compacted to the front, padded to cap with (-32768, -32768) / -1; d_path (vertex ids) optional
+ *   d_len          number of kept points
+ *   d_keep         optional output: npaths x cap indices of the kept entries in the input row, -1 padded
+ *   d_cost         optional output: the cost above
+ * Rows with d_len <= 0 or d_len > cap (rows rrtk_extract_paths_xy leaves unwritten) are not touched in any array.  Every point of
+ * a processed row must lie inside the (W, H) grid (as for rrtk_collision_segments; rrtk_ctx_shortcut checks it).
+ * 1 <= cap <= RRTK_SHORTCUT_MAX_CAP (RRTK_ERR_CAPACITY above), W, H <= 16384. */
+#define RRTK_SHORTCUT_MAX_CAP 4096
+int rrtk_shortcut_paths(const uint32_t *d_bits, int W, int H, const int32_t *d_world, int npaths, int cap, int16_t *d_xy,
+                        int32_t *d_len, int32_t *d_path, int32_t *d_keep, double *d_cost, void *stream);
+
 /* ---- K8: planners the reference advertises but does not ship ---------------------------------------- */
 /*
  * README.md:12,18-19 of the reference lists a "Dubins Primitive Module", a "Dubins Vehicle RRT Planner" and a
@@ -420,11 +439,17 @@ int rrtk_ctx_plan_worlds(rrtk_ctx *ctx, int kind, const uint8_t *h_og, int nworl
  *                   The descriptors carry the rotation as before; a plan whose rotation is not finite (start == goal)
  *                   and that reaches the ellipse phase makes the call fail with RRTK_ERR_INVALID naming it (found on the
  *                   device, so reported when the call returns).  rrtk_ctx_plan2_worlds takes the flag with cfg->informed
- *                   and cfg->balls == NULL. */
+ *                   and cfg->balls == NULL.
+ *   RRTK_OUT_SHORTCUT  the path records come back shortcut (rrtk_shortcut_paths, one launch per chunk on the chunk's grids
+ *                   after the extraction): h_path / h_xy / h_len hold the kept tree vertices, h_path_cost the pruned cost.
+ *                   Needs RRTK_OUT_PATHS and path_cap <= RRTK_SHORTCUT_MAX_CAP (RRTK_ERR_INVALID / RRTK_ERR_CAPACITY before any
+ *                   device work).  Trees and statistics are unchanged.  rrtk_ctx_plan2_worlds does not read this flag: straight
+ *                   shortcuts would break the heading constraints of Dubins paths. */
 #define RRTK_IN_BITS 1
 #define RRTK_OUT_TREES 2
 #define RRTK_OUT_PATHS 4
 #define RRTK_SEED_BALLS 8
+#define RRTK_OUT_SHORTCUT 16
 int rrtk_ctx_plan_worlds2(rrtk_ctx *ctx, int kind, const void *h_grids, int nworlds, int W, int H,
                           const rrtk_plan_desc *h_plans, int nplans, int n, double r_rewire, double r_goal,
                           const int16_t *h_samples, const uint64_t *h_state, const double *h_balls, int flags,
@@ -448,6 +473,11 @@ int rrtk_ctx_samples(rrtk_ctx *ctx, const rrtk_plan_desc *h_plans, int nplans, i
 /* host-buffer forms of K1-K3 on the context's world `world` */
 int rrtk_ctx_collision(rrtk_ctx *ctx, int world, const int32_t *h_segs, int64_t nseg, uint8_t *h_free,
                        int32_t *h_cells);
+/* host-buffer form of rrtk_shortcut_paths on the context's worlds (h_world per path, NULL = world 0).  Checks every world
+ * index and every point of the processed rows (RRTK_ERR_INVALID) before any device work.  h_path, h_keep, h_cost optional;
+ * rows the call does not process come back as they went in, in every array. */
+int rrtk_ctx_shortcut(rrtk_ctx *ctx, const int32_t *h_world, int npaths, int cap, int16_t *h_xy, int32_t *h_len, int32_t *h_path,
+                      int32_t *h_keep, double *h_cost);
 int rrtk_ctx_nearest(rrtk_ctx *ctx, const int32_t *h_pts, int npts, const int32_t *h_queries, int nq,
                      int32_t *h_idx, int64_t *h_d2);
 int rrtk_ctx_within(rrtk_ctx *ctx, const int32_t *h_pts, int npts, const int32_t *h_queries, int nq,

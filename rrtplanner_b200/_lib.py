@@ -20,7 +20,8 @@ STAT_COUNT = len(STAT_NAMES)
 
 MODEL_EUCLID, MODEL_DUBINS = 0, 1
 # flags of rrtk_ctx_plan_worlds2 / rrtk_ctx_plan2_worlds
-IN_BITS, OUT_TREES, OUT_PATHS, SEED_BALLS = 1, 2, 4, 8
+IN_BITS, OUT_TREES, OUT_PATHS, SEED_BALLS, OUT_SHORTCUT = 1, 2, 4, 8, 16
+SHORTCUT_MAX_CAP = 4096            # RRTK_SHORTCUT_MAX_CAP: longest path row rrtk_shortcut_paths takes
 STAT2_NAMES = ("j", "vgoal", "found", "checks", "accepted", "rewires", "propagated", "ring_members", "len_evals", "overflow",
                "ell_iters", "first_solution_iter")
 DUBINS_WORDS = ("LSL", "RSR", "LSR", "RSL", "RLR", "LRL")
@@ -91,6 +92,7 @@ SIGNATURES = {
     "rrtk_plan_footprint": (_i, [_i, _i, _i, _i, _i, _vp, _vp]),
     "rrtk_extract_paths": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
     "rrtk_extract_paths_xy": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
+    "rrtk_shortcut_paths": (_i, [_vp, _i, _i, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
     "rrtk_create": (_i, [_vp]),
     "rrtk_destroy": (_i, [_vp]),
     "rrtk_ctx_set_grids": (_i, [_vp, _vp, _i, _i, _i, _vp]),
@@ -103,6 +105,7 @@ SIGNATURES = {
     "rrtk_seed_states": (_i, [_vp, _i, _vp]),
     "rrtk_ctx_samples": (_i, [_vp, _vp, _i, _i, _vp, _vp]),
     "rrtk_ctx_collision": (_i, [_vp, _i, _vp, _i64, _vp, _vp]),
+    "rrtk_ctx_shortcut": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp]),
     "rrtk_ctx_nearest": (_i, [_vp, _vp, _i, _vp, _i, _vp, _vp]),
     "rrtk_ctx_nearest_f64": (_i, [_vp, _vp, _i, _vp, _i, _vp, _vp]),
     "rrtk_ctx_within": (_i, [_vp, _vp, _i, _vp, _i, _d, _i, _vp, _vp]),
@@ -269,12 +272,13 @@ class Context:
         return pts, cost, parent, stats, ell
 
     def plan_worlds2(self, kind, grids, W, H, desc, n, r_rewire=0.0, r_goal=0.0, samples=None, states=None, balls=None,
-                     bits=False, trees=False, paths=True, path_cap=256, out=None, chunk=0, seed_balls=False):
+                     bits=False, trees=False, paths=True, path_cap=256, out=None, chunk=0, seed_balls=False, shortcut=False):
         """rrtk_ctx_plan_worlds2: ``grids`` is (nworlds, W, H) uint8, or with ``bits=True`` the (nworlds, words) uint32 tiled
         bit grids of pack_grids_host.  Returns a dict with ``stats`` and, as requested, the trees (``pts``, ``cost``,
         ``parent``, ``ell``) and / or the path records (``path``, ``xy``, ``len``, ``path_cost``).  ``out``: optional dict of
         preallocated (e.g. pinned) host arrays under the same names.  ``seed_balls`` (informed, with ``states``, no ``balls``):
-        the ellipse phase draws from each plan's own generator, as a seeded RRTStarInformed object does (RRTK_SEED_BALLS)."""
+        the ellipse phase draws from each plan's own generator, as a seeded RRTStarInformed object does (RRTK_SEED_BALLS).
+        ``shortcut`` (with ``paths``): the path records come back pruned by line of sight (RRTK_OUT_SHORTCUT, see shortcut())."""
         grids = np.ascontiguousarray(grids, dtype=np.uint32 if bits else np.uint8)
         nw = grids.shape[0]
         nplans = desc.shape[0]
@@ -285,7 +289,7 @@ class Context:
                 out[name] = np.empty(shape, dtype=dtype)
             return out[name]
         buf("stats", (nplans, STAT_COUNT), np.int64)
-        flags = (1 if bits else 0) | (2 if trees else 0) | (4 if paths else 0) | (SEED_BALLS if seed_balls else 0)
+        flags = (1 if bits else 0) | (2 if trees else 0) | (4 if paths else 0) | (SEED_BALLS if seed_balls else 0) | (OUT_SHORTCUT if shortcut else 0)
         if trees:
             buf("pts", (nplans, n + 1, 2), np.int16); buf("cost", (nplans, n + 1), np.float64); buf("parent", (nplans, n + 1), np.int32)
             if kind == KIND_INFORMED:
@@ -427,6 +431,25 @@ class Context:
         check(lib().rrtk_ctx_dubins_sample(self._h, ptr(q), q.shape[0], int(nheadings), float(rho), float(ds), int(cap), ptr(xyth),
                                            ptr(cnt)), "rrtk_ctx_dubins_sample")
         return xyth, cnt
+
+    def shortcut(self, xy, ln, world=None, path=None):
+        """Greedy line-of-sight shortcut of path rows on the context's worlds (rrtk_ctx_shortcut): ``xy`` (P, cap, 2) points root
+        first, ``ln`` (P,) their counts, ``world`` (P,) world per row (None = world 0), ``path`` (P, cap) vertex ids or None.
+        From each kept point the farthest later point the walk of RRT.collisionfree (rrt.py:183-229) reaches is kept next.
+        Returns a new dict: ``xy``, ``len``, ``path`` (None without one) with the kept entries compacted to the front, ``keep``
+        (P, cap) their indices in the input row and ``cost`` (P,) the summed segment lengths.  Rows with ``len`` outside
+        [1, cap] are not processed: their ``keep`` is -1 and their ``cost`` NaN, the rest as given."""
+        xy = np.array(xy, dtype=np.int16, order="C")
+        if xy.ndim != 3 or xy.shape[2] != 2:
+            raise ValueError("xy must have shape (npaths, cap, 2)")
+        P, cap = xy.shape[0], xy.shape[1]
+        ln = np.array(ln, dtype=np.int32, order="C").reshape(P)
+        w = None if world is None else np.ascontiguousarray(world, dtype=np.int32).reshape(P)
+        path = None if path is None else np.array(path, dtype=np.int32, order="C").reshape(P, cap)
+        keep = np.full((P, cap), -1, dtype=np.int32)
+        cost = np.full(P, np.nan)
+        check(lib().rrtk_ctx_shortcut(self._h, ptr(w), P, cap, ptr(xy), ptr(ln), ptr(path), ptr(keep), ptr(cost)), "rrtk_ctx_shortcut")
+        return dict(xy=xy, len=ln, path=path, keep=keep, cost=cost)
 
     # -- queries -------------------------------------------------------------------------------
     def collision(self, segs, world=0, cells=False):

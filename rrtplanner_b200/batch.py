@@ -257,6 +257,42 @@ def plan_batch(kind, ogs, n, starts, goals, world_ids=None, r_rewire=0.0, r_goal
     return BatchResult(pts, cost, parent, stats, ell)
 
 
+def shortcut_paths(ogs, xy, ln, world_ids=None, path=None, ctx: Optional[_lib.Context] = None) -> dict:
+    """Greedy line-of-sight shortcut of path rows, host arrays in and out (``Context.shortcut`` on ``ogs``).
+
+    ogs: (nworlds, W, H) or (W, H), non-zero = obstacle.  ``xy`` (P, cap, 2) holds each path's points root first, as
+    ``path_records`` / ``plan_worlds2(paths=True)`` return them, ``ln`` (P,) their counts, ``world_ids`` (P,) the world of
+    each row (None = world 0) and ``path`` (P, cap) optional vertex ids.  From each kept point, the farthest later point
+    the walk of RRT.collisionfree (rrt.py:183-229) reaches from it is kept next.  Returns a dict with ``xy``, ``len``,
+    ``path``, ``keep`` (indices into the input rows) and ``cost``; the inputs are not modified.  World indices and the
+    points of the rows to process (1 <= len <= cap) are checked against the grids before any device work."""
+    ogs = np.asarray(ogs)
+    if ogs.ndim == 2:
+        ogs = ogs[None]
+    nw, W, H = ogs.shape
+    xy = np.asarray(xy)
+    if xy.ndim != 3 or xy.shape[2] != 2:
+        raise ValueError("xy must have shape (npaths, cap, 2)")
+    P, cap = xy.shape[:2]
+    ln = np.asarray(ln).reshape(P)
+    if world_ids is not None:
+        world_ids = np.asarray(world_ids).reshape(P)
+        if P and (world_ids.min() < 0 or world_ids.max() >= nw):
+            raise ValueError(f"world index out of range [0, {nw})")
+    live = np.arange(cap)[None, :] < np.where((ln >= 1) & (ln <= cap), ln, 0)[:, None]
+    pts = xy[live]
+    if pts.size and (pts.min() < 0 or pts[:, 0].max() >= W or pts[:, 1].max() >= H):
+        raise ValueError(f"a path point lies outside the ({W}, {H}) grid")
+    own = ctx is None
+    ctx = ctx or _lib.Context()
+    try:
+        ctx.set_grids(ogs if ogs.dtype == np.uint8 else (ogs != 0).astype(np.uint8))
+        return ctx.shortcut(xy, ln, world_ids, path)
+    finally:
+        if own:
+            ctx.close()
+
+
 class DeviceBatch:
     """HBM-resident batch on one GPU.  torch is plumbing only: allocation, stream, copies."""
 
@@ -451,6 +487,18 @@ class DeviceBatch:
             _lib.check(self.L.rrtk_extract_paths_xy(self._p(self.out["parent"]), self._p(self.out["pts"]), self._p(self.out["cost"]),
                                                     self._p(self.out["stats"]), P, self.n, cap, self._p(rec["path"]), self._p(rec["xy"]),
                                                     self._p(rec["len"]), self._p(rec["path_cost"]), self._stream()), "extract_paths_xy")
+        return rec
+
+    def shortcut_records(self, rec):
+        """Shortcut the path records of ``path_records()`` in place on torch's current stream (rrtk_shortcut_paths, each plan
+        on its own world): ``path``, ``xy`` and ``len`` then hold the kept vertices and ``path_cost`` the pruned cost.  Plans
+        whose path did not fit the records keep them as they were.  Returns ``rec``."""
+        cap = int(rec["xy"].shape[1])
+        world = self.desc.view(self.torch.int32)[:, 0].contiguous()
+        with self.torch.cuda.device(self.dev):
+            _lib.check(self.L.rrtk_shortcut_paths(self._p(self.bits), self.W, self.H, self._p(world), self.nplans, cap, self._p(rec["xy"]),
+                                                  self._p(rec["len"]), self._p(rec["path"]), None, self._p(rec["path_cost"]),
+                                                  self._stream()), "shortcut_paths")
         return rec
 
     def footprint(self):

@@ -58,6 +58,8 @@ int paths_launch(const int32_t *, const int64_t *, int, int, int, int32_t *, int
 int path_heads_launch(const int32_t *, const uint8_t *, int, int, int, uint8_t *, cudaStream_t);
 int paths_xy_launch(const int32_t *, const int16_t *, const double *, const int64_t *, int, int, int, int32_t *, int16_t *, int32_t *,
                     double *, cudaStream_t);
+int shortcut_launch(const uint32_t *, int, int, const int32_t *, int, int, int, int16_t *, int32_t *, int32_t *, int32_t *, double *,
+                    cudaStream_t);
 int plan2_launch(const rrtk_plan2_cfg &, const uint32_t *, int, int, const rrtk_plan_desc *, int, int, const int16_t *, const uint8_t *,
                  int16_t *, uint8_t *, double *, double *, int32_t *, int64_t *, void *, int, int, cudaStream_t);
 size_t plan2_scratch_bytes(int, int);
@@ -430,6 +432,28 @@ int rrtk_extract_paths_xy(const int32_t *d_parent, const int16_t *d_pts, const d
     return paths_xy_launch(d_parent, d_pts, d_cost, d_stats, nplans, n, cap, d_path, d_xy, d_len, d_path_cost, (cudaStream_t)stream);
 }
 
+static int check_shortcut_cap(int cap, const char *who)
+{
+    if (cap < 1) {
+        set_error("%s: cap must be at least 1", who);
+        return RRTK_ERR_INVALID;
+    }
+    if (cap > RRTK_SHORTCUT_MAX_CAP) {
+        set_error("%s: cap %d above RRTK_SHORTCUT_MAX_CAP (%d): the row is staged in shared memory", who, cap, RRTK_SHORTCUT_MAX_CAP);
+        return RRTK_ERR_CAPACITY;
+    }
+    return RRTK_OK;
+}
+
+int rrtk_shortcut_paths(const uint32_t *d_bits, int W, int H, const int32_t *d_world, int npaths, int cap, int16_t *d_xy, int32_t *d_len,
+                        int32_t *d_path, int32_t *d_keep, double *d_cost, void *stream)
+{
+    RRTK_REQUIRE(npaths >= 0 && (npaths == 0 || (d_bits && d_xy && d_len)), "rrtk_shortcut_paths: null pointer or negative count");
+    RRTK_TRY(check_shortcut_cap(cap, "rrtk_shortcut_paths"));
+    RRTK_TRY(check_grid_dims(W, H, 16384));
+    return shortcut_launch(d_bits, W, H, d_world, 1, npaths, cap, d_xy, d_len, d_path, d_keep, d_cost, (cudaStream_t)stream);
+}
+
 // ---- measured roofline denominators (csrc/peaks.cu) ---------------------------------------------------
 int rrtk_peak_l2_read(const void *d_buf, size_t bytes, int passes, uint32_t *d_sink, int64_t *bytes_read, void *stream)
 {
@@ -695,7 +719,9 @@ int rrtk_ctx_plan_worlds2(rrtk_ctx *c, int kind, const void *h_grids, int nworld
                           int chunk_plans)
 {
     const bool in_bits = flags & RRTK_IN_BITS, out_trees = flags & RRTK_OUT_TREES, out_paths = flags & RRTK_OUT_PATHS;
-    const bool seed_balls = flags & RRTK_SEED_BALLS;
+    const bool seed_balls = flags & RRTK_SEED_BALLS, shortcut = flags & RRTK_OUT_SHORTCUT;
+    RRTK_REQUIRE(!shortcut || out_paths, "rrtk_ctx_plan_worlds2: RRTK_OUT_SHORTCUT needs RRTK_OUT_PATHS");
+    if (shortcut) RRTK_TRY(check_shortcut_cap(path_cap, "rrtk_ctx_plan_worlds2"));
     RRTK_REQUIRE(!seed_balls || h_state, "rrtk_ctx_plan_worlds2: RRTK_SEED_BALLS needs seed mode (h_state)");
     RRTK_REQUIRE(!seed_balls || kind == RRTK_INFORMED, "rrtk_ctx_plan_worlds2: RRTK_SEED_BALLS needs kind RRTK_INFORMED");
     RRTK_REQUIRE(!seed_balls || !h_balls, "rrtk_ctx_plan_worlds2: RRTK_SEED_BALLS draws the unit-disc stream itself (pass h_balls = NULL)");
@@ -865,6 +891,9 @@ int rrtk_ctx_plan_worlds2(rrtk_ctx *c, int kind, const void *h_grids, int nworld
         if (out_paths) {
             ok = rrtk_ok(paths_xy_launch(s.parent.as<int32_t>(), s.pts.as<int16_t>(), s.cost.as<double>(), s.stats.as<int64_t>(), m, n, path_cap,
                                          s.path.as<int32_t>(), s.xy.as<int16_t>(), s.len.as<int32_t>(), s.pcost.as<double>(), st)) &&
+                 (!shortcut || rrtk_ok(shortcut_launch(s.bits.as<uint32_t>(), W, H, &s.plans.as<rrtk_plan_desc>()->world,
+                                                       (int)(sizeof(rrtk_plan_desc) / 4), m, path_cap, s.xy.as<int16_t>(), s.len.as<int32_t>(),
+                                                       s.path.as<int32_t>(), nullptr, s.pcost.as<double>(), st))) &&
                  cuda_ok(cudaMemcpyAsync(h_path + (size_t)p0 * path_cap, s.path.p, (size_t)m * path_cap * 4, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(path)") &&
                  cuda_ok(cudaMemcpyAsync(h_xy + (size_t)p0 * path_cap * 2, s.xy.p, (size_t)m * path_cap * 4, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(xy)") &&
                  cuda_ok(cudaMemcpyAsync(h_len + p0, s.len.p, (size_t)m * 4, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(len)") &&
@@ -1013,6 +1042,56 @@ int rrtk_ctx_collision(rrtk_ctx *c, int world, const int32_t *h_segs, int64_t ns
     RRTK_TRY(rrtk_collision_segments(bits, c->W, c->H, c->a.as<int32_t>(), nullptr, nseg, c->b.as<uint8_t>(), c->c.as<int32_t>(), st));
     RRTK_CUDA(cudaMemcpyAsync(h_free, c->b.p, (size_t)nseg, cudaMemcpyDeviceToHost, st));
     if (h_cells) RRTK_CUDA(cudaMemcpyAsync(h_cells, c->c.p, (size_t)nseg * 4, cudaMemcpyDeviceToHost, st));
+    RRTK_CUDA(cudaStreamSynchronize(st));
+    return RRTK_OK;
+}
+
+int rrtk_ctx_shortcut(rrtk_ctx *c, const int32_t *h_world, int npaths, int cap, int16_t *h_xy, int32_t *h_len, int32_t *h_path,
+                      int32_t *h_keep, double *h_cost)
+{
+    RRTK_REQUIRE(c && npaths >= 0 && (npaths == 0 || (h_xy && h_len)), "rrtk_ctx_shortcut: null pointer or negative count");
+    RRTK_TRY(check_shortcut_cap(cap, "rrtk_ctx_shortcut"));
+    RRTK_REQUIRE(c->nworlds > 0, "rrtk_ctx_shortcut: no worlds (call rrtk_ctx_set_grids)");
+    for (int p = 0; p < npaths; ++p) {
+        const int w = h_world ? h_world[p] : 0;
+        if (w < 0 || w >= c->nworlds) {
+            set_error("rrtk_ctx_shortcut: path %d: world %d out of range [0, %d)", p, w, c->nworlds);
+            return RRTK_ERR_INVALID;
+        }
+        const int m = h_len[p];
+        if (m <= 0 || m > cap) continue;                                          // not processed
+        for (int k = 0; k < m; ++k) {
+            const int x = h_xy[((size_t)p * cap + k) * 2], y = h_xy[((size_t)p * cap + k) * 2 + 1];
+            if (x < 0 || x >= c->W || y < 0 || y >= c->H) {
+                set_error("rrtk_ctx_shortcut: point %d of path %d lies outside the (%d, %d) grid", k, p, c->W, c->H);
+                return RRTK_ERR_INVALID;
+            }
+        }
+    }
+    if (npaths == 0) return RRTK_OK;
+    cudaStream_t st = c->stream;
+    const size_t rows = (size_t)npaths * cap;
+    RRTK_TRY(c->a.reserve(rows * 4));
+    RRTK_TRY(c->b.reserve(rows * 4));
+    RRTK_TRY(c->c.reserve(rows * 4));
+    RRTK_TRY(c->d.reserve((size_t)npaths * 12));
+    RRTK_TRY(c->e.reserve((size_t)npaths * 8));
+    int32_t *d_len = c->d.as<int32_t>(), *d_world = d_len + npaths;
+    RRTK_CUDA(cudaMemcpyAsync(c->a.p, h_xy, rows * 4, cudaMemcpyHostToDevice, st));
+    RRTK_CUDA(cudaMemcpyAsync(d_len, h_len, (size_t)npaths * 4, cudaMemcpyHostToDevice, st));
+    if (h_world) RRTK_CUDA(cudaMemcpyAsync(d_world, h_world, (size_t)npaths * 4, cudaMemcpyHostToDevice, st));
+    // the outputs go up too, so that the rows the kernel does not process come back unchanged
+    if (h_path) RRTK_CUDA(cudaMemcpyAsync(c->b.p, h_path, rows * 4, cudaMemcpyHostToDevice, st));
+    if (h_keep) RRTK_CUDA(cudaMemcpyAsync(c->c.p, h_keep, rows * 4, cudaMemcpyHostToDevice, st));
+    if (h_cost) RRTK_CUDA(cudaMemcpyAsync(c->e.p, h_cost, (size_t)npaths * 8, cudaMemcpyHostToDevice, st));
+    RRTK_TRY(shortcut_launch(c->bits.as<uint32_t>(), c->W, c->H, h_world ? d_world : nullptr, 1, npaths, cap, c->a.as<int16_t>(), d_len,
+                             h_path ? c->b.as<int32_t>() : nullptr, h_keep ? c->c.as<int32_t>() : nullptr, h_cost ? c->e.as<double>() : nullptr,
+                             st));
+    RRTK_CUDA(cudaMemcpyAsync(h_xy, c->a.p, rows * 4, cudaMemcpyDeviceToHost, st));
+    RRTK_CUDA(cudaMemcpyAsync(h_len, d_len, (size_t)npaths * 4, cudaMemcpyDeviceToHost, st));
+    if (h_path) RRTK_CUDA(cudaMemcpyAsync(h_path, c->b.p, rows * 4, cudaMemcpyDeviceToHost, st));
+    if (h_keep) RRTK_CUDA(cudaMemcpyAsync(h_keep, c->c.p, rows * 4, cudaMemcpyDeviceToHost, st));
+    if (h_cost) RRTK_CUDA(cudaMemcpyAsync(h_cost, c->e.p, (size_t)npaths * 8, cudaMemcpyDeviceToHost, st));
     RRTK_CUDA(cudaStreamSynchronize(st));
     return RRTK_OK;
 }

@@ -120,6 +120,21 @@ class RRT(object):
         segs = [[T.nodes[a]["pt"], T.nodes[b]["pt"]] for a, b in zip(path[:-1], path[1:])]
         return np.array(segs)
 
+    def shortcut_path(self, T: nx.DiGraph, path: list) -> List[int]:
+        """The vertices of ``path`` (a ``route2gv`` list) kept by a greedy line-of-sight shortcut on the planner's current grid:
+        from each kept vertex, the farthest later one that ``collisionfree`` sees from it is kept next (walked from the
+        earlier vertex to the later one).  ``vertices_as_ndarray(T, shortcut_path(T, path))`` is the pruned polyline.
+        Runs on the device (rrtk_ctx_shortcut); paths up to 4096 vertices."""
+        path = list(path)
+        if not path:
+            return []
+        pts = np.array([np.asarray(T.nodes[v]["pt"]) for v in path])
+        shape = np.asarray(self.og).shape
+        if pts.min() < 0 or pts[:, 0].max() >= shape[0] or pts[:, 1].max() >= shape[1]:
+            raise ValueError(f"a path vertex lies outside the {shape} grid")
+        res = self._device().shortcut(pts.astype(np.int16)[None], [len(path)])
+        return [path[int(k)] for k in res["keep"][0, : int(res["len"][0])]]
+
     # ---- primitives (static in the reference: rrt.py:131,157,183) --------------------------------
     @staticmethod
     def near(points: np.ndarray, x: np.ndarray) -> np.ndarray:

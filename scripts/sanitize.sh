@@ -18,4 +18,7 @@ run racecheck "tests/test_gpu_rewire.py" "96x96_n500 or 96x96_n600 or several_pl
 run racecheck "tests/test_gpu_parity.py" "sample_stream or rejection_path"
 run synccheck "tests/test_gpu_rewire.py tests/test_gpu_parity.py" "96x96_n500 or 96x96_n600 or several_plans or (test_plan_golden and blobs)"
 run memcheck "tests/test_gpu_parity.py tests/test_gpu_replan.py tests/test_gpu_rewire.py tests/test_gpu_clearance.py" "pipelined or packed_grids or path_records or carry or inflate or edge_cases or 96x96 or dubins_collision or dubins_sample or clearance"
+# the path shortcut (csrc/shortcut.cu): rows staged in shared memory, rewritten in place, on the host entry and in the pipeline
+run memcheck "tests/test_gpu_shortcut.py" "random_polylines or host_entry or fused_flag or device_records"
+run racecheck "tests/test_gpu_shortcut.py" "hand_made or random_polylines"
 cat $LOG
