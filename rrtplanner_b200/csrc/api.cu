@@ -115,9 +115,14 @@ static int check_grid_dims(int W, int H, int limit)
 using namespace rrtk;
 
 // ---- device-side growable buffer used by the host-buffer context ---------------------------------
+// Owns its allocation: a buffer is freed with the struct that holds it, so rrtk_destroy needs no list of them.
 struct DevBuf {
     void *p = nullptr;
     size_t cap = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    ~DevBuf() { release(); }
     int reserve(size_t bytes)
     {
         if (bytes <= cap) return RRTK_OK;
@@ -165,6 +170,306 @@ struct rrtk_ctx {
     int32_t *pin_nfree = nullptr;               // pinned: free cells per world of a pipelined call (seed mode checks them)
     size_t pin_nfree_cap = 0;
 };
+
+// ---- host checks of the plan entries ---------------------------------------------------------------
+// World index and start / goal inside the grid.  ordered_by (the caller's name, or NULL): plans must come in world order, as
+// the pipelined calls upload the worlds of a chunk as one range.  nheadings > 0 (Dubins): the start / goal headings in
+// reserved[0] / reserved[1] must lie in [0, nheadings).
+static int check_plan_descs(const rrtk_plan_desc *h_plans, int nplans, int nworlds, int W, int H, const char *ordered_by, int nheadings)
+{
+    for (int p = 0; p < nplans; ++p) {
+        const rrtk_plan_desc &d = h_plans[p];
+        if (d.world < 0 || d.world >= nworlds || d.start_x < 0 || d.start_x >= W || d.goal_x < 0 || d.goal_x >= W ||
+            d.start_y < 0 || d.start_y >= H || d.goal_y < 0 || d.goal_y >= H) {
+            set_error("plan %d: world index or start/goal outside the grid", p);
+            return RRTK_ERR_INVALID;
+        }
+        if (ordered_by && p && d.world < h_plans[p - 1].world) {
+            set_error("%s: plans must be ordered by world index (plan %d)", ordered_by, p);
+            return RRTK_ERR_INVALID;
+        }
+        if (nheadings > 0 && (d.reserved[0] < 0 || d.reserved[0] >= nheadings || d.reserved[1] < 0 || d.reserved[1] >= nheadings)) {
+            set_error("plan %d: start / goal heading outside [0, %d)", p, nheadings);
+            return RRTK_ERR_INVALID;
+        }
+    }
+    return RRTK_OK;
+}
+
+// h_samples (NULL: nothing to check): n samples per plan, each inside the grid
+static int check_samples(const int16_t *h_samples, int nplans, int n, int W, int H)
+{
+    const size_t total = h_samples ? (size_t)nplans * n : 0;
+    for (size_t i = 0; i < total; ++i) {
+        const int x = h_samples[2 * i], y = h_samples[2 * i + 1];
+        if (x < 0 || x >= W || y < 0 || y >= H) {
+            set_error("sample %zu of plan %zu lies outside the grid", i % n, i / n);
+            return RRTK_ERR_INVALID;
+        }
+    }
+    return RRTK_OK;
+}
+
+// h_heads (NULL: nothing to check): n sample headings per plan, each below nheadings
+static int check_sample_heads(const uint8_t *h_heads, int nplans, int n, int nheadings)
+{
+    const size_t total = h_heads ? (size_t)nplans * n : 0;
+    for (size_t i = 0; i < total; ++i)
+        if (h_heads[i] >= nheadings) {
+            set_error("heading of sample %zu of plan %zu outside [0, %d)", i % n, i / n, nheadings);
+            return RRTK_ERR_INVALID;
+        }
+    return RRTK_OK;
+}
+
+// seed mode draws free[choice(nfree)] (rrt.py:240): a world without a free cell has nothing to draw (numpy raises).
+// nfree: free cells per world, nworlds entries.
+static int require_free_cells(const int32_t *nfree, int nworlds, const rrtk_plan_desc *h_plans, int nplans, const char *who)
+{
+    for (int p = 0; p < nplans; ++p) {
+        const int w = h_plans[p].world;
+        if (w >= 0 && w < nworlds && nfree[w] <= 0) {
+            set_error("%s: world %d of plan %d has no free cell to sample", who, w, p);
+            return RRTK_ERR_INVALID;
+        }
+    }
+    return RRTK_OK;
+}
+
+// K8: a plan whose rewire-radius set overflowed the kernel's list is invalid
+static int check_rewire_overflow(const int64_t *h_stats, int nplans)
+{
+    for (int p = 0; p < nplans; ++p)
+        if (h_stats[(size_t)p * RRTK_STAT_COUNT + RRTK_STAT2_OVERFLOW]) {
+            set_error("plan %d: a rewire-radius set exceeded the kernel's list (1024 vertices); reduce r_rewire", p);
+            return RRTK_ERR_CAPACITY;
+        }
+    return RRTK_OK;
+}
+
+// ---- pipelined plan calls (rrtk_ctx_plan_worlds2, rrtk_ctx_plan2_worlds) ----------------------------
+// What one pipelined call uploads and downloads, whichever planner family plans it.
+struct PipeCall {
+    const char *who;                            // the entry point, for messages
+    const void *grids;                          // nworlds uint8 grids, or tiled bit grids with in_bits
+    int nworlds, W, H;
+    const rrtk_plan_desc *plans;                // ordered by world index
+    int nplans, n;
+    const int16_t *samples;                     // exactly one of samples / state (seed mode)
+    const uint64_t *state;
+    const double *balls;                        // host unit-disc draws of informed plans, or NULL
+    bool in_bits, trees, paths, seed_balls;
+    bool ell;                                   // the plan kernel writes ellipse budgets into the slot's ell buffer
+    int first_col;                              // stats column of the first-solution iteration (RRTK_SEED_BALLS)
+    int16_t *pts; double *cost; int32_t *parent;                        // trees
+    int path_cap; int32_t *path; int16_t *xy; int32_t *len; double *path_cost;   // path records
+    double *ell_c;                              // ellipse budgets to download, or NULL
+    int64_t *stats;
+};
+
+// streams and events of one pipeline slot (and the two shared streams), created on first use; every pipelined call drains all of
+// them before it returns, so the slot's buffers may be regrown right after this
+static int pipe_slot_init(rrtk_ctx *c, PipeSlot &s)
+{
+    if (!c->pipe_prep) {
+        int lo = 0, hi = 0;
+        RRTK_CUDA(cudaDeviceGetStreamPriorityRange(&lo, &hi));                    // hi = numerically lowest = greatest priority
+        RRTK_CUDA(cudaStreamCreateWithPriority(&c->pipe_prep, cudaStreamNonBlocking, hi));
+        RRTK_CUDA(cudaStreamCreateWithPriority(&c->pipe_post, cudaStreamNonBlocking, hi));
+    }
+    if (!s.stream) {
+        RRTK_CUDA(cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking));
+        RRTK_CUDA(cudaEventCreateWithFlags(&s.ready, cudaEventDisableTiming));
+        RRTK_CUDA(cudaEventCreateWithFlags(&s.planned, cudaEventDisableTiming));
+        RRTK_CUDA(cudaEventCreateWithFlags(&s.done, cudaEventDisableTiming));
+    }
+    return RRTK_OK;
+}
+
+static int pipe_nfree_reserve(rrtk_ctx *c, size_t nworlds)
+{
+    if (nworlds <= c->pin_nfree_cap) return RRTK_OK;
+    if (c->pin_nfree) cudaFreeHost(c->pin_nfree);
+    c->pin_nfree = nullptr; c->pin_nfree_cap = 0;
+    RRTK_CUDA(cudaHostAlloc(reinterpret_cast<void **>(&c->pin_nfree), nworlds * sizeof(int32_t), cudaHostAllocDefault));
+    c->pin_nfree_cap = nworlds;
+    return RRTK_OK;
+}
+
+// RRTK_SEED_BALLS: with start == goal the ellipse has no orientation (rotation_to_world_frame raises, rrt.py:601-613), which
+// the reference meets only once the plan reaches the ellipse phase, i.e. once it has a first solution vertex
+static int pipe_require_rotations(const rrtk_plan_desc *h_plans, const int64_t *h_stats, int nplans, int first_col, const char *who)
+{
+    for (int p = 0; p < nplans; ++p) {
+        const double *r = h_plans[p].rot;
+        if (h_stats[(size_t)p * RRTK_STAT_COUNT + first_col] >= 0 &&
+            !(std::isfinite(r[0]) && std::isfinite(r[1]) && std::isfinite(r[2]) && std::isfinite(r[3]))) {
+            set_error("%s: plan %d reaches the ellipse phase but its rotation is not finite (start == goal)", who, p);
+            return RRTK_ERR_INVALID;
+        }
+    }
+    return RRTK_OK;
+}
+
+// Upload, plan and download in chunks of plans on rotating slots, so that host<->device copies of one chunk overlap the
+// kernels of its neighbours.  Chunks hold first_chunk plans, then twice as many each time up to chunk_plans.  Family supplies
+// what differs between the planner families, each hook returning an RRTK status:
+//   reserve(a, slot, max_m)          the family's own slot buffers, for chunks of up to max_m plans
+//   prepare(a, slot, p0, m, stream)  its own uploads of the chunk (preparation stream)
+//   plan(a, slot, m, balls, stream)  the plan launch (plan stream); balls = NULL for the probe of RRTK_SEED_BALLS
+//   paths(a, slot, p0, m, stream)    after path extraction, before the path records go down (output stream)
+//   trees(a, slot, p0, m, stream)    its own tree downloads (output stream)
+template <class Family>
+static int pipe_run(rrtk_ctx *c, const PipeCall &a, int first_chunk, int chunk_plans, Family &f)
+{
+    DevInfo *di;
+    RRTK_TRY(dev_info(&di));
+    const int W = a.W, H = a.H, n = a.n;
+    const size_t cells = (size_t)W * H, words = grid_words(W, H), rows1 = (size_t)n + 1;
+    const size_t grid_bytes = a.in_bits ? words * 4 : cells;
+    // chunk list, then every slot sized once for the largest chunk (growing a buffer later would free it under the pipeline)
+    std::vector<int> starts;
+    for (int p0 = 0, sz = first_chunk; p0 < a.nplans; p0 += sz, sz = (2 * sz < chunk_plans) ? 2 * sz : chunk_plans) starts.push_back(p0);
+    starts.push_back(a.nplans);
+    size_t max_m = 0, max_nw = 0;
+    for (size_t k = 0; k + 1 < starts.size(); ++k) {
+        const size_t m = (size_t)(starts[k + 1] - starts[k]);
+        const size_t nw = (size_t)(a.plans[starts[k + 1] - 1].world - a.plans[starts[k]].world + 1);
+        max_m = m > max_m ? m : max_m;
+        max_nw = nw > max_nw ? nw : max_nw;
+    }
+    // Everything that can fail on the host side happens before the first copy is enqueued; from then on an error is
+    // recorded, the loop stops, and every stream is drained before returning, so that no copy is still writing into the
+    // caller's buffers when the call comes back.
+    int status = RRTK_OK;
+    auto cuda_ok = [&](cudaError_t e, const char *what) {
+        if (e != cudaSuccess && status == RRTK_OK) status = cuda_fail(e, what);
+        return e == cudaSuccess;
+    };
+    auto rrtk_ok = [&](int rc) {
+        if (rc != RRTK_OK && status == RRTK_OK) status = rc;
+        return rc == RRTK_OK;
+    };
+    if (a.state) RRTK_TRY(pipe_nfree_reserve(c, (size_t)a.nworlds));
+    const bool balls = a.balls || a.seed_balls;                                   // the plan kernel reads unit-disc draws
+    const size_t nslots = starts.size() - 1 < (size_t)kPipeSlots ? starts.size() - 1 : (size_t)kPipeSlots;
+    for (size_t k = 0; k < nslots && status == RRTK_OK; ++k) {
+        PipeSlot &s = c->pipe[k];
+        if (!rrtk_ok(pipe_slot_init(c, s))) break;
+        bool ok = rrtk_ok(s.bits.reserve(words * 4 * max_nw)) && rrtk_ok(s.rowcum.reserve((size_t)(W + 1) * 4 * max_nw)) &&
+                  rrtk_ok(s.plans.reserve(sizeof(rrtk_plan_desc) * max_m)) && rrtk_ok(s.samples.reserve(max_m * n * 4)) &&
+                  rrtk_ok(s.state.reserve(max_m * 32)) && rrtk_ok(s.pts.reserve(rows1 * max_m * 4)) &&
+                  rrtk_ok(s.cost.reserve(rows1 * max_m * 8)) && rrtk_ok(s.parent.reserve(rows1 * max_m * 4)) &&
+                  rrtk_ok(s.stats.reserve(max_m * RRTK_STAT_COUNT * 8));
+        if (ok && !a.in_bits) ok = rrtk_ok(s.og.reserve(cells * max_nw));
+        if (ok && balls) ok = rrtk_ok(s.balls.reserve(max_m * n * 16));
+        if (ok && a.ell) ok = rrtk_ok(s.ell.reserve(rows1 * max_m * 8));
+        if (ok && a.paths)
+            ok = rrtk_ok(s.path.reserve(max_m * a.path_cap * 4)) && rrtk_ok(s.xy.reserve(max_m * a.path_cap * 4)) &&
+                 rrtk_ok(s.len.reserve(max_m * 4)) && rrtk_ok(s.pcost.reserve(max_m * 8));
+        if (ok) rrtk_ok(f.reserve(a, s, max_m));
+    }
+    // RRTK_PIPE_TRACE=1 (diagnosis): device-side time stamps of every chunk's stages, printed to stderr after the call
+    const bool trace = getenv("RRTK_PIPE_TRACE") != nullptr;
+    std::vector<cudaEvent_t> tev;
+    auto stamp = [&](cudaStream_t on) {
+        if (!trace) return;
+        cudaEvent_t e = nullptr;
+        cudaEventCreate(&e);
+        cudaEventRecord(e, on);
+        tev.push_back(e);
+    };
+    const auto host_t0 = std::chrono::steady_clock::now();
+    std::vector<double> host_ms;
+    for (size_t ci = 0; ci + 1 < starts.size() && status == RRTK_OK; ++ci) {
+        const int p0 = starts[ci], m = starts[ci + 1] - starts[ci];
+        PipeSlot &s = c->pipe[ci % kPipeSlots];
+        cudaStream_t st = c->pipe_prep;                                           // preparation first (see PipeSlot), then the plan stream
+        if (trace) host_ms.push_back(std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - host_t0).count());
+        stamp(st);                                                                // [0] preparation of the chunk begins
+        if (ci >= (size_t)kPipeSlots && !cuda_ok(cudaStreamWaitEvent(st, s.done, 0), "cudaStreamWaitEvent")) break;   // the slot's last chunk still reads these buffers
+        const int w0 = a.plans[p0].world, w1 = a.plans[p0 + m - 1].world, nw = w1 - w0 + 1;
+        const uint8_t *src = static_cast<const uint8_t *>(a.grids) + grid_bytes * w0;
+        if (a.in_bits) {
+            if (!cuda_ok(cudaMemcpyAsync(s.bits.p, src, grid_bytes * nw, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync(bits)")) break;
+        } else {
+            if (!cuda_ok(cudaMemcpyAsync(s.og.p, src, grid_bytes * nw, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync(og)")) break;
+            if (!rrtk_ok(pack_launch(s.og.as<uint8_t>(), nw, W, H, s.bits.as<uint32_t>(), st))) break;
+        }
+        s.desc.assign(a.plans + p0, a.plans + p0 + m);
+        for (rrtk_plan_desc &d : s.desc) d.world -= w0;
+        if (!cuda_ok(cudaMemcpyAsync(s.plans.p, s.desc.data(), sizeof(rrtk_plan_desc) * m, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync(plans)")) break;
+        if (a.samples) {
+            if (!cuda_ok(cudaMemcpyAsync(s.samples.p, a.samples + (size_t)p0 * n * 2, (size_t)m * n * 4, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync(samples)")) break;
+        } else {
+            if (!rrtk_ok(free_rows_launch(s.bits.as<uint32_t>(), nw, W, H, s.rowcum.as<int32_t>(), st))) break;
+            if (!cuda_ok(cudaMemcpy2DAsync(c->pin_nfree + w0, 4, s.rowcum.as<int32_t>() + W, (size_t)(W + 1) * 4, 4, nw, cudaMemcpyDeviceToHost, st),
+                         "cudaMemcpy2DAsync(nfree)")) break;
+            if (!cuda_ok(cudaMemcpyAsync(s.state.p, a.state + (size_t)p0 * 4, (size_t)m * 32, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync(state)")) break;
+            if (!rrtk_ok(sample_streams_launch(s.bits.as<uint32_t>(), s.rowcum.as<int32_t>(), W, H, s.plans.as<rrtk_plan_desc>(), m,
+                                               s.state.as<uint64_t>(), n, s.samples.as<int16_t>(), di->optin, st))) break;
+        }
+        if (a.balls &&
+            !cuda_ok(cudaMemcpyAsync(s.balls.p, a.balls + (size_t)p0 * n * 2, (size_t)m * n * 16, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync(balls)")) break;
+        if (!rrtk_ok(f.prepare(a, s, p0, m, st))) break;
+        if (!cuda_ok(cudaEventRecord(s.ready, st), "cudaEventRecord")) break;
+        stamp(st);                                                                // [1] inputs ready
+        st = s.stream;
+        if (!cuda_ok(cudaStreamWaitEvent(st, s.ready, 0), "cudaStreamWaitEvent")) break;
+        stamp(st);                                                                // [2] plan stream free and inputs ready
+        if (a.seed_balls) {
+            // probe (stops at the first solution vertex), then the unit-disc stream from the generator past that iteration
+            if (!rrtk_ok(f.plan(a, s, m, nullptr, st))) break;
+            if (!rrtk_ok(ball_streams_launch(s.rowcum.as<int32_t>(), W, s.plans.as<rrtk_plan_desc>(), m, n, s.state.as<uint64_t>(), nullptr,
+                                             s.stats.as<int64_t>() + a.first_col, RRTK_STAT_COUNT, s.balls.as<double>(), nullptr,
+                                             nullptr, st))) break;
+        }
+        if (!rrtk_ok(f.plan(a, s, m, balls ? s.balls.as<double>() : nullptr, st))) break;
+        stamp(st);                                                                // [3] plan kernel done
+        if (!cuda_ok(cudaEventRecord(s.planned, st), "cudaEventRecord")) break;
+        st = c->pipe_post;                                                        // outputs: extraction and downloads, high priority
+        if (!cuda_ok(cudaStreamWaitEvent(st, s.planned, 0), "cudaStreamWaitEvent")) break;
+        bool ok = true;
+        if (a.paths) {
+            const int cap = a.path_cap;
+            ok = rrtk_ok(paths_xy_launch(s.parent.as<int32_t>(), s.pts.as<int16_t>(), s.cost.as<double>(), s.stats.as<int64_t>(), m, n, cap,
+                                         s.path.as<int32_t>(), s.xy.as<int16_t>(), s.len.as<int32_t>(), s.pcost.as<double>(), st)) &&
+                 rrtk_ok(f.paths(a, s, p0, m, st)) &&
+                 cuda_ok(cudaMemcpyAsync(a.path + (size_t)p0 * cap, s.path.p, (size_t)m * cap * 4, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(path)") &&
+                 cuda_ok(cudaMemcpyAsync(a.xy + (size_t)p0 * cap * 2, s.xy.p, (size_t)m * cap * 4, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(xy)") &&
+                 cuda_ok(cudaMemcpyAsync(a.len + p0, s.len.p, (size_t)m * 4, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(len)") &&
+                 cuda_ok(cudaMemcpyAsync(a.path_cost + p0, s.pcost.p, (size_t)m * 8, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(path_cost)");
+        }
+        if (ok && a.trees)
+            ok = cuda_ok(cudaMemcpyAsync(a.pts + (size_t)p0 * rows1 * 2, s.pts.p, rows1 * m * 4, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(pts)") &&
+                 cuda_ok(cudaMemcpyAsync(a.cost + (size_t)p0 * rows1, s.cost.p, rows1 * m * 8, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(cost)") &&
+                 cuda_ok(cudaMemcpyAsync(a.parent + (size_t)p0 * rows1, s.parent.p, rows1 * m * 4, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(parent)") &&
+                 rrtk_ok(f.trees(a, s, p0, m, st));
+        if (ok && a.ell_c) ok = cuda_ok(cudaMemcpyAsync(a.ell_c + (size_t)p0 * rows1, s.ell.p, rows1 * m * 8, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(ell)");
+        if (ok) cuda_ok(cudaMemcpyAsync(a.stats + (size_t)p0 * RRTK_STAT_COUNT, s.stats.p, (size_t)m * RRTK_STAT_COUNT * 8, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(stats)");
+        cuda_ok(cudaEventRecord(s.done, st), "cudaEventRecord");
+        stamp(st);                                                                // [4] results on the host
+    }
+    auto drain = [&](cudaStream_t on) { if (on) cuda_ok(cudaStreamSynchronize(on), "cudaStreamSynchronize"); };
+    drain(c->pipe_prep);
+    for (PipeSlot &s : c->pipe) drain(s.stream);
+    drain(c->pipe_post);
+    if (trace && status == RRTK_OK && tev.size() == 5 * (starts.size() - 1)) {
+        const double host_end = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - host_t0).count();
+        fprintf(stderr, "rrtk pipe trace (ms after the first chunk's preparation began; host = when the host enqueued the chunk; call returned at host %.2f)\n", host_end);
+        for (size_t ci = 0; ci + 1 < starts.size(); ++ci) {
+            float t[5];
+            for (int k = 0; k < 5; ++k) cudaEventElapsedTime(&t[k], tev[0], tev[5 * ci + k]);
+            fprintf(stderr, "  chunk %2zu plans %5d..%5d host %6.2f | prep %6.2f ready %6.2f | plan start %6.2f end %6.2f | out %6.2f\n", ci, starts[ci],
+                    starts[ci + 1], host_ms[ci], t[0], t[1], t[2], t[3], t[4]);
+        }
+    }
+    for (cudaEvent_t e : tev) cudaEventDestroy(e);
+    // seed mode: the free-cell counts came down with the chunks, so a world without a free cell is found only now
+    if (status == RRTK_OK && a.state) status = require_free_cells(c->pin_nfree, a.nworlds, a.plans, a.nplans, a.who);
+    if (status == RRTK_OK && a.seed_balls) status = pipe_require_rotations(a.plans, a.stats, a.nplans, a.first_col, a.who);
+    return status;
+}
 
 extern "C" {
 
@@ -496,13 +801,7 @@ int rrtk_create(rrtk_ctx **out)
 int rrtk_destroy(rrtk_ctx *c)
 {
     if (!c) return RRTK_OK;
-    DevBuf *all[] = {&c->og, &c->bits, &c->rowcum, &c->plans, &c->samples, &c->state, &c->balls, &c->pts,
-                     &c->cost, &c->parent, &c->stats, &c->ell, &c->a, &c->b, &c->c, &c->d, &c->e,
-                     &c->heads, &c->head_out, &c->elen, &c->scratch2, &c->dtable};
-    for (DevBuf *b : all) b->release();
     for (PipeSlot &p : c->pipe) {
-        DevBuf *pb[] = {&p.og, &p.bits, &p.rowcum, &p.plans, &p.samples, &p.state, &p.balls, &p.pts, &p.cost, &p.parent, &p.stats, &p.ell};
-        for (DevBuf *b : pb) b->release();
         if (p.stream) cudaStreamDestroy(p.stream);
         if (p.ready) cudaEventDestroy(p.ready);
         if (p.planned) cudaEventDestroy(p.planned);
@@ -512,7 +811,7 @@ int rrtk_destroy(rrtk_ctx *c)
     if (c->pipe_prep) cudaStreamDestroy(c->pipe_prep);
     if (c->pipe_post) cudaStreamDestroy(c->pipe_post);
     if (c->stream) cudaStreamDestroy(c->stream);
-    delete c;
+    delete c;                                   // the device buffers free themselves
     return RRTK_OK;
 }
 
@@ -534,19 +833,6 @@ int rrtk_ctx_set_grids(rrtk_ctx *c, const uint8_t *h_og, int nworlds, int W, int
     RRTK_CUDA(cudaStreamSynchronize(c->stream));
     if (h_nfree) memcpy(h_nfree, c->nfree.data(), (size_t)nworlds * 4);
     c->W = W; c->H = H; c->nworlds = nworlds;
-    return RRTK_OK;
-}
-
-// seed mode draws free[choice(nfree)] (rrt.py:240): a world without a free cell has nothing to draw (numpy raises)
-static int require_free_cells(const rrtk_ctx *c, const rrtk_plan_desc *h_plans, int nplans, const char *who)
-{
-    for (int p = 0; p < nplans; ++p) {
-        const int w = h_plans[p].world;
-        if (w >= 0 && w < c->nworlds && c->nfree[w] <= 0) {
-            set_error("%s: world %d of plan %d has no free cell to sample", who, w, p);
-            return RRTK_ERR_INVALID;
-        }
-    }
     return RRTK_OK;
 }
 
@@ -583,25 +869,9 @@ int rrtk_ctx_plan(rrtk_ctx *c, int kind, const rrtk_plan_desc *h_plans, int npla
     RRTK_REQUIRE(kind != RRTK_INFORMED || h_ell_c, "rrtk_ctx_plan: informed plans need h_ell_c");
     RRTK_REQUIRE(nplans >= 0 && n >= 1 && n <= 65534, "rrtk_ctx_plan: need nplans >= 0 and 1 <= n <= 65534");
     if (nplans == 0) return RRTK_OK;
-    for (int p = 0; p < nplans; ++p) {
-        const rrtk_plan_desc &d = h_plans[p];
-        if (d.world < 0 || d.world >= c->nworlds || d.start_x < 0 || d.start_x >= c->W || d.goal_x < 0 || d.goal_x >= c->W ||
-            d.start_y < 0 || d.start_y >= c->H || d.goal_y < 0 || d.goal_y >= c->H) {
-            set_error("plan %d: world index or start/goal outside the grid", p);
-            return RRTK_ERR_INVALID;
-        }
-    }
-    if (h_samples) {
-        const size_t total = (size_t)nplans * n;
-        for (size_t i = 0; i < total; ++i) {
-            const int x = h_samples[2 * i], y = h_samples[2 * i + 1];
-            if (x < 0 || x >= c->W || y < 0 || y >= c->H) {
-                set_error("sample %zu of plan %zu lies outside the grid", i % n, i / n);
-                return RRTK_ERR_INVALID;
-            }
-        }
-    }
-    if (h_state) RRTK_TRY(require_free_cells(c, h_plans, nplans, "rrtk_ctx_plan"));
+    RRTK_TRY(check_plan_descs(h_plans, nplans, c->nworlds, c->W, c->H, nullptr, 0));
+    RRTK_TRY(check_samples(h_samples, nplans, n, c->W, c->H));
+    if (h_state) RRTK_TRY(require_free_cells(c->nfree.data(), c->nworlds, h_plans, nplans, "rrtk_ctx_plan"));
     const size_t rows = (size_t)nplans * (n + 1);
     cudaStream_t st = c->stream;
     RRTK_TRY(c->plans.reserve(sizeof(rrtk_plan_desc) * nplans));
@@ -641,77 +911,31 @@ int rrtk_ctx_plan(rrtk_ctx *c, int kind, const rrtk_plan_desc *h_plans, int npla
     return RRTK_OK;
 }
 
-// Upload, plan and download in chunks of plans on rotating streams, so that host<->device copies of
-// one chunk overlap the kernels of its neighbours.  Plans must be ordered by world index.
+// K7 in the pipeline: rrtk_plan_batch, and the path records shortcut on the chunk's grids with RRTK_OUT_SHORTCUT
+struct K7Pipe {
+    int kind;
+    double r_rewire, r_goal;
+    bool shortcut;
+    int reserve(const PipeCall &, PipeSlot &, size_t) { return RRTK_OK; }
+    int prepare(const PipeCall &, PipeSlot &, int, int, cudaStream_t) { return RRTK_OK; }
+    int plan(const PipeCall &a, PipeSlot &s, int m, const double *balls, cudaStream_t st)
+    {
+        return rrtk_plan_batch(kind, s.bits.as<uint32_t>(), a.W, a.H, s.plans.as<rrtk_plan_desc>(), m, a.n, r_rewire, r_goal,
+                               s.samples.as<int16_t>(), balls, s.pts.as<int16_t>(), s.cost.as<double>(), s.parent.as<int32_t>(),
+                               s.stats.as<int64_t>(), s.ell.as<double>(), 0, st);
+    }
+    int paths(const PipeCall &a, PipeSlot &s, int, int m, cudaStream_t st)
+    {
+        if (!shortcut) return RRTK_OK;
+        return shortcut_launch(s.bits.as<uint32_t>(), a.W, a.H, &s.plans.as<rrtk_plan_desc>()->world, (int)(sizeof(rrtk_plan_desc) / 4), m,
+                               a.path_cap, s.xy.as<int16_t>(), s.len.as<int32_t>(), s.path.as<int32_t>(), nullptr, s.pcost.as<double>(), st);
+    }
+    int trees(const PipeCall &, PipeSlot &, int, int, cudaStream_t) { return RRTK_OK; }
+};
+
+// Upload, plan and download in chunks (pipe_run).  Plans must be ordered by world index.
 // flags: RRTK_IN_BITS (h_grids = tiled bit grids, 1/8 of the bytes), RRTK_OUT_TREES, RRTK_OUT_PATHS (path records of
 // path_cap entries per plan); statistics always come back.
-// streams and events of one pipeline slot (and the two shared streams), created on first use; every pipelined call drains all of
-// them before it returns, so the slot's buffers may be regrown right after this
-static int pipe_slot_init(rrtk_ctx *c, PipeSlot &s)
-{
-    if (!c->pipe_prep) {
-        int lo = 0, hi = 0;
-        RRTK_CUDA(cudaDeviceGetStreamPriorityRange(&lo, &hi));                    // hi = numerically lowest = greatest priority
-        RRTK_CUDA(cudaStreamCreateWithPriority(&c->pipe_prep, cudaStreamNonBlocking, hi));
-        RRTK_CUDA(cudaStreamCreateWithPriority(&c->pipe_post, cudaStreamNonBlocking, hi));
-    }
-    if (!s.stream) {
-        RRTK_CUDA(cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking));
-        RRTK_CUDA(cudaEventCreateWithFlags(&s.ready, cudaEventDisableTiming));
-        RRTK_CUDA(cudaEventCreateWithFlags(&s.planned, cudaEventDisableTiming));
-        RRTK_CUDA(cudaEventCreateWithFlags(&s.done, cudaEventDisableTiming));
-    }
-    return RRTK_OK;
-}
-
-static int pipe_nfree_reserve(rrtk_ctx *c, size_t nworlds)
-{
-    if (nworlds <= c->pin_nfree_cap) return RRTK_OK;
-    if (c->pin_nfree) cudaFreeHost(c->pin_nfree);
-    c->pin_nfree = nullptr; c->pin_nfree_cap = 0;
-    RRTK_CUDA(cudaHostAlloc(reinterpret_cast<void **>(&c->pin_nfree), nworlds * sizeof(int32_t), cudaHostAllocDefault));
-    c->pin_nfree_cap = nworlds;
-    return RRTK_OK;
-}
-
-// seed mode draws free[choice(nfree)] (rrt.py:240): the results of a plan on a world without a free cell mean nothing
-static int pipe_require_free_cells(const rrtk_ctx *c, const rrtk_plan_desc *h_plans, int nplans, const char *who)
-{
-    for (int p = 0; p < nplans; ++p)
-        if (c->pin_nfree[h_plans[p].world] <= 0) {
-            set_error("%s: world %d of plan %d has no free cell to sample", who, h_plans[p].world, p);
-            return RRTK_ERR_INVALID;
-        }
-    return RRTK_OK;
-}
-
-// RRTK_SEED_BALLS: with start == goal the ellipse has no orientation (rotation_to_world_frame raises, rrt.py:601-613), which
-// the reference meets only once the plan reaches the ellipse phase, i.e. once it has a first solution vertex
-static int pipe_require_rotations(const rrtk_plan_desc *h_plans, const int64_t *h_stats, int nplans, int first_col, const char *who)
-{
-    for (int p = 0; p < nplans; ++p) {
-        const double *r = h_plans[p].rot;
-        if (h_stats[(size_t)p * RRTK_STAT_COUNT + first_col] >= 0 &&
-            !(std::isfinite(r[0]) && std::isfinite(r[1]) && std::isfinite(r[2]) && std::isfinite(r[3]))) {
-            set_error("%s: plan %d reaches the ellipse phase but its rotation is not finite (start == goal)", who, p);
-            return RRTK_ERR_INVALID;
-        }
-    }
-    return RRTK_OK;
-}
-
-static void pipe_drain(rrtk_ctx *c, int *status)
-{
-    auto sync = [&](cudaStream_t st) {
-        if (!st) return;
-        const cudaError_t e = cudaStreamSynchronize(st);
-        if (e != cudaSuccess && *status == RRTK_OK) *status = cuda_fail(e, "cudaStreamSynchronize");
-    };
-    sync(c->pipe_prep);
-    for (PipeSlot &s : c->pipe) sync(s.stream);
-    sync(c->pipe_post);
-}
-
 int rrtk_ctx_plan_worlds2(rrtk_ctx *c, int kind, const void *h_grids, int nworlds, int W, int H, const rrtk_plan_desc *h_plans,
                           int nplans, int n, double r_rewire, double r_goal, const int16_t *h_samples, const uint64_t *h_state,
                           const double *h_balls, int flags, int path_cap, int16_t *h_pts, double *h_cost, int32_t *h_parent,
@@ -734,7 +958,9 @@ int rrtk_ctx_plan_worlds2(rrtk_ctx *c, int kind, const void *h_grids, int nworld
     RRTK_REQUIRE(nworlds >= 1 && nplans >= 0 && n >= 1 && n <= 65534, "rrtk_ctx_plan_worlds2: need nworlds >= 1, nplans >= 0, 1 <= n <= 65534");
     RRTK_TRY(check_grid_dims(W, H, 16384));
     if (nplans == 0) return RRTK_OK;
-    bool ramp = false;
+    RRTK_TRY(check_plan_descs(h_plans, nplans, nworlds, W, H, "rrtk_ctx_plan_worlds2", 0));
+    RRTK_TRY(check_samples(h_samples, nplans, n, W, H));
+    int first_chunk = chunk_plans;
     if (chunk_plans <= 0) {
         // Chunks of two plan blocks per SM (a fraction of a wave): the next chunks' uploads, packing and sampler kernel
         // need free SM resources to overlap the running plan blocks, and a chunk that fills every SM leaves none until
@@ -749,182 +975,21 @@ int rrtk_ctx_plan_worlds2(rrtk_ctx *c, int kind, const void *h_grids, int nworld
         if (in_bits && !out_trees) chunk_plans = 4 * di->sms;
         if (plan_footprint(kind, W, H, n, 0, di->optin, di->sm_smem, &smem, &per_sm) == RRTK_OK && per_sm > 0 && per_sm < 2)
             chunk_plans = di->sms * per_sm;
-        ramp = true;
+        first_chunk = di->sms < chunk_plans ? di->sms : chunk_plans;              // ramp: the first chunk is on the device sooner
     }
-    for (int p = 0; p < nplans; ++p) {
-        const rrtk_plan_desc &d = h_plans[p];
-        if (d.world < 0 || d.world >= nworlds || d.start_x < 0 || d.start_x >= W || d.goal_x < 0 || d.goal_x >= W ||
-            d.start_y < 0 || d.start_y >= H || d.goal_y < 0 || d.goal_y >= H) {
-            set_error("plan %d: world index or start/goal outside the grid", p);
-            return RRTK_ERR_INVALID;
-        }
-        if (p && d.world < h_plans[p - 1].world) {
-            set_error("rrtk_ctx_plan_worlds: plans must be ordered by world index (plan %d)", p);
-            return RRTK_ERR_INVALID;
-        }
-    }
-    if (h_samples) {
-        const size_t total = (size_t)nplans * n;
-        for (size_t i = 0; i < total; ++i) {
-            const int x = h_samples[2 * i], y = h_samples[2 * i + 1];
-            if (x < 0 || x >= W || y < 0 || y >= H) {
-                set_error("sample %zu of plan %zu lies outside the grid", i % n, i / n);
-                return RRTK_ERR_INVALID;
-            }
-        }
-    }
-    DevInfo *di;
-    RRTK_TRY(dev_info(&di));
-    const size_t cells = (size_t)W * H, words = grid_words(W, H), rows1 = (size_t)n + 1;
-    const size_t grid_bytes = in_bits ? words * 4 : cells;
-    // chunk list, then every slot sized once for the largest chunk (growing a buffer later would free it under the pipeline)
-    std::vector<int> starts;
-    {
-        int sz = ramp ? (di->sms < chunk_plans ? di->sms : chunk_plans) : chunk_plans;
-        for (int p0 = 0; p0 < nplans; p0 += sz, sz = (2 * sz < chunk_plans) ? 2 * sz : chunk_plans) {
-            starts.push_back(p0);
-            if (p0 + sz >= nplans) break;
-        }
-        starts.push_back(nplans);
-    }
-    size_t max_m = 0, max_nw = 0;
-    for (size_t k = 0; k + 1 < starts.size(); ++k) {
-        const size_t m = (size_t)(starts[k + 1] - starts[k]);
-        const size_t nw = (size_t)(h_plans[starts[k + 1] - 1].world - h_plans[starts[k]].world + 1);
-        max_m = m > max_m ? m : max_m;
-        max_nw = nw > max_nw ? nw : max_nw;
-    }
-    // Everything that can fail on the host side happens before the first copy is enqueued; from then on an error is
-    // recorded, the loop stops, and every stream is drained before returning, so that no copy is still writing into the
-    // caller's buffers when the call comes back.
-    int status = RRTK_OK;
-    auto cuda_ok = [&](cudaError_t e, const char *what) {
-        if (e != cudaSuccess && status == RRTK_OK) status = cuda_fail(e, what);
-        return e == cudaSuccess;
-    };
-    auto rrtk_ok = [&](int rc) {
-        if (rc != RRTK_OK && status == RRTK_OK) status = rc;
-        return rc == RRTK_OK;
-    };
-    if (h_state) RRTK_TRY(pipe_nfree_reserve(c, (size_t)nworlds));
-    const size_t nslots = starts.size() - 1 < (size_t)kPipeSlots ? starts.size() - 1 : (size_t)kPipeSlots;
-    for (size_t k = 0; k < nslots && status == RRTK_OK; ++k) {
-        PipeSlot &s = c->pipe[k];
-        if (!rrtk_ok(pipe_slot_init(c, s))) break;
-        bool ok = rrtk_ok(s.bits.reserve(words * 4 * max_nw)) && rrtk_ok(s.rowcum.reserve((size_t)(W + 1) * 4 * max_nw)) &&
-                  rrtk_ok(s.plans.reserve(sizeof(rrtk_plan_desc) * max_m)) && rrtk_ok(s.samples.reserve(max_m * n * 4)) &&
-                  rrtk_ok(s.state.reserve(max_m * 32)) && rrtk_ok(s.pts.reserve(rows1 * max_m * 4)) &&
-                  rrtk_ok(s.cost.reserve(rows1 * max_m * 8)) && rrtk_ok(s.parent.reserve(rows1 * max_m * 4)) &&
-                  rrtk_ok(s.stats.reserve(max_m * RRTK_STAT_COUNT * 8));
-        if (ok && !in_bits) ok = rrtk_ok(s.og.reserve(cells * max_nw));
-        if (ok && kind == RRTK_INFORMED)
-            ok = rrtk_ok(s.ell.reserve(rows1 * max_m * 8)) && ((!h_balls && !seed_balls) || rrtk_ok(s.balls.reserve(max_m * n * 16)));
-        if (ok && out_paths)
-            ok = rrtk_ok(s.path.reserve(max_m * path_cap * 4)) && rrtk_ok(s.xy.reserve(max_m * path_cap * 4)) &&
-                 rrtk_ok(s.len.reserve(max_m * 4)) && rrtk_ok(s.pcost.reserve(max_m * 8));
-    }
-    // RRTK_PIPE_TRACE=1 (diagnosis): device-side time stamps of every chunk's stages, printed to stderr after the call
-    const bool trace = getenv("RRTK_PIPE_TRACE") != nullptr;
-    std::vector<cudaEvent_t> tev;
-    auto stamp = [&](cudaStream_t on) {
-        if (!trace) return;
-        cudaEvent_t e = nullptr;
-        cudaEventCreate(&e);
-        cudaEventRecord(e, on);
-        tev.push_back(e);
-    };
-    const auto host_t0 = std::chrono::steady_clock::now();
-    std::vector<double> host_ms;
-    for (size_t ci = 0; ci + 1 < starts.size() && status == RRTK_OK; ++ci) {
-        const int p0 = starts[ci], m = starts[ci + 1] - starts[ci];
-        PipeSlot &s = c->pipe[ci % kPipeSlots];
-        cudaStream_t st = c->pipe_prep;                                           // preparation first (see PipeSlot), then the plan stream
-        if (trace) host_ms.push_back(std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - host_t0).count());
-        stamp(st);                                                                // [0] preparation of the chunk begins
-        if (ci >= (size_t)kPipeSlots && !cuda_ok(cudaStreamWaitEvent(st, s.done, 0), "cudaStreamWaitEvent")) break;   // the slot's last chunk still reads these buffers
-        const int w0 = h_plans[p0].world, w1 = h_plans[p0 + m - 1].world, nw = w1 - w0 + 1;
-        const uint8_t *src = static_cast<const uint8_t *>(h_grids) + grid_bytes * w0;
-        if (in_bits) {
-            if (!cuda_ok(cudaMemcpyAsync(s.bits.p, src, grid_bytes * nw, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync(bits)")) break;
-        } else {
-            if (!cuda_ok(cudaMemcpyAsync(s.og.p, src, grid_bytes * nw, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync(og)")) break;
-            if (!rrtk_ok(pack_launch(s.og.as<uint8_t>(), nw, W, H, s.bits.as<uint32_t>(), st))) break;
-        }
-        if (!rrtk_ok(free_rows_launch(s.bits.as<uint32_t>(), nw, W, H, s.rowcum.as<int32_t>(), st))) break;
-        if (h_state && !cuda_ok(cudaMemcpy2DAsync(c->pin_nfree + w0, 4, s.rowcum.as<int32_t>() + W, (size_t)(W + 1) * 4, 4, nw, cudaMemcpyDeviceToHost, st),
-                                "cudaMemcpy2DAsync(nfree)")) break;
-        s.desc.assign(h_plans + p0, h_plans + p0 + m);
-        for (rrtk_plan_desc &d : s.desc) d.world -= w0;
-        if (!cuda_ok(cudaMemcpyAsync(s.plans.p, s.desc.data(), sizeof(rrtk_plan_desc) * m, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync(plans)")) break;
-        if (h_samples) {
-            if (!cuda_ok(cudaMemcpyAsync(s.samples.p, h_samples + (size_t)p0 * n * 2, (size_t)m * n * 4, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync(samples)")) break;
-        } else {
-            if (!cuda_ok(cudaMemcpyAsync(s.state.p, h_state + (size_t)p0 * 4, (size_t)m * 32, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync(state)")) break;
-            if (!rrtk_ok(sample_streams_launch(s.bits.as<uint32_t>(), s.rowcum.as<int32_t>(), W, H, s.plans.as<rrtk_plan_desc>(), m,
-                                               s.state.as<uint64_t>(), n, s.samples.as<int16_t>(), di->optin, st))) break;
-        }
-        if (kind == RRTK_INFORMED && h_balls &&
-            !cuda_ok(cudaMemcpyAsync(s.balls.p, h_balls + (size_t)p0 * n * 2, (size_t)m * n * 16, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync(balls)")) break;
-        if (!cuda_ok(cudaEventRecord(s.ready, st), "cudaEventRecord")) break;
-        stamp(st);                                                                // [1] inputs ready
-        st = s.stream;
-        if (!cuda_ok(cudaStreamWaitEvent(st, s.ready, 0), "cudaStreamWaitEvent")) break;
-        stamp(st);                                                                // [2] plan stream free and inputs ready
-        if (seed_balls) {
-            // probe (stops at the first solution vertex), then the unit-disc stream from the generator past that iteration
-            if (!rrtk_ok(rrtk_plan_batch(kind, s.bits.as<uint32_t>(), W, H, s.plans.as<rrtk_plan_desc>(), m, n, r_rewire, r_goal,
-                                         s.samples.as<int16_t>(), nullptr, s.pts.as<int16_t>(), s.cost.as<double>(), s.parent.as<int32_t>(),
-                                         s.stats.as<int64_t>(), s.ell.as<double>(), 0, st))) break;
-            if (!rrtk_ok(ball_streams_launch(s.rowcum.as<int32_t>(), W, s.plans.as<rrtk_plan_desc>(), m, n, s.state.as<uint64_t>(), nullptr,
-                                             s.stats.as<int64_t>() + RRTK_STAT_FIRST_SOL_ITER, RRTK_STAT_COUNT, s.balls.as<double>(), nullptr,
-                                             nullptr, st))) break;
-        }
-        if (!rrtk_ok(rrtk_plan_batch(kind, s.bits.as<uint32_t>(), W, H, s.plans.as<rrtk_plan_desc>(), m, n, r_rewire, r_goal,
-                                     s.samples.as<int16_t>(), (kind == RRTK_INFORMED && (h_balls || seed_balls)) ? s.balls.as<double>() : nullptr,
-                                     s.pts.as<int16_t>(), s.cost.as<double>(), s.parent.as<int32_t>(), s.stats.as<int64_t>(),
-                                     s.ell.as<double>(), 0, st))) break;
-        stamp(st);                                                                // [3] plan kernel done
-        if (!cuda_ok(cudaEventRecord(s.planned, st), "cudaEventRecord")) break;
-        st = c->pipe_post;                                                        // outputs: extraction and downloads, high priority
-        if (!cuda_ok(cudaStreamWaitEvent(st, s.planned, 0), "cudaStreamWaitEvent")) break;
-        bool ok = true;
-        if (out_paths) {
-            ok = rrtk_ok(paths_xy_launch(s.parent.as<int32_t>(), s.pts.as<int16_t>(), s.cost.as<double>(), s.stats.as<int64_t>(), m, n, path_cap,
-                                         s.path.as<int32_t>(), s.xy.as<int16_t>(), s.len.as<int32_t>(), s.pcost.as<double>(), st)) &&
-                 (!shortcut || rrtk_ok(shortcut_launch(s.bits.as<uint32_t>(), W, H, &s.plans.as<rrtk_plan_desc>()->world,
-                                                       (int)(sizeof(rrtk_plan_desc) / 4), m, path_cap, s.xy.as<int16_t>(), s.len.as<int32_t>(),
-                                                       s.path.as<int32_t>(), nullptr, s.pcost.as<double>(), st))) &&
-                 cuda_ok(cudaMemcpyAsync(h_path + (size_t)p0 * path_cap, s.path.p, (size_t)m * path_cap * 4, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(path)") &&
-                 cuda_ok(cudaMemcpyAsync(h_xy + (size_t)p0 * path_cap * 2, s.xy.p, (size_t)m * path_cap * 4, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(xy)") &&
-                 cuda_ok(cudaMemcpyAsync(h_len + p0, s.len.p, (size_t)m * 4, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(len)") &&
-                 cuda_ok(cudaMemcpyAsync(h_path_cost + p0, s.pcost.p, (size_t)m * 8, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(path_cost)");
-        }
-        if (ok && out_trees) {
-            ok = cuda_ok(cudaMemcpyAsync(h_pts + (size_t)p0 * rows1 * 2, s.pts.p, rows1 * m * 4, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(pts)") &&
-                 cuda_ok(cudaMemcpyAsync(h_cost + (size_t)p0 * rows1, s.cost.p, rows1 * m * 8, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(cost)") &&
-                 cuda_ok(cudaMemcpyAsync(h_parent + (size_t)p0 * rows1, s.parent.p, rows1 * m * 4, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(parent)");
-            if (ok && kind == RRTK_INFORMED)
-                ok = cuda_ok(cudaMemcpyAsync(h_ell_c + (size_t)p0 * rows1, s.ell.p, rows1 * m * 8, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(ell)");
-        }
-        if (ok) cuda_ok(cudaMemcpyAsync(h_stats + (size_t)p0 * RRTK_STAT_COUNT, s.stats.p, (size_t)m * RRTK_STAT_COUNT * 8, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(stats)");
-        cuda_ok(cudaEventRecord(s.done, st), "cudaEventRecord");
-        stamp(st);                                                                // [4] results on the host
-    }
-    pipe_drain(c, &status);
-    if (trace && status == RRTK_OK && tev.size() == 5 * (starts.size() - 1)) {
-        const double host_end = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - host_t0).count();
-        fprintf(stderr, "rrtk pipe trace (ms after the first chunk's preparation began; host = when the host enqueued the chunk; call returned at host %.2f)\n", host_end);
-        for (size_t ci = 0; ci + 1 < starts.size(); ++ci) {
-            float t[5];
-            for (int k = 0; k < 5; ++k) cudaEventElapsedTime(&t[k], tev[0], tev[5 * ci + k]);
-            fprintf(stderr, "  chunk %2zu plans %5d..%5d host %6.2f | prep %6.2f ready %6.2f | plan start %6.2f end %6.2f | out %6.2f\n", ci, starts[ci],
-                    starts[ci + 1], host_ms[ci], t[0], t[1], t[2], t[3], t[4]);
-        }
-    }
-    for (cudaEvent_t e : tev) cudaEventDestroy(e);
-    if (status == RRTK_OK && h_state) status = pipe_require_free_cells(c, h_plans, nplans, "rrtk_ctx_plan_worlds2");
-    if (status == RRTK_OK && seed_balls) status = pipe_require_rotations(h_plans, h_stats, nplans, RRTK_STAT_FIRST_SOL_ITER, "rrtk_ctx_plan_worlds2");
-    return status;
+    const bool informed = kind == RRTK_INFORMED;
+    PipeCall a = {};
+    a.who = "rrtk_ctx_plan_worlds2";
+    a.grids = h_grids; a.nworlds = nworlds; a.W = W; a.H = H;
+    a.plans = h_plans; a.nplans = nplans; a.n = n;
+    a.samples = h_samples; a.state = h_state; a.balls = informed ? h_balls : nullptr;
+    a.in_bits = in_bits; a.trees = out_trees; a.paths = out_paths; a.seed_balls = seed_balls;
+    a.ell = informed; a.first_col = RRTK_STAT_FIRST_SOL_ITER;
+    a.pts = h_pts; a.cost = h_cost; a.parent = h_parent;
+    a.path_cap = path_cap; a.path = h_path; a.xy = h_xy; a.len = h_len; a.path_cost = h_path_cost;
+    a.ell_c = informed && out_trees ? h_ell_c : nullptr; a.stats = h_stats;
+    K7Pipe f = {kind, r_rewire, r_goal, shortcut};
+    return pipe_run(c, a, first_chunk, chunk_plans, f);
 }
 
 // the round-1 form: uint8 grids in, every tree out
@@ -1005,7 +1070,7 @@ int rrtk_ctx_samples(rrtk_ctx *c, const rrtk_plan_desc *h_plans, int nplans, int
     RRTK_REQUIRE(c && h_plans && h_state && h_samples && nplans >= 1 && n >= 1, "rrtk_ctx_samples: bad argument");
     RRTK_REQUIRE(c->nworlds > 0, "rrtk_ctx_samples: call rrtk_ctx_set_grids first");
     for (int p = 0; p < nplans; ++p) RRTK_REQUIRE(h_plans[p].world >= 0 && h_plans[p].world < c->nworlds, "rrtk_ctx_samples: bad world index");
-    RRTK_TRY(require_free_cells(c, h_plans, nplans, "rrtk_ctx_samples"));
+    RRTK_TRY(require_free_cells(c->nfree.data(), c->nworlds, h_plans, nplans, "rrtk_ctx_samples"));
     DevInfo *d;
     RRTK_TRY(dev_info(&d));
     cudaStream_t st = c->stream;
@@ -1319,35 +1384,11 @@ int rrtk_ctx_plan2(rrtk_ctx *c, const rrtk_plan2_cfg *cfg, const rrtk_plan_desc 
     RRTK_REQUIRE(nplans >= 0 && n >= 1 && n <= 65534, "rrtk_ctx_plan2: need nplans >= 0 and 1 <= n <= 65534");
     if (nplans == 0) return RRTK_OK;
     const bool dub = cfg->model == RRTK_MODEL_DUBINS;
-    for (int p = 0; p < nplans; ++p) {
-        const rrtk_plan_desc &d = h_plans[p];
-        if (d.world < 0 || d.world >= c->nworlds || d.start_x < 0 || d.start_x >= c->W || d.goal_x < 0 || d.goal_x >= c->W ||
-            d.start_y < 0 || d.start_y >= c->H || d.goal_y < 0 || d.goal_y >= c->H) {
-            set_error("plan %d: world index or start/goal outside the grid", p);
-            return RRTK_ERR_INVALID;
-        }
-        if (dub && (d.reserved[0] < 0 || d.reserved[0] >= cfg->nheadings || d.reserved[1] < 0 || d.reserved[1] >= cfg->nheadings)) {
-            set_error("plan %d: start / goal heading outside [0, %d)", p, cfg->nheadings);
-            return RRTK_ERR_INVALID;
-        }
-    }
-    if (h_state) RRTK_TRY(require_free_cells(c, h_plans, nplans, "rrtk_ctx_plan2"));
-    const size_t total = (size_t)nplans * n;
-    if (h_samples)
-        for (size_t i = 0; i < total; ++i) {
-            const int x = h_samples[2 * i], y = h_samples[2 * i + 1];
-            if (x < 0 || x >= c->W || y < 0 || y >= c->H) {
-                set_error("sample %zu of plan %zu lies outside the grid", i % n, i / n);
-                return RRTK_ERR_INVALID;
-            }
-        }
-    if (dub && h_heads)
-        for (size_t i = 0; i < total; ++i)
-            if (h_heads[i] >= cfg->nheadings) {
-                set_error("heading of sample %zu of plan %zu outside [0, %d)", i % n, i / n, cfg->nheadings);
-                return RRTK_ERR_INVALID;
-            }
-    const size_t rows = (size_t)nplans * (n + 1);
+    RRTK_TRY(check_plan_descs(h_plans, nplans, c->nworlds, c->W, c->H, nullptr, dub ? cfg->nheadings : 0));
+    if (h_state) RRTK_TRY(require_free_cells(c->nfree.data(), c->nworlds, h_plans, nplans, "rrtk_ctx_plan2"));
+    RRTK_TRY(check_samples(h_samples, nplans, n, c->W, c->H));
+    RRTK_TRY(check_sample_heads(dub ? h_heads : nullptr, nplans, n, cfg->nheadings));
+    const size_t total = (size_t)nplans * n, rows = (size_t)nplans * (n + 1);
     cudaStream_t st = c->stream;
     RRTK_TRY(c->plans.reserve(sizeof(rrtk_plan_desc) * nplans));
     RRTK_TRY(c->samples.reserve(total * 4));
@@ -1399,13 +1440,52 @@ int rrtk_ctx_plan2(rrtk_ctx *c, const rrtk_plan2_cfg *cfg, const rrtk_plan_desc 
     RRTK_CUDA(cudaMemcpyAsync(h_stats, c->stats.p, (size_t)nplans * RRTK_STAT_COUNT * 8, cudaMemcpyDeviceToHost, st));
     if (h_ell) RRTK_CUDA(cudaMemcpyAsync(h_ell, c->ell.p, rows * 8, cudaMemcpyDeviceToHost, st));
     RRTK_CUDA(cudaStreamSynchronize(st));
-    for (int p = 0; p < nplans; ++p)
-        if (h_stats[(size_t)p * RRTK_STAT_COUNT + RRTK_STAT2_OVERFLOW]) {
-            set_error("plan %d: a rewire-radius set exceeded the kernel's list (1024 vertices); reduce r_rewire", p);
-            return RRTK_ERR_CAPACITY;
-        }
-    return RRTK_OK;
+    return check_rewire_overflow(h_stats, nplans);
 }
+
+// K8 in the pipeline: sample headings in, rrtk_plan2_batch, the headings of the trees and path records out
+struct K8Pipe {
+    rrtk_plan2_cfg use;                         // the caller's configuration with the context's Dubins memo
+    const uint8_t *heads;                       // host sample headings, or NULL
+    uint8_t *head, *path_head;                  // host outputs: tree headings (with trees), path record headings (or NULL)
+    double *elen;                               // host output with trees
+    int reserve(const PipeCall &a, PipeSlot &s, size_t max_m)
+    {
+        const size_t rows = ((size_t)a.n + 1) * max_m;
+        RRTK_TRY(s.heads.reserve(max_m * a.n));
+        RRTK_TRY(s.head_out.reserve(rows));
+        RRTK_TRY(s.elen.reserve(rows * 8));
+        RRTK_TRY(s.scratch2.reserve(plan2_scratch_bytes((int)max_m, a.n)));
+        return a.paths ? s.phead.reserve(max_m * a.path_cap) : RRTK_OK;
+    }
+    int prepare(const PipeCall &a, PipeSlot &s, int p0, int m, cudaStream_t st)
+    {
+        if (heads) RRTK_CUDA(cudaMemcpyAsync(s.heads.p, heads + (size_t)p0 * a.n, (size_t)m * a.n, cudaMemcpyHostToDevice, st));
+        return RRTK_OK;
+    }
+    int plan(const PipeCall &a, PipeSlot &s, int m, const double *balls, cudaStream_t st)
+    {
+        use.balls = balls;
+        use.ell_c = a.ell ? s.ell.as<double>() : nullptr;
+        return rrtk_plan2_batch(&use, s.bits.as<uint32_t>(), a.W, a.H, s.plans.as<rrtk_plan_desc>(), m, a.n, s.samples.as<int16_t>(),
+                                heads ? s.heads.as<uint8_t>() : nullptr, s.pts.as<int16_t>(), s.head_out.as<uint8_t>(), s.cost.as<double>(),
+                                s.elen.as<double>(), s.parent.as<int32_t>(), s.stats.as<int64_t>(), s.scratch2.p, 0, st);
+    }
+    int paths(const PipeCall &a, PipeSlot &s, int p0, int m, cudaStream_t st)
+    {
+        if (!path_head) return RRTK_OK;
+        RRTK_TRY(path_heads_launch(s.path.as<int32_t>(), s.head_out.as<uint8_t>(), m, a.n, a.path_cap, s.phead.as<uint8_t>(), st));
+        RRTK_CUDA(cudaMemcpyAsync(path_head + (size_t)p0 * a.path_cap, s.phead.p, (size_t)m * a.path_cap, cudaMemcpyDeviceToHost, st));
+        return RRTK_OK;
+    }
+    int trees(const PipeCall &a, PipeSlot &s, int p0, int m, cudaStream_t st)
+    {
+        const size_t rows1 = (size_t)a.n + 1;
+        RRTK_CUDA(cudaMemcpyAsync(head + (size_t)p0 * rows1, s.head_out.p, rows1 * m, cudaMemcpyDeviceToHost, st));
+        RRTK_CUDA(cudaMemcpyAsync(elen + (size_t)p0 * rows1, s.elen.p, rows1 * m * 8, cudaMemcpyDeviceToHost, st));
+        return RRTK_OK;
+    }
+};
 
 // K8 from host buffers with the worlds in the same call, chunked and pipelined like rrtk_ctx_plan_worlds2
 int rrtk_ctx_plan2_worlds(rrtk_ctx *c, const rrtk_plan2_cfg *cfg, const void *h_grids, int nworlds, int W, int H, const rrtk_plan_desc *h_plans,
@@ -1429,37 +1509,9 @@ int rrtk_ctx_plan2_worlds(rrtk_ctx *c, const rrtk_plan2_cfg *cfg, const void *h_
     RRTK_TRY(check_grid_dims(W, H, 16384));
     if (nplans == 0) return RRTK_OK;
     const bool dub = cfg->model == RRTK_MODEL_DUBINS;
-    for (int p = 0; p < nplans; ++p) {
-        const rrtk_plan_desc &d = h_plans[p];
-        if (d.world < 0 || d.world >= nworlds || d.start_x < 0 || d.start_x >= W || d.goal_x < 0 || d.goal_x >= W ||
-            d.start_y < 0 || d.start_y >= H || d.goal_y < 0 || d.goal_y >= H) {
-            set_error("plan %d: world index or start/goal outside the grid", p);
-            return RRTK_ERR_INVALID;
-        }
-        if (p && d.world < h_plans[p - 1].world) {
-            set_error("rrtk_ctx_plan2_worlds: plans must be ordered by world index (plan %d)", p);
-            return RRTK_ERR_INVALID;
-        }
-        if (dub && (d.reserved[0] < 0 || d.reserved[0] >= cfg->nheadings || d.reserved[1] < 0 || d.reserved[1] >= cfg->nheadings)) {
-            set_error("plan %d: start / goal heading outside [0, %d)", p, cfg->nheadings);
-            return RRTK_ERR_INVALID;
-        }
-    }
-    const size_t total = (size_t)nplans * n;
-    if (h_samples)
-        for (size_t i = 0; i < total; ++i) {
-            const int x = h_samples[2 * i], y = h_samples[2 * i + 1];
-            if (x < 0 || x >= W || y < 0 || y >= H) {
-                set_error("sample %zu of plan %zu lies outside the grid", i % n, i / n);
-                return RRTK_ERR_INVALID;
-            }
-        }
-    if (dub && h_heads)
-        for (size_t i = 0; i < total; ++i)
-            if (h_heads[i] >= cfg->nheadings) {
-                set_error("heading of sample %zu of plan %zu outside [0, %d)", i % n, i / n, cfg->nheadings);
-                return RRTK_ERR_INVALID;
-            }
+    RRTK_TRY(check_plan_descs(h_plans, nplans, nworlds, W, H, "rrtk_ctx_plan2_worlds", dub ? cfg->nheadings : 0));
+    RRTK_TRY(check_samples(h_samples, nplans, n, W, H));
+    RRTK_TRY(check_sample_heads(dub ? h_heads : nullptr, nplans, n, cfg->nheadings));
     DevInfo *di;
     RRTK_TRY(dev_info(&di));
     if (chunk_plans <= 0) {
@@ -1467,131 +1519,20 @@ int rrtk_ctx_plan2_worlds(rrtk_ctx *c, const rrtk_plan2_cfg *cfg, const void *h_
         // plans of the chunks before it, and the first chunk is on the device after 1/16 of the uploads
         chunk_plans = di->sms;
     }
-    rrtk_plan2_cfg use = *cfg;
-    RRTK_TRY(ctx_dubins_memo(c, &use, c->stream));
-    const double *h_balls = cfg->informed ? cfg->balls : nullptr;      // host arrays in this form of the call
-    double *h_ell = cfg->informed ? cfg->ell_c : nullptr;
-    use.balls = nullptr; use.ell_c = nullptr;
-    const size_t cells = (size_t)W * H, words = grid_words(W, H), rows1 = (size_t)n + 1;
-    const size_t grid_bytes = in_bits ? words * 4 : cells;
-    std::vector<int> starts;
-    for (int p0 = 0; p0 < nplans; p0 += chunk_plans) starts.push_back(p0);
-    starts.push_back(nplans);
-    size_t max_m = 0, max_nw = 0;
-    for (size_t k = 0; k + 1 < starts.size(); ++k) {
-        const size_t m = (size_t)(starts[k + 1] - starts[k]);
-        const size_t nw = (size_t)(h_plans[starts[k + 1] - 1].world - h_plans[starts[k]].world + 1);
-        max_m = m > max_m ? m : max_m;
-        max_nw = nw > max_nw ? nw : max_nw;
-    }
-    int status = RRTK_OK;
-    auto cuda_ok = [&](cudaError_t e, const char *what) {
-        if (e != cudaSuccess && status == RRTK_OK) status = cuda_fail(e, what);
-        return e == cudaSuccess;
-    };
-    auto rrtk_ok = [&](int rc) {
-        if (rc != RRTK_OK && status == RRTK_OK) status = rc;
-        return rc == RRTK_OK;
-    };
-    if (h_state) RRTK_TRY(pipe_nfree_reserve(c, (size_t)nworlds));
-    const size_t nslots = starts.size() - 1 < (size_t)kPipeSlots ? starts.size() - 1 : (size_t)kPipeSlots;
-    for (size_t k = 0; k < nslots && status == RRTK_OK; ++k) {
-        PipeSlot &s = c->pipe[k];
-        if (!rrtk_ok(pipe_slot_init(c, s))) break;
-        bool ok = rrtk_ok(s.bits.reserve(words * 4 * max_nw)) && rrtk_ok(s.rowcum.reserve((size_t)(W + 1) * 4 * max_nw)) &&
-                  rrtk_ok(s.plans.reserve(sizeof(rrtk_plan_desc) * max_m)) && rrtk_ok(s.samples.reserve(max_m * n * 4)) &&
-                  rrtk_ok(s.state.reserve(max_m * 32)) && rrtk_ok(s.heads.reserve(max_m * n)) && rrtk_ok(s.pts.reserve(rows1 * max_m * 4)) &&
-                  rrtk_ok(s.head_out.reserve(rows1 * max_m)) && rrtk_ok(s.cost.reserve(rows1 * max_m * 8)) &&
-                  rrtk_ok(s.elen.reserve(rows1 * max_m * 8)) && rrtk_ok(s.parent.reserve(rows1 * max_m * 4)) &&
-                  rrtk_ok(s.stats.reserve(max_m * RRTK_STAT_COUNT * 8)) && rrtk_ok(s.scratch2.reserve(plan2_scratch_bytes((int)max_m, n)));
-        if (ok && !in_bits) ok = rrtk_ok(s.og.reserve(cells * max_nw));
-        if (ok && (h_balls || seed_balls)) ok = rrtk_ok(s.balls.reserve(max_m * n * 16));
-        if (ok && h_ell) ok = rrtk_ok(s.ell.reserve(rows1 * max_m * 8));
-        if (ok && out_paths)
-            ok = rrtk_ok(s.path.reserve(max_m * path_cap * 4)) && rrtk_ok(s.xy.reserve(max_m * path_cap * 4)) &&
-                 rrtk_ok(s.phead.reserve(max_m * path_cap)) && rrtk_ok(s.len.reserve(max_m * 4)) && rrtk_ok(s.pcost.reserve(max_m * 8));
-    }
-    for (size_t ci = 0; ci + 1 < starts.size() && status == RRTK_OK; ++ci) {
-        const int p0 = starts[ci], m = starts[ci + 1] - starts[ci];
-        PipeSlot &s = c->pipe[ci % kPipeSlots];
-        cudaStream_t st = c->pipe_prep;
-        if (ci >= (size_t)kPipeSlots && !cuda_ok(cudaStreamWaitEvent(st, s.done, 0), "cudaStreamWaitEvent")) break;
-        const int w0 = h_plans[p0].world, w1 = h_plans[p0 + m - 1].world, nw = w1 - w0 + 1;
-        const uint8_t *src = static_cast<const uint8_t *>(h_grids) + grid_bytes * w0;
-        if (in_bits) {
-            if (!cuda_ok(cudaMemcpyAsync(s.bits.p, src, grid_bytes * nw, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync(bits)")) break;
-        } else {
-            if (!cuda_ok(cudaMemcpyAsync(s.og.p, src, grid_bytes * nw, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync(og)")) break;
-            if (!rrtk_ok(pack_launch(s.og.as<uint8_t>(), nw, W, H, s.bits.as<uint32_t>(), st))) break;
-        }
-        s.desc.assign(h_plans + p0, h_plans + p0 + m);
-        for (rrtk_plan_desc &d : s.desc) d.world -= w0;
-        if (!cuda_ok(cudaMemcpyAsync(s.plans.p, s.desc.data(), sizeof(rrtk_plan_desc) * m, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync(plans)")) break;
-        if (h_samples) {
-            if (!cuda_ok(cudaMemcpyAsync(s.samples.p, h_samples + (size_t)p0 * n * 2, (size_t)m * n * 4, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync(samples)")) break;
-        } else {
-            if (!rrtk_ok(free_rows_launch(s.bits.as<uint32_t>(), nw, W, H, s.rowcum.as<int32_t>(), st))) break;
-            if (!cuda_ok(cudaMemcpy2DAsync(c->pin_nfree + w0, 4, s.rowcum.as<int32_t>() + W, (size_t)(W + 1) * 4, 4, nw, cudaMemcpyDeviceToHost, st),
-                           "cudaMemcpy2DAsync(nfree)")) break;
-            if (!cuda_ok(cudaMemcpyAsync(s.state.p, h_state + (size_t)p0 * 4, (size_t)m * 32, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync(state)")) break;
-            if (!rrtk_ok(sample_streams_launch(s.bits.as<uint32_t>(), s.rowcum.as<int32_t>(), W, H, s.plans.as<rrtk_plan_desc>(), m,
-                                               s.state.as<uint64_t>(), n, s.samples.as<int16_t>(), di->optin, st))) break;
-        }
-        if (h_heads && !cuda_ok(cudaMemcpyAsync(s.heads.p, h_heads + (size_t)p0 * n, (size_t)m * n, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync(heads)")) break;
-        if (h_balls && !cuda_ok(cudaMemcpyAsync(s.balls.p, h_balls + (size_t)p0 * n * 2, (size_t)m * n * 16, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync(balls)")) break;
-        if (!cuda_ok(cudaEventRecord(s.ready, st), "cudaEventRecord")) break;
-        st = s.stream;
-        if (!cuda_ok(cudaStreamWaitEvent(st, s.ready, 0), "cudaStreamWaitEvent")) break;
-        use.ell_c = h_ell ? s.ell.as<double>() : nullptr;
-        if (seed_balls) {
-            // probe (stops at the first solution vertex), then the unit-disc stream from the generator past that iteration
-            use.balls = nullptr;
-            if (!rrtk_ok(rrtk_plan2_batch(&use, s.bits.as<uint32_t>(), W, H, s.plans.as<rrtk_plan_desc>(), m, n, s.samples.as<int16_t>(),
-                                          h_heads ? s.heads.as<uint8_t>() : nullptr, s.pts.as<int16_t>(), s.head_out.as<uint8_t>(), s.cost.as<double>(),
-                                          s.elen.as<double>(), s.parent.as<int32_t>(), s.stats.as<int64_t>(), s.scratch2.p, 0, st))) break;
-            if (!rrtk_ok(ball_streams_launch(s.rowcum.as<int32_t>(), W, s.plans.as<rrtk_plan_desc>(), m, n, s.state.as<uint64_t>(), nullptr,
-                                             s.stats.as<int64_t>() + RRTK_STAT2_FIRST_SOL, RRTK_STAT_COUNT, s.balls.as<double>(), nullptr,
-                                             nullptr, st))) break;
-        }
-        use.balls = (h_balls || seed_balls) ? s.balls.as<double>() : nullptr;
-        if (!rrtk_ok(rrtk_plan2_batch(&use, s.bits.as<uint32_t>(), W, H, s.plans.as<rrtk_plan_desc>(), m, n, s.samples.as<int16_t>(),
-                                      h_heads ? s.heads.as<uint8_t>() : nullptr, s.pts.as<int16_t>(), s.head_out.as<uint8_t>(), s.cost.as<double>(),
-                                      s.elen.as<double>(), s.parent.as<int32_t>(), s.stats.as<int64_t>(), s.scratch2.p, 0, st))) break;
-        if (!cuda_ok(cudaEventRecord(s.planned, st), "cudaEventRecord")) break;
-        st = c->pipe_post;
-        if (!cuda_ok(cudaStreamWaitEvent(st, s.planned, 0), "cudaStreamWaitEvent")) break;
-        bool ok = true;
-        if (out_paths) {
-            ok = rrtk_ok(paths_xy_launch(s.parent.as<int32_t>(), s.pts.as<int16_t>(), s.cost.as<double>(), s.stats.as<int64_t>(), m, n, path_cap,
-                                         s.path.as<int32_t>(), s.xy.as<int16_t>(), s.len.as<int32_t>(), s.pcost.as<double>(), st)) &&
-                 cuda_ok(cudaMemcpyAsync(h_path + (size_t)p0 * path_cap, s.path.p, (size_t)m * path_cap * 4, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(path)") &&
-                 cuda_ok(cudaMemcpyAsync(h_xy + (size_t)p0 * path_cap * 2, s.xy.p, (size_t)m * path_cap * 4, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(xy)") &&
-                 cuda_ok(cudaMemcpyAsync(h_len + p0, s.len.p, (size_t)m * 4, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(len)") &&
-                 cuda_ok(cudaMemcpyAsync(h_path_cost + p0, s.pcost.p, (size_t)m * 8, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(path_cost)");
-            if (ok && h_path_head)
-                ok = rrtk_ok(path_heads_launch(s.path.as<int32_t>(), s.head_out.as<uint8_t>(), m, n, path_cap, s.phead.as<uint8_t>(), st)) &&
-                     cuda_ok(cudaMemcpyAsync(h_path_head + (size_t)p0 * path_cap, s.phead.p, (size_t)m * path_cap, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(path_head)");
-        }
-        if (ok && out_trees)
-            ok = cuda_ok(cudaMemcpyAsync(h_pts + (size_t)p0 * rows1 * 2, s.pts.p, rows1 * m * 4, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(pts)") &&
-                 cuda_ok(cudaMemcpyAsync(h_head + (size_t)p0 * rows1, s.head_out.p, rows1 * m, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(head)") &&
-                 cuda_ok(cudaMemcpyAsync(h_cost + (size_t)p0 * rows1, s.cost.p, rows1 * m * 8, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(cost)") &&
-                 cuda_ok(cudaMemcpyAsync(h_elen + (size_t)p0 * rows1, s.elen.p, rows1 * m * 8, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(elen)") &&
-                 cuda_ok(cudaMemcpyAsync(h_parent + (size_t)p0 * rows1, s.parent.p, rows1 * m * 4, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(parent)");
-        if (ok && h_ell) ok = cuda_ok(cudaMemcpyAsync(h_ell + (size_t)p0 * rows1, s.ell.p, rows1 * m * 8, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(ell)");
-        if (ok) cuda_ok(cudaMemcpyAsync(h_stats + (size_t)p0 * RRTK_STAT_COUNT, s.stats.p, (size_t)m * RRTK_STAT_COUNT * 8, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(stats)");
-        cuda_ok(cudaEventRecord(s.done, st), "cudaEventRecord");
-    }
-    pipe_drain(c, &status);
-    if (status != RRTK_OK) return status;
-    if (h_state) RRTK_TRY(pipe_require_free_cells(c, h_plans, nplans, "rrtk_ctx_plan2_worlds"));
-    if (seed_balls) RRTK_TRY(pipe_require_rotations(h_plans, h_stats, nplans, RRTK_STAT2_FIRST_SOL, "rrtk_ctx_plan2_worlds"));
-    for (int p = 0; p < nplans; ++p)
-        if (h_stats[(size_t)p * RRTK_STAT_COUNT + RRTK_STAT2_OVERFLOW]) {
-            set_error("plan %d: a rewire-radius set exceeded the kernel's list (1024 vertices); reduce r_rewire", p);
-            return RRTK_ERR_CAPACITY;
-        }
-    return RRTK_OK;
+    K8Pipe f = {*cfg, h_heads, h_head, h_path_head, h_elen};
+    RRTK_TRY(ctx_dubins_memo(c, &f.use, c->stream));
+    PipeCall a = {};
+    a.who = "rrtk_ctx_plan2_worlds";
+    a.grids = h_grids; a.nworlds = nworlds; a.W = W; a.H = H;
+    a.plans = h_plans; a.nplans = nplans; a.n = n;
+    a.samples = h_samples; a.state = h_state; a.balls = cfg->informed ? cfg->balls : nullptr;     // host arrays in this form of the call
+    a.in_bits = in_bits; a.trees = out_trees; a.paths = out_paths; a.seed_balls = seed_balls;
+    a.ell_c = cfg->informed ? cfg->ell_c : nullptr; a.ell = a.ell_c != nullptr; a.first_col = RRTK_STAT2_FIRST_SOL;
+    a.pts = h_pts; a.cost = h_cost; a.parent = h_parent;
+    a.path_cap = path_cap; a.path = h_path; a.xy = h_xy; a.len = h_len; a.path_cost = h_path_cost;
+    a.stats = h_stats;
+    RRTK_TRY(pipe_run(c, a, chunk_plans, chunk_plans, f));
+    return check_rewire_overflow(h_stats, nplans);
 }
 
 int rrtk_ctx_dubins_paths(rrtk_ctx *c, const int32_t *h_q, int64_t nq, int nheadings, double rho, int32_t *h_word, double *h_tpq,
