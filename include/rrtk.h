@@ -123,6 +123,21 @@ int rrtk_gen_worlds(const int32_t *d_seeds, int nworlds, int W, int H, int thres
 int rrtk_inflate_grid(const uint32_t *d_bits, int nworlds, int W, int H, int iterations, const int32_t *d_holes,
                       int nout, uint32_t *d_out, uint32_t *d_scratch, void *stream);
 
+/* Configuration space of a disc-shaped robot: output grid o (o < nout) is source world d_src[o] with every cell (x, y) set for
+ * which some obstacle cell (u, v) INSIDE the grid has (x - u)^2 + (y - v)^2 <= d_r2[o] (distances between cell indices).  That
+ * is scipy.ndimage.binary_dilation(og != 0, structure = {(i, j): i^2 + j^2 <= r2}, border_value = 0): cells outside the grid
+ * are free, an obstacle-free world stays free, r2 = 0 returns the grid.  For a robot radius rho >= 0 in cells the caller passes
+ * r2 = floor(rho * rho) computed in double and clamped to INT32_MAX, so the test d^2 <= r2 equals d^2 <= rho^2 (EDT <= rho).
+ * Outputs are ordinary tiled bit grids (padding bits set) and feed the planners unchanged; one launch can mix radii and reuse
+ * a world at several.  Exact separable distance transform, time independent of r2 (csrc/disc.cu).
+ *   d_src, d_r2   DEVICE int32 per output; an output whose d_src is outside [0, nworlds) or whose d_r2 < 0 is left unwritten
+ *                 (rrtk_ctx_inflate_disc rejects both)
+ *   d_scratch     rrtk_inflate_disc_scratch_bytes(nworlds, W, H) bytes (2 per cell of every source world)
+ * d_out holds nout grids; neither d_out nor d_scratch may alias d_bits.  W, H <= 32768. */
+size_t rrtk_inflate_disc_scratch_bytes(int nworlds, int W, int H);
+int rrtk_inflate_disc(const uint32_t *d_bits, int nworlds, int W, int H, const int32_t *d_src, const int32_t *d_r2, int nout,
+                      uint32_t *d_out, void *d_scratch, void *stream);
+
 /* ---- K1: RRT.collisionfree (rrt.py:183-229), batched ------------------------------------------- */
 /* d_segs: nseg x (ax, ay, bx, by) int32, all points inside the grid.  d_world: optional per-segment
  * world index (NULL = world 0).  d_free[s] = 1 iff the walk a->b meets no obstacle (both ends
@@ -401,6 +416,13 @@ int rrtk_ctx_set_grids(rrtk_ctx *ctx, const uint8_t *h_og, int nworlds, int W, i
  * grids (one per hole triple in h_holes, or a single one without holes when h_holes is NULL and nout = 1) */
 int rrtk_ctx_inflate(rrtk_ctx *ctx, const uint8_t *h_og, int W, int H, int iterations, const int32_t *h_holes, int nout,
                      uint8_t *h_out);
+
+/* host-buffer form of rrtk_inflate_disc: h_og holds nworlds (W, H) uint8 grids (non-zero = obstacle), h_src / h_r2 one source
+ * world and one r2 = floor(rho * rho) per output (same contract as above; RRTK_ERR_INVALID for a source outside [0, nworlds) or
+ * r2 < 0, before any device work).  h_out receives nout packed grids of rrtk_grid_words(W, H) uint32 each, the layout of
+ * rrtk_pack_grid_host, so they feed RRTK_IN_BITS directly.  W, H <= 16384. */
+int rrtk_ctx_inflate_disc(rrtk_ctx *ctx, const uint8_t *h_og, int nworlds, int W, int H, const int32_t *h_src, const int32_t *h_r2,
+                          int nout, uint32_t *h_out);
 
 /* full plan() from host memory: H2D of descriptors (+ samples / balls / PCG64 states), K7, D2H of
  * the trees.  Exactly one of h_samples / h_state must be non-NULL (explicit stream vs. seed mode).

@@ -68,6 +68,8 @@ SIGNATURES = {
     "rrtk_unpack_grid": (_i, [_vp, _i, _i, _i, _vp, _vp]),
     "rrtk_inflate_grid": (_i, [_vp, _i, _i, _i, _i, _vp, _i, _vp, _vp, _vp]),
     "rrtk_free_rows": (_i, [_vp, _i, _i, _i, _vp, _vp]),
+    "rrtk_inflate_disc_scratch_bytes": (_sz, [_i, _i, _i]),
+    "rrtk_inflate_disc": (_i, [_vp, _i, _i, _i, _vp, _vp, _i, _vp, _vp, _vp]),
     "rrtk_gen_worlds": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _vp]),
     "rrtk_collision_segments": (_i, [_vp, _i, _i, _vp, _vp, _i64, _vp, _vp, _vp]),
     "rrtk_clearance_field": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _vp]),
@@ -97,6 +99,7 @@ SIGNATURES = {
     "rrtk_destroy": (_i, [_vp]),
     "rrtk_ctx_set_grids": (_i, [_vp, _vp, _i, _i, _i, _vp]),
     "rrtk_ctx_inflate": (_i, [_vp, _vp, _i, _i, _i, _vp, _i, _vp]),
+    "rrtk_ctx_inflate_disc": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _i, _vp]),
     "rrtk_ctx_plan": (_i, [_vp, _i, _vp, _i, _i, _d, _d, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "rrtk_ctx_plan_worlds": (_i, [_vp, _i, _vp, _i, _i, _i, _vp, _i, _i, _d, _d, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i]),
     "rrtk_ctx_plan_worlds2": (_i, [_vp, _i, _vp, _i, _i, _i, _vp, _i, _i, _d, _d, _vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp,
@@ -157,6 +160,28 @@ def pack_grids_host(ogs) -> np.ndarray:
     bits = np.empty((nw, int(lib().rrtk_grid_words(W, H))), dtype=np.uint32)
     check(lib().rrtk_pack_grid_host(ptr(og), nw, W, H, ptr(bits)), "rrtk_pack_grid_host")
     return bits
+
+
+INT32_MAX = 2 ** 31 - 1
+
+
+def disc_r2(radius):
+    """Squared-distance threshold of a disc robot of radius ``radius`` cells (scalar or array): ``floor(radius * radius)`` in
+    float64, clamped to INT32_MAX, as int32.  A cell is blocked iff its squared distance d^2 (an integer) to an obstacle cell is
+    <= this, which equals d^2 <= radius^2.  Raises ValueError for a negative, NaN or infinite radius."""
+    r = np.asarray(radius, dtype=np.float64)
+    if not np.isfinite(r).all() or (r < 0).any():
+        raise ValueError("robot_radius must be a finite number >= 0 (cells)")
+    with np.errstate(over="ignore"):
+        return np.minimum(np.floor(r * r), INT32_MAX).astype(np.int32)
+
+
+def unpack_grids_host(bits, W: int, H: int) -> np.ndarray:
+    """Inverse of pack_grids_host: (nworlds, rrtk_grid_words(W, H)) uint32 tiled bit grids -> (nworlds, W, H) uint8 of 0 / 1."""
+    TX, TY = (W + 31) // 32, (H + 31) // 32
+    b = np.ascontiguousarray(bits, dtype="<u4").reshape(-1, TX, TY, 32)                 # [world, tx, ty, x & 31]
+    cells = np.unpackbits(b.view(np.uint8).reshape(*b.shape, 4), axis=-1, bitorder="little")   # [..., y & 31]
+    return cells.transpose(0, 1, 3, 2, 4).reshape(b.shape[0], TX * 32, TY * 32)[:, :W, :H].copy()
 
 
 def check(rc: int, what: str = ""):
@@ -323,6 +348,23 @@ class Context:
         nout = 1 if h is None else h.shape[0]
         out = np.empty((nout, W, H), dtype=np.uint8)
         check(lib().rrtk_ctx_inflate(self._h, ptr(og_u8), W, H, int(iterations), ptr(h), nout, ptr(out)), "rrtk_ctx_inflate")
+        return out
+
+    def inflate_disc(self, og_u8: np.ndarray, src, r2) -> np.ndarray:
+        """Configuration-space grids of a disc robot (rrtk_ctx_inflate_disc): ``og_u8`` (nworlds, W, H), non-zero = obstacle;
+        output o blocks every cell within squared distance ``r2[o]`` (``disc_r2(radius)``) of an obstacle cell of world
+        ``src[o]``.  Returns (nout, rrtk_grid_words(W, H)) uint32 tiled bit grids, the form ``plan_worlds2(bits=True)`` takes."""
+        og_u8 = np.ascontiguousarray(og_u8, dtype=np.uint8)
+        if og_u8.ndim != 3:
+            raise ValueError("og_u8 must have shape (nworlds, W, H)")
+        nw, W, H = og_u8.shape
+        src = np.ascontiguousarray(src, dtype=np.int32).reshape(-1)
+        r2 = np.ascontiguousarray(r2, dtype=np.int32).reshape(-1)
+        if src.shape != r2.shape:
+            raise ValueError("src and r2 need one entry per output")
+        out = np.empty((src.shape[0], int(lib().rrtk_grid_words(W, H))), dtype=np.uint32)
+        check(lib().rrtk_ctx_inflate_disc(self._h, ptr(og_u8), nw, W, H, ptr(src), ptr(r2), src.shape[0], ptr(out)),
+              "rrtk_ctx_inflate_disc")
         return out
 
     # -- K8: rewire / Dubins planners, Dubins primitive ---------------------------------------

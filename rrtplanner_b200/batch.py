@@ -175,7 +175,7 @@ class BatchResult:
 
 
 def plan_batch(kind, ogs, n, starts, goals, world_ids=None, r_rewire=0.0, r_goal=0.0, samples=None, seeds=None,
-               balls=None, rots=None, ctx: Optional[_lib.Context] = None) -> BatchResult:
+               balls=None, rots=None, ctx: Optional[_lib.Context] = None, robot_radius=None) -> BatchResult:
     """End-to-end batched plan() from host arrays through ``rrtk_ctx_plan_worlds``.
 
     ogs: (nworlds, W, H) array, non-zero = obstacle.  Either ``samples`` (P, n, 2) -- the explicit
@@ -194,6 +194,11 @@ def plan_batch(kind, ogs, n, starts, goals, world_ids=None, r_rewire=0.0, r_goal
     device runs a probe to each plan's first solution vertex and draws the unit-disc stream past it (RRTK_SEED_BALLS of
     ``rrtk_ctx_plan_worlds2``), so nothing per iteration is uploaded.  ``rots`` defaults to ``informed_rotations``; a plan
     with start == goal that reaches the ellipse phase raises ``np.linalg.LinAlgError``, as the class does.
+
+    ``robot_radius`` (a number, or one per plan; None = point robot): plan p runs on the configuration-space grid of a disc of
+    that radius in its world (``rrtk_inflate_disc``), i.e. it is what the planner class built with ``robot_radius`` computes.
+    Each distinct (world, floor(radius^2)) pair is inflated once on the device, the packed grids come back once (1 bit per
+    cell) and the plans run through ``rrtk_ctx_plan_worlds2`` on them.
     """
     k = KINDS[kind] if isinstance(kind, str) else int(kind)
     seed_balls = isinstance(balls, str)
@@ -216,33 +221,47 @@ def plan_batch(kind, ogs, n, starts, goals, world_ids=None, r_rewire=0.0, r_goal
         raise ValueError("balls='seed' needs one seed per plan")
     if world_ids is None:
         world_ids = np.arange(nplans) % ogs.shape[0]
+    r2 = None
+    if robot_radius is not None:
+        r2 = _lib.disc_r2(robot_radius)
+        if r2.ndim == 0:
+            r2 = np.full(nplans, r2, dtype=np.int32)
+        elif r2.shape != (nplans,):
+            raise ValueError("robot_radius must be a number or hold one value per plan")
     own = ctx is None
     ctx = ctx or _lib.Context()
     try:
         og_u8 = ogs if ogs.dtype == np.uint8 else (ogs != 0).astype(np.uint8)
-        desc = make_desc(world_ids, starts, goals, rots)
+        grids = og_u8
+        if r2 is not None:
+            # one configuration-space grid per distinct (world, r2) pair; the plans then index those grids
+            pairs, world_ids = np.unique(np.stack([np.asarray(world_ids, dtype=np.int64).reshape(nplans), r2.astype(np.int64)], axis=1),
+                                         axis=0, return_inverse=True)
+            grids = ctx.inflate_disc(og_u8, pairs[:, 0], pairs[:, 1])
+        desc = make_desc(np.asarray(world_ids).reshape(nplans), starts, goals, rots)
         states = None if seeds is None else seed_states(seeds)
         order = np.argsort(desc["world"], kind="stable")          # the pipelined call wants plans grouped by world
         sorted_ = bool((np.diff(desc["world"]) >= 0).all())
         if sorted_:
             order = np.arange(nplans)
-        if seed_balls:
+        take = lambda a: None if a is None else np.asarray(a)[order]          # noqa: E731
+        if seed_balls or r2 is not None:
             d = desc[order]
             stats = np.empty((nplans, _lib.STAT_COUNT), dtype=np.int64)
             try:
-                o = ctx.plan_worlds2(k, og_u8, og_u8.shape[1], og_u8.shape[2], d, n, r_rewire, r_goal, states=states[order],
-                                     trees=True, paths=False, seed_balls=True, out={"stats": stats})
+                o = ctx.plan_worlds2(k, grids, og_u8.shape[1], og_u8.shape[2], d, n, r_rewire, r_goal, samples=take(samples),
+                                     states=take(states), balls=None if seed_balls else take(balls), bits=r2 is not None,
+                                     trees=True, paths=False, seed_balls=seed_balls, out={"stats": stats})
             except ValueError as e:
                 bad = (stats[:, 5] >= 0) & ~np.isfinite(d["rot"]).all(axis=1)
                 if "start == goal" not in str(e) or not bad.any():
                     raise
                 raise np.linalg.LinAlgError(f"plan {int(order[np.argmax(bad)])}: start == goal, so the ellipse of the informed phase "
                                             "has no axis (rotation_to_world_frame, rrt.py:601-613)") from None
-            res = (o["pts"], o["cost"], o["parent"], o["stats"], o["ell"])
+            res = (o["pts"], o["cost"], o["parent"], o["stats"], o.get("ell"))
         elif sorted_:
             res = ctx.plan_worlds(k, og_u8, desc, n, r_rewire, r_goal, samples=samples, states=states, balls=balls)
         else:
-            take = lambda a: None if a is None else np.asarray(a)[order]          # noqa: E731
             res = ctx.plan_worlds(k, og_u8, desc[order], n, r_rewire, r_goal, samples=take(samples), states=take(states),
                                   balls=take(balls))
         if sorted_:
@@ -358,6 +377,30 @@ class DeviceBatch:
                 _lib.check(self.L.rrtk_gen_worlds(self._p(d_seeds[lo:]), m, self.W, self.H, int(round(thresh * 1000)),
                                                   self._p(scratch), self._p(og[lo:]), self._stream()), "gen_worlds")
         return self.set_worlds_u8(og)
+
+    def inflate_disc(self, radius):
+        """Replace every world by its configuration-space grid for a disc robot of ``radius`` cells (a number, or one per world),
+        on the device and on torch's current stream: ``bits`` then blocks every cell within squared distance
+        ``floor(radius^2)`` of an obstacle cell (rrtk_inflate_disc) and ``rowcum`` is rebuilt from it (rrtk_free_rows), so every
+        later sampler, plan, path and shortcut call of the batch sees the inflated grid.  ``og`` keeps the worlds as given.
+        Returns self."""
+        t = self.torch
+        nw = int(self.bits.shape[0])
+        r2 = _lib.disc_r2(radius)
+        if r2.ndim == 0:
+            r2 = np.full(nw, r2, dtype=np.int32)
+        elif r2.shape != (nw,):
+            raise ValueError("radius must be a number or hold one value per world")
+        d_r2 = t.from_numpy(np.ascontiguousarray(r2)).to(self.dev)
+        d_src = t.arange(nw, dtype=t.int32, device=self.dev)
+        scratch = self._empty((int(self.L.rrtk_inflate_disc_scratch_bytes(nw, self.W, self.H)),), t.uint8)
+        bits = self._empty((nw, self.words), t.int32)
+        with t.cuda.device(self.dev):
+            _lib.check(self.L.rrtk_inflate_disc(self._p(self.bits), nw, self.W, self.H, self._p(d_src), self._p(d_r2), nw, self._p(bits),
+                                                self._p(scratch), self._stream()), "inflate_disc")
+            _lib.check(self.L.rrtk_free_rows(self._p(bits), nw, self.W, self.H, self._p(self.rowcum), self._stream()), "free_rows")
+        self.bits = bits
+        return self
 
     def nfree(self) -> np.ndarray:
         return self.rowcum[:, self.W].cpu().numpy()

@@ -38,6 +38,8 @@ int clearance_dir16_launch(const uint32_t *, int, int, int, int, uint8_t *, cuda
 int collision_cf_launch(const uint8_t *, int, int, const int32_t *, const int32_t *, int, int64_t, uint8_t *, int32_t *, int, cudaStream_t);
 int unpack_launch(const uint32_t *, int, int, int, uint8_t *, cudaStream_t);
 int inflate_launch(const uint32_t *, int, int, int, int, const int32_t *, int, uint32_t *, uint32_t *, cudaStream_t);
+int disc_launch(const uint32_t *, int, int, int, const int32_t *, const int32_t *, int, uint32_t *, void *, cudaStream_t);
+size_t disc_scratch_bytes(int, int, int);
 int nearest_launch(const int32_t *, int, const int32_t *, const int32_t *, int, int32_t *, int64_t *, cudaStream_t);
 int nearest_launch_f64(const double *, int, const double *, const int32_t *, int, int32_t *, double *, cudaStream_t);
 int within_launch(const int32_t *, int, const int32_t *, const int32_t *, int, double, int, int32_t *, int32_t *, cudaStream_t);
@@ -524,6 +526,24 @@ int rrtk_inflate_grid(const uint32_t *d_bits, int nworlds, int W, int H, int ite
     return inflate_launch(d_bits, nworlds, W, H, iterations, d_holes, nout, d_out, d_scratch, (cudaStream_t)stream);
 }
 
+size_t rrtk_inflate_disc_scratch_bytes(int nworlds, int W, int H)
+{
+    return (nworlds < 1 || W < 1 || H < 1 || W > 32768 || H > 32768) ? 0 : disc_scratch_bytes(nworlds, W, H);
+}
+
+int rrtk_inflate_disc(const uint32_t *d_bits, int nworlds, int W, int H, const int32_t *d_src, const int32_t *d_r2, int nout,
+                      uint32_t *d_out, void *d_scratch, void *stream)
+{
+    RRTK_REQUIRE(nworlds >= 0 && nout >= 0, "rrtk_inflate_disc: negative count");
+    RRTK_TRY(check_grid_dims(W, H, 32768));
+    if (nout == 0) return RRTK_OK;
+    RRTK_REQUIRE(nworlds >= 1, "rrtk_inflate_disc: nout > 0 needs at least one source world");
+    RRTK_REQUIRE(d_bits && d_src && d_r2 && d_out && d_scratch, "rrtk_inflate_disc: null pointer");
+    RRTK_REQUIRE((const void *)d_out != (const void *)d_bits && d_scratch != (void *)d_bits && d_scratch != (void *)d_out,
+                 "rrtk_inflate_disc: buffers must not alias");
+    return disc_launch(d_bits, nworlds, W, H, d_src, d_r2, nout, d_out, d_scratch, (cudaStream_t)stream);
+}
+
 int rrtk_free_rows(const uint32_t *d_bits, int nworlds, int W, int H, int32_t *d_rowcum, void *stream)
 {
     RRTK_REQUIRE(d_bits && d_rowcum && nworlds >= 0, "rrtk_free_rows: null pointer or negative count");
@@ -856,6 +876,42 @@ int rrtk_ctx_inflate(rrtk_ctx *c, const uint8_t *h_og, int W, int H, int iterati
     RRTK_TRY(unpack_launch(c->c.as<uint32_t>(), nout, W, H, c->a.as<uint8_t>(), c->stream));
     RRTK_CUDA(cudaMemcpyAsync(h_out, c->a.p, cells * nout, cudaMemcpyDeviceToHost, c->stream));
     RRTK_CUDA(cudaStreamSynchronize(c->stream));
+    return RRTK_OK;
+}
+
+int rrtk_ctx_inflate_disc(rrtk_ctx *c, const uint8_t *h_og, int nworlds, int W, int H, const int32_t *h_src, const int32_t *h_r2, int nout,
+                          uint32_t *h_out)
+{
+    RRTK_REQUIRE(c && nworlds >= 0 && nout >= 0, "rrtk_ctx_inflate_disc: bad argument");
+    RRTK_TRY(check_grid_dims(W, H, 16384));
+    if (nout == 0) return RRTK_OK;
+    RRTK_REQUIRE(h_og && h_src && h_r2 && h_out, "rrtk_ctx_inflate_disc: null pointer");
+    for (int o = 0; o < nout; ++o) {
+        if (h_src[o] < 0 || h_src[o] >= nworlds) {
+            set_error("rrtk_ctx_inflate_disc: output %d names source world %d, outside [0, %d)", o, h_src[o], nworlds);
+            return RRTK_ERR_INVALID;
+        }
+        if (h_r2[o] < 0) {
+            set_error("rrtk_ctx_inflate_disc: output %d has r2 = %d < 0", o, h_r2[o]);
+            return RRTK_ERR_INVALID;
+        }
+    }
+    const size_t cells = (size_t)W * H, wb = grid_words(W, H) * 4;
+    // scratch buffers of the context: a = source uint8, b = source bits, c = result bits, d = row distances, e = src / r2
+    RRTK_TRY(c->a.reserve(cells * nworlds));
+    RRTK_TRY(c->b.reserve(wb * nworlds));
+    RRTK_TRY(c->c.reserve(wb * nout));
+    RRTK_TRY(c->d.reserve(disc_scratch_bytes(nworlds, W, H)));
+    RRTK_TRY(c->e.reserve((size_t)nout * 8));
+    cudaStream_t st = c->stream;
+    RRTK_CUDA(cudaMemcpyAsync(c->a.p, h_og, cells * nworlds, cudaMemcpyHostToDevice, st));
+    RRTK_CUDA(cudaMemcpyAsync(c->e.p, h_src, (size_t)nout * 4, cudaMemcpyHostToDevice, st));
+    RRTK_CUDA(cudaMemcpyAsync(c->e.as<int32_t>() + nout, h_r2, (size_t)nout * 4, cudaMemcpyHostToDevice, st));
+    RRTK_TRY(pack_launch(c->a.as<uint8_t>(), nworlds, W, H, c->b.as<uint32_t>(), st));
+    RRTK_TRY(disc_launch(c->b.as<uint32_t>(), nworlds, W, H, c->e.as<int32_t>(), c->e.as<int32_t>() + nout, nout, c->c.as<uint32_t>(),
+                         c->d.p, st));
+    RRTK_CUDA(cudaMemcpyAsync(h_out, c->c.p, wb * nout, cudaMemcpyDeviceToHost, st));
+    RRTK_CUDA(cudaStreamSynchronize(st));
     return RRTK_OK;
 }
 

@@ -10,7 +10,9 @@ oracle/rewire_oracle.c (parity UNPINNED: it is this project's own definition).
 
 Model: a configuration is ``(x, y, h)`` -- an integer grid cell and a heading index ``h`` in ``[0, nheadings)``,
 heading angle ``h * 2 pi / nheadings`` measured from the +x axis towards +y.  Edges are shortest Dubins paths
-(turning radius ``rho`` cells) checked against the grid at points every ``ds`` cells of arc length.  Nearest and
+(turning radius ``rho`` cells) checked against the grid at points every ``ds`` cells of arc length.  ``robot_radius``
+(keyword-only) plans for a disc-shaped vehicle on the configuration-space grid, as for the planners of rrt.py; the footprint
+does not depend on the heading.  Nearest and
 rewire-radius queries are Euclidean on ``(x, y)`` exactly as in the reference's planners.
 """
 from __future__ import annotations
@@ -85,8 +87,8 @@ class RRTDubins(RRT):
     _STAR = False
 
     def __init__(self, og: np.ndarray, n: int, rho: float, nheadings: int = 16, ds: float = 1.0, costfn: callable = None,
-                 pbar: bool = True, seed: int = 0):
-        super().__init__(og, n, costfn=costfn, pbar=pbar, seed=seed)
+                 pbar: bool = True, seed: int = 0, *, robot_radius=None):
+        super().__init__(og, n, costfn=costfn, pbar=pbar, seed=seed, robot_radius=robot_radius)
         if not (0 < rho <= 16384 and 0.05 <= ds <= 16384):
             raise ValueError("need 0 < rho <= 16384 and 0.05 <= ds <= 16384 (cells)")
         if not (1 <= int(nheadings) <= 255):
@@ -176,7 +178,7 @@ class RRTStarDubins(RRTDubins):
     _STAR = True
 
     def __init__(self, og: np.ndarray, n: int, r_rewire: float, rho: float, nheadings: int = 16, ds: float = 1.0,
-                 costfn: callable = None, pbar: bool = True, seed: int = 0, *, rewire: bool = True):
-        super().__init__(og, n, rho, nheadings=nheadings, ds=ds, costfn=costfn, pbar=pbar, seed=seed)
+                 costfn: callable = None, pbar: bool = True, seed: int = 0, *, rewire: bool = True, robot_radius=None):
+        super().__init__(og, n, rho, nheadings=nheadings, ds=ds, costfn=costfn, pbar=pbar, seed=seed, robot_radius=robot_radius)
         self.r_rewire = r_rewire
         self.rewire = bool(rewire)

@@ -18,6 +18,13 @@ section 0):
 * the grid is copied to the device in ``__init__`` / ``set_og``; later in-place edits of the
   caller's array are not seen until ``set_og`` is called again (the reference holds ``og`` by
   reference, rrt.py:65).
+* ``robot_radius`` (keyword-only, not in the reference): plan for a disc of that radius in cells instead of a point.  The
+  planner works on the configuration-space grid, which blocks every cell within squared distance ``floor(radius^2)`` of an
+  obstacle cell of ``og`` (csrc/disc.cu, rrtk_inflate_disc); a plan is by definition the same plan on that grid, so the tree
+  equals what the class builds when constructed on the inflated grid with the same seed.  ``self.og`` stays the caller's
+  object; ``self.free``, the device grid, ``go2goal`` and ``shortcut_path`` use the inflated grid, ``set_og`` inflates again,
+  the static ``collisionfree`` is unchanged.  A start or goal inside the inflated obstacles behaves as an occupied one does:
+  no growth from the root, or the goal is not found.  ``None`` (default) and radii below 1 (r2 = 0) leave the grid as it is.
 * points must be integer arrays inside the grid (the reference's Numba kernel rejects float
   points with a TypingError and reads out of bounds for outside points); grids up to
   16384 x 16384, n <= 65534.
@@ -77,14 +84,20 @@ class RRT(object):
 
     _KIND = None
 
-    def __init__(self, og: np.ndarray, n: int, costfn: callable = None, pbar: bool = True, seed: int = 0):
+    def __init__(self, og: np.ndarray, n: int, costfn: callable = None, pbar: bool = True, seed: int = 0, *, robot_radius=None):
         if costfn is not None:
             raise NotImplementedError(
                 "custom cost functions are Python callables and cannot run on the device; "
                 "rrtplanner_b200 has no CPU fallback (pass costfn=None)")
         self.pbar = pbar
         self.n = n
-        self.free = np.argwhere(og == 0)
+        self.robot_radius = robot_radius
+        if robot_radius is not None and np.ndim(robot_radius) != 0:
+            raise ValueError("robot_radius must be a number (cells)")
+        self._r2 = None if robot_radius is None else int(_lib.disc_r2(robot_radius))
+        self._ctx = None
+        self._cspace = self._inflate(og)
+        self.free = np.argwhere((og if self._cspace is None else self._cspace) == 0)
         self.og = og
 
         def costfn(vcosts, points, v, x):
@@ -94,7 +107,6 @@ class RRT(object):
         self.not_a_point = [np.inf, np.inf]
         self.not_a_dist = np.inf
         self.rand_gen = np.random.default_rng(seed)
-        self._ctx = None
         self._dirty = True
 
     # ---- device state ------------------------------------------------------------------------
@@ -106,9 +118,23 @@ class RRT(object):
             og = np.asarray(self.og)
             if og.ndim != 2:
                 raise ValueError("og must be a 2-D occupancy grid")
-            self._ctx.set_grids((og != 0).astype(np.uint8)[None])
+            self._ctx.set_grids(((og != 0).astype(np.uint8) if self._cspace is None else self._cspace)[None])
             self._dirty = False
         return self._ctx
+
+    def _inflate(self, og):
+        """The configuration-space grid of ``og`` for ``robot_radius`` as (W, H) uint8 of 0 / 1, or None when nothing is
+        inflated (no radius, or r2 = 0).  Inflated on the device, downloaded packed (1 bit per cell)."""
+        if not self._r2:
+            return None
+        og = np.asarray(og)
+        if og.ndim != 2:
+            raise ValueError("og must be a 2-D occupancy grid")
+        if self._ctx is None:
+            self._ctx = _lib.Context()
+            self._dirty = True
+        bits = self._ctx.inflate_disc((og != 0).astype(np.uint8)[None], [0], [self._r2])
+        return _lib.unpack_grids_host(bits, *og.shape)[0]
 
     # ---- graph helpers (host, rrt.py:87-129) -----------------------------------------------------
     def route2gv(self, T: nx.DiGraph, gv) -> List[int]:
@@ -199,7 +225,8 @@ class RRT(object):
     def set_og(self, og_new: np.ndarray):
         """New occupancy grid: refresh free space (rrt.py:261-272) and the device copy."""
         self.og = og_new
-        self.free = np.argwhere(og_new == 0)
+        self._cspace = self._inflate(og_new)
+        self.free = np.argwhere((og_new if self._cspace is None else self._cspace) == 0)
         self._dirty = True
 
     def set_n(self, n: int):
@@ -327,8 +354,8 @@ class RRTStandard(RRT):
 
     _KIND = _lib.KIND_STANDARD
 
-    def __init__(self, og: np.ndarray, n: int, costfn: callable = None, pbar=True, seed: int = 0):
-        super().__init__(og, n, costfn=costfn, pbar=pbar, seed=seed)
+    def __init__(self, og: np.ndarray, n: int, costfn: callable = None, pbar=True, seed: int = 0, *, robot_radius=None):
+        super().__init__(og, n, costfn=costfn, pbar=pbar, seed=seed, robot_radius=robot_radius)
 
     def plan(self, xstart: np.ndarray, xgoal: np.ndarray) -> Tuple[nx.DiGraph, int]:
         self._check_hooks()
@@ -354,8 +381,8 @@ class RRTStar(RRT):
     _KIND = _lib.KIND_STAR
 
     def __init__(self, og: np.ndarray, n: int, r_rewire: float, costfn: callable = None, pbar=True, seed: int = 0, *,
-                 rewire: str = "reference"):
-        super().__init__(og, n, costfn=costfn, pbar=pbar, seed=seed)
+                 rewire: str = "reference", robot_radius=None):
+        super().__init__(og, n, costfn=costfn, pbar=pbar, seed=seed, robot_radius=robot_radius)
         self.r_rewire = r_rewire
         if rewire not in ("reference", "rrtstar"):
             raise ValueError("rewire must be 'reference' or 'rrtstar'")
@@ -391,8 +418,8 @@ class RRTStarInformed(RRT):
     _KIND = _lib.KIND_INFORMED
 
     def __init__(self, og: np.ndarray, n: int, r_rewire: float, r_goal: float, costfn: callable = None,
-                 pbar: bool = True, seed: int = 0, *, rewire: str = "reference"):
-        super().__init__(og, n, costfn=costfn, pbar=pbar, seed=seed)
+                 pbar: bool = True, seed: int = 0, *, rewire: str = "reference", robot_radius=None):
+        super().__init__(og, n, costfn=costfn, pbar=pbar, seed=seed, robot_radius=robot_radius)
         self.r_rewire = r_rewire
         self.r_goal = r_goal
         self.ellipses = {}
