@@ -138,6 +138,25 @@ size_t rrtk_inflate_disc_scratch_bytes(int nworlds, int W, int H);
 int rrtk_inflate_disc(const uint32_t *d_bits, int nworlds, int W, int H, const int32_t *d_src, const int32_t *d_r2, int nout,
                       uint32_t *d_out, void *d_scratch, void *stream);
 
+/* Configuration space of a body with a heading (a car: long and narrow), one grid per heading layer.  The body is given as L
+ * stencils, one per layer l = 0 .. L - 1, each an odd S x S mask centred on offset (0, 0): entry [l, i, j] is the offset
+ * d = (i - k, j - k), k = (S - 1) / 2, in grid index coordinates.  Layer l of world w blocks cell c iff some d of stencil l has
+ * c + d INSIDE the grid and og[c + d] != 0 (cells outside the grid are free, as for the disc), i.e.
+ *     layer[l] = scipy.ndimage.binary_dilation(og != 0, structure = S_l[::-1, ::-1], border_value = 0)
+ * The projection blocks a cell iff every layer blocks it: the free cells a planner samples from.  A pose with heading angle
+ * theta (radians, any real) tests layer floor(theta * (L / 2 pi) + 1/2) mod L (rrtk_plan2_batch_layers); with L = nheadings a
+ * vertex heading h tests layer h.
+ *   d_runs        DEVICE int32 triples (dx, dy_lo, dy_hi), one per run of set cells of a stencil row, grouped by layer (a row
+ *                 may hold several runs); every offset within [-127, 127] (S <= 255), dy_lo <= dy_hi
+ *   d_layer_runs  DEVICE int32, L + 1 prefix offsets: the runs of layer l are [d_layer_runs[l], d_layer_runs[l + 1])
+ *   d_layers      nworlds * L tiled bit grids (padding bits set), world-major: grid w * L + l, rrtk_grid_words(W, H) words each
+ *   d_proj        optional (NULL = not written): nworlds projection grids
+ * 1 <= L <= 256, the centre cell set in every layer (so no layer is larger than the free space), W, H <= 16384; anything else
+ * is RRTK_ERR_INVALID before a kernel runs.  The launch is sized by the stencils' extent, so the call copies the runs back and
+ * synchronises stream once.  One launch serves every layer of every world (csrc/body.cu).  No buffer may alias another. */
+int rrtk_inflate_body(const uint32_t *d_bits, int nworlds, int W, int H, const int32_t *d_runs, const int32_t *d_layer_runs, int nlayers,
+                      uint32_t *d_layers, uint32_t *d_proj, void *stream);
+
 /* ---- K1: RRT.collisionfree (rrt.py:183-229), batched ------------------------------------------- */
 /* d_segs: nseg x (ax, ay, bx, by) int32, all points inside the grid.  d_world: optional per-segment
  * world index (NULL = world 0).  d_free[s] = 1 iff the walk a->b meets no obstacle (both ends
@@ -381,6 +400,16 @@ int rrtk_plan2_batch(const rrtk_plan2_cfg *cfg, const uint32_t *d_bits, int W, i
                      int nplans, int n, const int16_t *d_samples, const uint8_t *d_heads, int16_t *d_pts, uint8_t *d_head,
                      double *d_cost, double *d_elen, int32_t *d_parent, int64_t *d_stats, void *d_scratch, int threads,
                      void *stream);
+/* rrtk_plan2_batch for a body with a heading: d_bits holds nlayers heading-layer grids per world (the d_layers of
+ * rrtk_inflate_body, world-major).  Every sampled pose of a Dubins edge tests, at its rounded cell, the layer of its own angle
+ * (floor(theta * (nlayers / 2 pi) + 1/2) mod nlayers); the end cell tests the layer of the end vertex's heading angle
+ * h * 2 pi / nheadings.  Leaving the grid still blocks.  Model DUBINS only (RRTK_ERR_INVALID otherwise); memo table,
+ * informed plans, rewire and both block sizes as for rrtk_plan2_batch.  With nlayers = 1 and the 1 x 1 stencil the trees are
+ * those of rrtk_plan2_batch on the grid itself. */
+int rrtk_plan2_batch_layers(const rrtk_plan2_cfg *cfg, const uint32_t *d_bits, int W, int H, int nlayers, const rrtk_plan_desc *d_plans,
+                            int nplans, int n, const int16_t *d_samples, const uint8_t *d_heads, int16_t *d_pts, uint8_t *d_head,
+                            double *d_cost, double *d_elen, int32_t *d_parent, int64_t *d_stats, void *d_scratch, int threads,
+                            void *stream);
 int rrtk_plan2_footprint(int n, int threads, int *smem_bytes, int *blocks_per_sm);
 
 /* Memo of the Dubins primitive: with integer cells and indexed headings the shortest path depends only on
@@ -397,6 +426,9 @@ int rrtk_dubins_paths(const int32_t *d_q, int64_t nq, int nheadings, double rho,
 /* sampled collision test of the shortest path of each query (the edge test above); d_world optional per query */
 int rrtk_dubins_collision(const uint32_t *d_bits, int W, int H, const int32_t *d_q, const int32_t *d_world, int64_t nq,
                           int nheadings, double rho, double ds, uint8_t *d_free, void *stream);
+/* the same test on nlayers heading-layer grids per world (the layer rule of rrtk_plan2_batch_layers) */
+int rrtk_dubins_collision_layers(const uint32_t *d_bits, int W, int H, int nlayers, const int32_t *d_q, const int32_t *d_world,
+                                 int64_t nq, int nheadings, double rho, double ds, uint8_t *d_free, void *stream);
 /* poses (x, y, theta) of each query's shortest path every ds cells: d_xyth nq x cap x 3, d_count[q] = number of
  * poses the path has (floor(len / ds) + 1; only the first cap are stored) */
 int rrtk_dubins_sample(const int32_t *d_q, int64_t nq, int nheadings, double rho, double ds, int cap, double *d_xyth,
@@ -423,6 +455,14 @@ int rrtk_ctx_inflate(rrtk_ctx *ctx, const uint8_t *h_og, int W, int H, int itera
  * rrtk_pack_grid_host, so they feed RRTK_IN_BITS directly.  W, H <= 16384. */
 int rrtk_ctx_inflate_disc(rrtk_ctx *ctx, const uint8_t *h_og, int nworlds, int W, int H, const int32_t *h_src, const int32_t *h_r2,
                           int nout, uint32_t *h_out);
+
+/* rrtk_ctx_set_grids for a body with a heading: uploads the nworlds uint8 grids and the body's runs (HOST arrays, the encoding
+ * of rrtk_inflate_body, checked before any device work) and builds the heading layers and their projection on the device.  The
+ * projections become the context's worlds (seed-mode sampling, h_nfree, the K7 and segment calls); rrtk_ctx_plan2 (model DUBINS
+ * only: EUCLID is RRTK_ERR_INVALID) and rrtk_ctx_dubins_collision test the layers.  rrtk_ctx_set_grids drops them again.  The
+ * pipelined calls take their own grids and ignore the body. */
+int rrtk_ctx_set_body_grids(rrtk_ctx *ctx, const uint8_t *h_og, int nworlds, int W, int H, const int32_t *h_runs,
+                            const int32_t *h_layer_runs, int nlayers, int32_t *h_nfree);
 
 /* full plan() from host memory: H2D of descriptors (+ samples / balls / PCG64 states), K7, D2H of
  * the trees.  Exactly one of h_samples / h_state must be non-NULL (explicit stream vs. seed mode).

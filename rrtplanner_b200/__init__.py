@@ -13,6 +13,7 @@ from . import worlds  # noqa: F401
 from .worlds import perlin_occupancygrid  # noqa: F401
 from .rrt import RRT, RRTStandard, RRTStar, RRTStarInformed, r2norm, random_point_og  # noqa: F401
 from .dubins import RRTDubins, RRTStarDubins, dubins_collisionfree, dubins_length, dubins_path, dubins_points  # noqa: F401
+from .body import body_layer, body_runs, car_body  # noqa: F401
 from .batch import Batch2Result, BatchResult, DeviceBatch, DeviceBatch2, plan_batch, shard, shortcut_paths  # noqa: F401
 
 __version__ = "0.1.0"

@@ -70,6 +70,7 @@ SIGNATURES = {
     "rrtk_free_rows": (_i, [_vp, _i, _i, _i, _vp, _vp]),
     "rrtk_inflate_disc_scratch_bytes": (_sz, [_i, _i, _i]),
     "rrtk_inflate_disc": (_i, [_vp, _i, _i, _i, _vp, _vp, _i, _vp, _vp, _vp]),
+    "rrtk_inflate_body": (_i, [_vp, _i, _i, _i, _vp, _vp, _i, _vp, _vp, _vp]),
     "rrtk_gen_worlds": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _vp]),
     "rrtk_collision_segments": (_i, [_vp, _i, _i, _vp, _vp, _i64, _vp, _vp, _vp]),
     "rrtk_clearance_field": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _vp]),
@@ -100,6 +101,7 @@ SIGNATURES = {
     "rrtk_ctx_set_grids": (_i, [_vp, _vp, _i, _i, _i, _vp]),
     "rrtk_ctx_inflate": (_i, [_vp, _vp, _i, _i, _i, _vp, _i, _vp]),
     "rrtk_ctx_inflate_disc": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _i, _vp]),
+    "rrtk_ctx_set_body_grids": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _i, _vp]),
     "rrtk_ctx_plan": (_i, [_vp, _i, _vp, _i, _i, _d, _d, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "rrtk_ctx_plan_worlds": (_i, [_vp, _i, _vp, _i, _i, _i, _vp, _i, _i, _d, _d, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i]),
     "rrtk_ctx_plan_worlds2": (_i, [_vp, _i, _vp, _i, _i, _i, _vp, _i, _i, _d, _d, _vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp,
@@ -119,9 +121,11 @@ SIGNATURES = {
     "rrtk_dubins_table_build": (_i, [_i, _i, _d, _vp, _vp]),
     "rrtk_plan2_scratch_bytes": (_sz, [_i, _i]),
     "rrtk_plan2_batch": (_i, [_vp, _vp, _i, _i, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp]),
+    "rrtk_plan2_batch_layers": (_i, [_vp, _vp, _i, _i, _i, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp]),
     "rrtk_plan2_footprint": (_i, [_i, _i, _vp, _vp]),
     "rrtk_dubins_paths": (_i, [_vp, _i64, _i, _d, _vp, _vp, _vp, _vp]),
     "rrtk_dubins_collision": (_i, [_vp, _i, _i, _vp, _vp, _i64, _i, _d, _d, _vp, _vp]),
+    "rrtk_dubins_collision_layers": (_i, [_vp, _i, _i, _i, _vp, _vp, _i64, _i, _d, _d, _vp, _vp]),
     "rrtk_dubins_sample": (_i, [_vp, _i64, _i, _d, _d, _i, _vp, _vp, _vp]),
     "rrtk_ctx_plan2": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "rrtk_ctx_plan2_worlds": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp, _i, _i, _vp, _vp, _vp, _i, _i] + [_vp] * 11 + [_i]),
@@ -222,6 +226,7 @@ class Context:
         check(lib().rrtk_create(C.byref(self._h)), "rrtk_create")
         self.shape = None
         self.nworlds = 0
+        self.nlayers = 0
 
     def close(self):
         if self._h:
@@ -241,7 +246,24 @@ class Context:
         nw, W, H = og_u8.shape
         nfree = np.empty(nw, dtype=np.int32)
         check(lib().rrtk_ctx_set_grids(self._h, ptr(og_u8), nw, W, H, ptr(nfree)), "rrtk_ctx_set_grids")
-        self.shape, self.nworlds = (W, H), nw
+        self.shape, self.nworlds, self.nlayers = (W, H), nw, 0
+        return nfree
+
+    def set_body_grids(self, og_u8: np.ndarray, runs, layer_runs) -> np.ndarray:
+        """Worlds for a body with a heading (rrtk_ctx_set_body_grids): ``og_u8`` (nworlds, W, H), non-zero = obstacle; ``runs`` /
+        ``layer_runs`` the body's stencils as ``body.body_runs`` encodes them.  The context's worlds become the projections (a
+        cell is blocked iff every heading layer blocks it); ``plan2`` (Dubins) and ``dubins_collision`` test the layers until the
+        next ``set_grids``.  Returns the free cells per world of the projections."""
+        og_u8 = np.ascontiguousarray(og_u8, dtype=np.uint8)
+        if og_u8.ndim != 3:
+            raise ValueError("og_u8 must have shape (nworlds, W, H)")
+        nw, W, H = og_u8.shape
+        runs = np.ascontiguousarray(runs, dtype=np.int32).reshape(-1, 3)
+        layer_runs = np.ascontiguousarray(layer_runs, dtype=np.int32).reshape(-1)
+        nfree = np.empty(nw, dtype=np.int32)
+        check(lib().rrtk_ctx_set_body_grids(self._h, ptr(og_u8), nw, W, H, ptr(runs), ptr(layer_runs), layer_runs.shape[0] - 1, ptr(nfree)),
+              "rrtk_ctx_set_body_grids")
+        self.shape, self.nworlds, self.nlayers = (W, H), nw, layer_runs.shape[0] - 1
         return nfree
 
     # -- plans ---------------------------------------------------------------------------------

@@ -594,6 +594,7 @@ class DeviceBatch2(DeviceBatch):
         self.balls2 = None
         self.nheadings = int(self.cfg["nheadings"][0])
         self.heads = None
+        self.layers, self.nlayers = None, 0
         self.scratch = None
         self.table = None
         if use_table and m == _lib.MODEL_DUBINS and star and 1.0 <= float(r_rewire) <= 1024.0:
@@ -606,6 +607,34 @@ class DeviceBatch2(DeviceBatch):
                     _lib.check(self.L.rrtk_dubins_table_build(R, self.nheadings, float(rho), self._p(self.table), self._stream()),
                                "dubins_table_build")
                 self.cfg["dubins_table"], self.cfg["table_radius"] = self.table.data_ptr(), R
+
+    def set_worlds_u8(self, og_u8):
+        self.layers, self.nlayers = None, 0          # new worlds: a body's layers must be built again
+        return super().set_worlds_u8(og_u8)
+
+    def inflate_body(self, stencils):
+        """Plan for a body with a heading: ``stencils`` (nlayers, S, S) as ``body.car_body`` makes them.  On the device and on
+        torch's current stream, builds ``layers`` (nworlds * nlayers heading-layer grids, rrtk_inflate_body), replaces ``bits``
+        by their projection (a cell is blocked iff every layer blocks it) and rebuilds ``rowcum`` from it, so the samplers draw
+        from the projection; ``run()`` then plans on the layers (rrtk_plan2_batch_layers).  Dubins batches only.  Returns self."""
+        if int(self.cfg["model"][0]) != _lib.MODEL_DUBINS:
+            raise ValueError("a body with a heading needs model 'dubins'")
+        from .body import body_runs
+
+        t = self.torch
+        runs, layer_runs = body_runs(stencils)
+        L = layer_runs.shape[0] - 1
+        nw = int(self.bits.shape[0])
+        d_runs = t.from_numpy(np.concatenate([runs.reshape(-1), np.zeros(1, np.int32)])).to(self.dev)
+        d_lr = t.from_numpy(layer_runs).to(self.dev)
+        layers = self._empty((nw * L, self.words), t.int32)
+        proj = self._empty((nw, self.words), t.int32)
+        with t.cuda.device(self.dev):
+            _lib.check(self.L.rrtk_inflate_body(self._p(self.bits), nw, self.W, self.H, self._p(d_runs), self._p(d_lr), L, self._p(layers),
+                                                self._p(proj), self._stream()), "inflate_body")
+            _lib.check(self.L.rrtk_free_rows(self._p(proj), nw, self.W, self.H, self._p(self.rowcum), self._stream()), "free_rows")
+        self.bits, self.layers, self.nlayers = proj, layers, L
+        return self
 
     def set_plans(self, desc: np.ndarray):
         t = self.torch
@@ -654,6 +683,13 @@ class DeviceBatch2(DeviceBatch):
     def run(self):
         o = self.out
         with self.torch.cuda.device(self.dev):
+            if self.layers is not None:
+                _lib.check(self.L.rrtk_plan2_batch_layers(_lib.ptr(self.cfg), self._p(self.layers), self.W, self.H, self.nlayers,
+                                                          self._p(self.desc), self.nplans, self.n, self._p(self.samples), self._p(self.heads),
+                                                          self._p(o["pts"]), self._p(o["head"]), self._p(o["cost"]), self._p(o["elen"]),
+                                                          self._p(o["parent"]), self._p(o["stats"]), self._p(self.scratch), self.threads,
+                                                          self._stream()), "plan2_batch_layers")
+                return self
             _lib.check(self.L.rrtk_plan2_batch(_lib.ptr(self.cfg), self._p(self.bits), self.W, self.H, self._p(self.desc), self.nplans,
                                                self.n, self._p(self.samples), self._p(self.heads), self._p(o["pts"]), self._p(o["head"]),
                                                self._p(o["cost"]), self._p(o["elen"]), self._p(o["parent"]), self._p(o["stats"]),

@@ -16,7 +16,7 @@ CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "librrtk.so")
 SOURCES = ["api.cu", "grid.cu", "inflate.cu", "collision.cu", "clearance.cu", "queries.cu", "rng.cu", "plan.cu", "plan_wide.cu",
            "plan_scan_standard.cu", "plan_scan_star.cu", "plan_scan_informed.cu", "plan_grid.cu", "plan_rewire.cu", "peaks.cu",
-           "shortcut.cu", "disc.cu"]
+           "shortcut.cu", "disc.cu", "body.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "--fmad=false",            # cost arithmetic must be mul / add / sqrt in IEEE double, never fused

@@ -1,5 +1,6 @@
 // extern "C" surface of librrtk.so (declared in include/rrtk.h): argument checks, device info,
 // the host-buffer context, and thin forwards to the kernel launchers.
+#include <algorithm>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -40,6 +41,8 @@ int unpack_launch(const uint32_t *, int, int, int, uint8_t *, cudaStream_t);
 int inflate_launch(const uint32_t *, int, int, int, int, const int32_t *, int, uint32_t *, uint32_t *, cudaStream_t);
 int disc_launch(const uint32_t *, int, int, int, const int32_t *, const int32_t *, int, uint32_t *, void *, cudaStream_t);
 size_t disc_scratch_bytes(int, int, int);
+int body_launch(const uint32_t *, int, int, int, const int32_t *, const int32_t *, int, int, int, uint32_t *, uint32_t *, cudaStream_t);
+size_t body_smem_bytes(int, int);
 int nearest_launch(const int32_t *, int, const int32_t *, const int32_t *, int, int32_t *, int64_t *, cudaStream_t);
 int nearest_launch_f64(const double *, int, const double *, const int32_t *, int, int32_t *, double *, cudaStream_t);
 int within_launch(const int32_t *, int, const int32_t *, const int32_t *, int, double, int, int32_t *, int32_t *, cudaStream_t);
@@ -62,7 +65,7 @@ int paths_xy_launch(const int32_t *, const int16_t *, const double *, const int6
                     double *, cudaStream_t);
 int shortcut_launch(const uint32_t *, int, int, const int32_t *, int, int, int, int16_t *, int32_t *, int32_t *, int32_t *, double *,
                     cudaStream_t);
-int plan2_launch(const rrtk_plan2_cfg &, const uint32_t *, int, int, const rrtk_plan_desc *, int, int, const int16_t *, const uint8_t *,
+int plan2_launch(const rrtk_plan2_cfg &, const uint32_t *, int, int, int, const rrtk_plan_desc *, int, int, const int16_t *, const uint8_t *,
                  int16_t *, uint8_t *, double *, double *, int32_t *, int64_t *, void *, int, int, cudaStream_t);
 size_t plan2_scratch_bytes(int, int);
 int plan2_footprint(int, int, int, int, int *, int *);
@@ -71,7 +74,7 @@ size_t dubins_table_bytes(int, int);
 int dubins_table_launch(int, int, double, void *, int, cudaStream_t);
 int l2_read_launch(const void *, size_t, int, int, uint32_t *, cudaStream_t);
 int smem_read_launch(int, int, int, uint32_t *, cudaStream_t);
-int dubins_walk_launch(const uint32_t *, int, int, const int32_t *, const int32_t *, int64_t, int, double, double, uint8_t *, int,
+int dubins_walk_launch(const uint32_t *, int, int, int, const int32_t *, const int32_t *, int64_t, int, double, double, uint8_t *, int,
                        double *, int32_t *, cudaStream_t);
 
 struct DevInfo { int dev = -1, sms = 0, optin = 0, sm_smem = 0; };
@@ -164,6 +167,8 @@ struct rrtk_ctx {
     DevBuf pts, cost, parent, stats, ell;       // plan outputs
     DevBuf a, b, c, d, e;                       // query scratch
     DevBuf heads, head_out, elen, scratch2;     // K8 (rrtk_ctx_plan2)
+    DevBuf layers;                              // rrtk_ctx_set_body_grids: nlayers heading-layer grids per world (0: none)
+    int nlayers = 0;
     DevBuf dtable;                              // memo of the Dubins primitive, valid for (dt_R, dt_NH, dt_rho)
     int dt_R = 0, dt_NH = 0;
     double dt_rho = 0.0;
@@ -246,6 +251,47 @@ static int check_rewire_overflow(const int64_t *h_stats, int nplans)
             set_error("plan %d: a rewire-radius set exceeded the kernel's list (1024 vertices); reduce r_rewire", p);
             return RRTK_ERR_CAPACITY;
         }
+    return RRTK_OK;
+}
+
+// Body stencils as runs (rrtk_inflate_body): nlayers in [1, 256], layer_runs non-decreasing from 0, every run inside the 255 x 255
+// mask around the centre with dy_lo <= dy_hi, and the centre cell in every layer.  *k: the largest |offset| of any run, *P: the
+// log-doubling levels the longest run needs.
+static int check_body_runs(const int32_t *runs, const int32_t *layer_runs, int nlayers, const char *who, int *k, int *P)
+{
+    if (nlayers < 1 || nlayers > 256) {
+        set_error("%s: need 1 <= nlayers <= 256 (got %d)", who, nlayers);
+        return RRTK_ERR_INVALID;
+    }
+    if (layer_runs[0] != 0) {
+        set_error("%s: layer_runs[0] must be 0", who);
+        return RRTK_ERR_INVALID;
+    }
+    for (int l = 0; l < nlayers; ++l)
+        if (layer_runs[l + 1] < layer_runs[l] || layer_runs[l + 1] - layer_runs[l] > 255 * 128) {
+            set_error("%s: layer %d: layer_runs must be non-decreasing with at most %d runs per layer", who, l, 255 * 128);
+            return RRTK_ERR_INVALID;
+        }
+    int kmax = 0, longest = 1;
+    for (int l = 0; l < nlayers; ++l) {
+        bool centre = false;
+        for (int r = layer_runs[l]; r < layer_runs[l + 1]; ++r) {
+            const int dx = runs[3 * r], lo = runs[3 * r + 1], hi = runs[3 * r + 2];
+            if (dx < -127 || dx > 127 || lo < -127 || hi > 127 || lo > hi) {
+                set_error("%s: run %d (%d, %d, %d) of layer %d lies outside the 255 x 255 stencil or has dy_lo > dy_hi", who, r, dx, lo, hi, l);
+                return RRTK_ERR_INVALID;
+            }
+            centre |= dx == 0 && lo <= 0 && hi >= 0;
+            kmax = std::max(kmax, std::max(std::abs(dx), std::max(-lo, hi)));
+            longest = std::max(longest, hi - lo + 1);
+        }
+        if (!centre) {
+            set_error("%s: layer %d does not contain the centre cell", who, l);
+            return RRTK_ERR_INVALID;
+        }
+    }
+    *k = kmax;
+    *P = 32 - __builtin_clz((unsigned)longest);
     return RRTK_OK;
 }
 
@@ -544,6 +590,37 @@ int rrtk_inflate_disc(const uint32_t *d_bits, int nworlds, int W, int H, const i
     return disc_launch(d_bits, nworlds, W, H, d_src, d_r2, nout, d_out, d_scratch, (cudaStream_t)stream);
 }
 
+int rrtk_inflate_body(const uint32_t *d_bits, int nworlds, int W, int H, const int32_t *d_runs, const int32_t *d_layer_runs, int nlayers,
+                      uint32_t *d_layers, uint32_t *d_proj, void *stream)
+{
+    RRTK_REQUIRE(nworlds >= 0, "rrtk_inflate_body: negative count");
+    RRTK_REQUIRE(d_bits && d_runs && d_layer_runs && d_layers, "rrtk_inflate_body: null pointer");
+    RRTK_REQUIRE(nlayers >= 1 && nlayers <= 256, "rrtk_inflate_body: need 1 <= nlayers <= 256");
+    RRTK_REQUIRE((const void *)d_layers != (const void *)d_bits && (const void *)d_proj != (const void *)d_bits &&
+                     (const void *)d_proj != (const void *)d_layers, "rrtk_inflate_body: buffers must not alias");
+    RRTK_TRY(check_grid_dims(W, H, 16384));
+    // the launch is sized by the stencils' extent, so the runs come back to the host first (one synchronisation of stream)
+    cudaStream_t st = (cudaStream_t)stream;
+    std::vector<int32_t> lr(nlayers + 1);
+    RRTK_CUDA(cudaMemcpyAsync(lr.data(), d_layer_runs, sizeof(int32_t) * (nlayers + 1), cudaMemcpyDeviceToHost, st));
+    RRTK_CUDA(cudaStreamSynchronize(st));
+    RRTK_REQUIRE(lr[0] == 0 && lr[nlayers] >= lr[0] && lr[nlayers] <= 256 * 255 * 128, "rrtk_inflate_body: bad layer_runs");
+    std::vector<int32_t> runs(3 * (size_t)lr[nlayers] + 1);
+    if (lr[nlayers]) {
+        RRTK_CUDA(cudaMemcpyAsync(runs.data(), d_runs, sizeof(int32_t) * 3 * (size_t)lr[nlayers], cudaMemcpyDeviceToHost, st));
+        RRTK_CUDA(cudaStreamSynchronize(st));
+    }
+    int k = 0, P = 1;
+    RRTK_TRY(check_body_runs(runs.data(), lr.data(), nlayers, "rrtk_inflate_body", &k, &P));
+    DevInfo *d;
+    RRTK_TRY(dev_info(&d));
+    if (body_smem_bytes(k, P) > (size_t)d->optin) {
+        set_error("rrtk_inflate_body: stencils of radius %d need %zu bytes of shared memory (limit %d)", k, body_smem_bytes(k, P), d->optin);
+        return RRTK_ERR_CAPACITY;
+    }
+    return body_launch(d_bits, nworlds, W, H, d_runs, d_layer_runs, nlayers, k, P, d_layers, d_proj, st);
+}
+
 int rrtk_free_rows(const uint32_t *d_bits, int nworlds, int W, int H, int32_t *d_rowcum, void *stream)
 {
     RRTK_REQUIRE(d_bits && d_rowcum && nworlds >= 0, "rrtk_free_rows: null pointer or negative count");
@@ -835,6 +912,19 @@ int rrtk_destroy(rrtk_ctx *c)
     return RRTK_OK;
 }
 
+// free-space index of the context's worlds (c->bits) and the free cells per world
+static int ctx_index_worlds(rrtk_ctx *c, int nworlds, int W, int H, int32_t *h_nfree)
+{
+    RRTK_TRY(free_rows_launch(c->bits.as<uint32_t>(), nworlds, W, H, c->rowcum.as<int32_t>(), c->stream));
+    c->nfree.assign(nworlds, 0);
+    RRTK_CUDA(cudaMemcpy2DAsync(c->nfree.data(), 4, c->rowcum.as<int32_t>() + W, (size_t)(W + 1) * 4, 4, nworlds,
+                                cudaMemcpyDeviceToHost, c->stream));
+    RRTK_CUDA(cudaStreamSynchronize(c->stream));
+    if (h_nfree) memcpy(h_nfree, c->nfree.data(), (size_t)nworlds * 4);
+    c->W = W; c->H = H; c->nworlds = nworlds;
+    return RRTK_OK;
+}
+
 int rrtk_ctx_set_grids(rrtk_ctx *c, const uint8_t *h_og, int nworlds, int W, int H, int32_t *h_nfree)
 {
     RRTK_REQUIRE(c && h_og && nworlds >= 1, "rrtk_ctx_set_grids: bad argument");
@@ -845,14 +935,43 @@ int rrtk_ctx_set_grids(rrtk_ctx *c, const uint8_t *h_og, int nworlds, int W, int
     RRTK_TRY(c->rowcum.reserve((size_t)(W + 1) * 4 * nworlds));
     RRTK_CUDA(cudaMemcpyAsync(c->og.p, h_og, cells * nworlds, cudaMemcpyHostToDevice, c->stream));
     RRTK_TRY(pack_launch(c->og.as<uint8_t>(), nworlds, W, H, c->bits.as<uint32_t>(), c->stream));
-    RRTK_TRY(free_rows_launch(c->bits.as<uint32_t>(), nworlds, W, H, c->rowcum.as<int32_t>(), c->stream));
     c->nworlds = 0;
-    c->nfree.assign(nworlds, 0);
-    RRTK_CUDA(cudaMemcpy2DAsync(c->nfree.data(), 4, c->rowcum.as<int32_t>() + W, (size_t)(W + 1) * 4, 4, nworlds,
-                                cudaMemcpyDeviceToHost, c->stream));
-    RRTK_CUDA(cudaStreamSynchronize(c->stream));
-    if (h_nfree) memcpy(h_nfree, c->nfree.data(), (size_t)nworlds * 4);
-    c->W = W; c->H = H; c->nworlds = nworlds;
+    c->nlayers = 0;
+    return ctx_index_worlds(c, nworlds, W, H, h_nfree);
+}
+
+int rrtk_ctx_set_body_grids(rrtk_ctx *c, const uint8_t *h_og, int nworlds, int W, int H, const int32_t *h_runs, const int32_t *h_layer_runs,
+                            int nlayers, int32_t *h_nfree)
+{
+    RRTK_REQUIRE(c && h_og && h_runs && h_layer_runs && nworlds >= 1, "rrtk_ctx_set_body_grids: bad argument");
+    RRTK_TRY(check_grid_dims(W, H, 16384));
+    int k = 0, P = 1;
+    RRTK_TRY(check_body_runs(h_runs, h_layer_runs, nlayers, "rrtk_ctx_set_body_grids", &k, &P));
+    DevInfo *d;
+    RRTK_TRY(dev_info(&d));
+    if (body_smem_bytes(k, P) > (size_t)d->optin) {
+        set_error("rrtk_ctx_set_body_grids: stencils of radius %d need %zu bytes of shared memory (limit %d)", k, body_smem_bytes(k, P), d->optin);
+        return RRTK_ERR_CAPACITY;
+    }
+    const size_t cells = (size_t)W * H, wb = grid_words(W, H) * 4, nruns = (size_t)h_layer_runs[nlayers];
+    cudaStream_t st = c->stream;
+    // og = source uint8, b = source bits, e = runs then layer_runs; the projection becomes the context's worlds
+    RRTK_TRY(c->og.reserve(cells * nworlds));
+    RRTK_TRY(c->b.reserve(wb * nworlds));
+    RRTK_TRY(c->e.reserve((nruns * 3 + nlayers + 1) * 4));
+    RRTK_TRY(c->layers.reserve(wb * nworlds * nlayers));
+    RRTK_TRY(c->bits.reserve(wb * nworlds));
+    RRTK_TRY(c->rowcum.reserve((size_t)(W + 1) * 4 * nworlds));
+    c->nworlds = 0;
+    c->nlayers = 0;
+    RRTK_CUDA(cudaMemcpyAsync(c->og.p, h_og, cells * nworlds, cudaMemcpyHostToDevice, st));
+    if (nruns) RRTK_CUDA(cudaMemcpyAsync(c->e.p, h_runs, nruns * 12, cudaMemcpyHostToDevice, st));
+    RRTK_CUDA(cudaMemcpyAsync(c->e.as<int32_t>() + nruns * 3, h_layer_runs, (size_t)(nlayers + 1) * 4, cudaMemcpyHostToDevice, st));
+    RRTK_TRY(pack_launch(c->og.as<uint8_t>(), nworlds, W, H, c->b.as<uint32_t>(), st));
+    RRTK_TRY(body_launch(c->b.as<uint32_t>(), nworlds, W, H, c->e.as<int32_t>(), c->e.as<int32_t>() + nruns * 3, nlayers, k, P,
+                         c->layers.as<uint32_t>(), c->bits.as<uint32_t>(), st));
+    RRTK_TRY(ctx_index_worlds(c, nworlds, W, H, h_nfree));
+    c->nlayers = nlayers;
     return RRTK_OK;
 }
 
@@ -1368,8 +1487,26 @@ int rrtk_plan2_batch(const rrtk_plan2_cfg *cfg, const uint32_t *d_bits, int W, i
     if (nplans == 0) return RRTK_OK;
     DevInfo *d;
     RRTK_TRY(dev_info(&d));
-    return plan2_launch(*cfg, d_bits, W, H, d_plans, nplans, n, d_samples, d_heads, d_pts, d_head, d_cost, d_elen, d_parent, d_stats,
+    return plan2_launch(*cfg, d_bits, W, H, 0, d_plans, nplans, n, d_samples, d_heads, d_pts, d_head, d_cost, d_elen, d_parent, d_stats,
                         d_scratch, threads, d->optin, (cudaStream_t)stream);
+}
+
+int rrtk_plan2_batch_layers(const rrtk_plan2_cfg *cfg, const uint32_t *d_bits, int W, int H, int nlayers, const rrtk_plan_desc *d_plans,
+                            int nplans, int n, const int16_t *d_samples, const uint8_t *d_heads, int16_t *d_pts, uint8_t *d_head,
+                            double *d_cost, double *d_elen, int32_t *d_parent, int64_t *d_stats, void *d_scratch, int threads, void *stream)
+{
+    RRTK_TRY(check_plan2_cfg(cfg));
+    RRTK_REQUIRE(cfg->model == RRTK_MODEL_DUBINS, "rrtk_plan2_batch_layers: heading layers need model DUBINS");
+    RRTK_REQUIRE(nlayers >= 1 && nlayers <= 256, "rrtk_plan2_batch_layers: need 1 <= nlayers <= 256");
+    RRTK_REQUIRE(d_bits && d_plans && d_samples && d_pts && d_head && d_cost && d_elen && d_parent && d_stats && d_scratch,
+                 "rrtk_plan2_batch_layers: null pointer");
+    RRTK_REQUIRE(nplans >= 0 && n >= 1 && n <= 65534, "rrtk_plan2_batch_layers: need nplans >= 0 and 1 <= n <= 65534");
+    RRTK_TRY(check_grid_dims(W, H, 16384));
+    if (nplans == 0) return RRTK_OK;
+    DevInfo *d;
+    RRTK_TRY(dev_info(&d));
+    return plan2_launch(*cfg, d_bits, W, H, nlayers, d_plans, nplans, n, d_samples, d_heads, d_pts, d_head, d_cost, d_elen, d_parent,
+                        d_stats, d_scratch, threads, d->optin, (cudaStream_t)stream);
 }
 
 int rrtk_plan2_footprint(int n, int threads, int *smem_bytes, int *blocks_per_sm)
@@ -1398,7 +1535,18 @@ int rrtk_dubins_collision(const uint32_t *d_bits, int W, int H, const int32_t *d
     RRTK_TRY(check_dubins_args(nheadings, rho, ds));
     RRTK_TRY(check_grid_dims(W, H, 16384));
     if (nq == 0) return RRTK_OK;
-    return dubins_walk_launch(d_bits, W, H, d_q, d_world, nq, nheadings, rho, ds, d_free, 0, nullptr, nullptr, (cudaStream_t)stream);
+    return dubins_walk_launch(d_bits, W, H, 0, d_q, d_world, nq, nheadings, rho, ds, d_free, 0, nullptr, nullptr, (cudaStream_t)stream);
+}
+
+int rrtk_dubins_collision_layers(const uint32_t *d_bits, int W, int H, int nlayers, const int32_t *d_q, const int32_t *d_world, int64_t nq,
+                                 int nheadings, double rho, double ds, uint8_t *d_free, void *stream)
+{
+    RRTK_REQUIRE(d_bits && d_q && d_free && nq >= 0, "rrtk_dubins_collision_layers: bad argument");
+    RRTK_REQUIRE(nlayers >= 1 && nlayers <= 256, "rrtk_dubins_collision_layers: need 1 <= nlayers <= 256");
+    RRTK_TRY(check_dubins_args(nheadings, rho, ds));
+    RRTK_TRY(check_grid_dims(W, H, 16384));
+    if (nq == 0) return RRTK_OK;
+    return dubins_walk_launch(d_bits, W, H, nlayers, d_q, d_world, nq, nheadings, rho, ds, d_free, 0, nullptr, nullptr, (cudaStream_t)stream);
 }
 
 int rrtk_dubins_sample(const int32_t *d_q, int64_t nq, int nheadings, double rho, double ds, int cap, double *d_xyth, int32_t *d_count,
@@ -1407,7 +1555,7 @@ int rrtk_dubins_sample(const int32_t *d_q, int64_t nq, int nheadings, double rho
     RRTK_REQUIRE(d_q && d_xyth && d_count && nq >= 0 && cap >= 1, "rrtk_dubins_sample: bad argument");
     RRTK_TRY(check_dubins_args(nheadings, rho, ds));
     if (nq == 0) return RRTK_OK;
-    return dubins_walk_launch(nullptr, 1, 1, d_q, nullptr, nq, nheadings, rho, ds, nullptr, cap, d_xyth, d_count, (cudaStream_t)stream);
+    return dubins_walk_launch(nullptr, 1, 1, 0, d_q, nullptr, nq, nheadings, rho, ds, nullptr, cap, d_xyth, d_count, (cudaStream_t)stream);
 }
 
 // memo of the Dubins primitive over the rewire radius, kept in the context while (radius, headings, rho) stay the same
@@ -1440,6 +1588,7 @@ int rrtk_ctx_plan2(rrtk_ctx *c, const rrtk_plan2_cfg *cfg, const rrtk_plan_desc 
     RRTK_REQUIRE(nplans >= 0 && n >= 1 && n <= 65534, "rrtk_ctx_plan2: need nplans >= 0 and 1 <= n <= 65534");
     if (nplans == 0) return RRTK_OK;
     const bool dub = cfg->model == RRTK_MODEL_DUBINS;
+    RRTK_REQUIRE(dub || c->nlayers == 0, "rrtk_ctx_plan2: the context holds heading layers of a body (rrtk_ctx_set_body_grids): only DUBINS plans on them");
     RRTK_TRY(check_plan_descs(h_plans, nplans, c->nworlds, c->W, c->H, nullptr, dub ? cfg->nheadings : 0));
     if (h_state) RRTK_TRY(require_free_cells(c->nfree.data(), c->nworlds, h_plans, nplans, "rrtk_ctx_plan2"));
     RRTK_TRY(check_samples(h_samples, nplans, n, c->W, c->H));
@@ -1484,10 +1633,16 @@ int rrtk_ctx_plan2(rrtk_ctx *c, const rrtk_plan2_cfg *cfg, const rrtk_plan_desc 
         use.ell_c = c->ell.as<double>();
     }
     cfg = &use;
-    RRTK_TRY(rrtk_plan2_batch(cfg, c->bits.as<uint32_t>(), c->W, c->H, c->plans.as<rrtk_plan_desc>(), nplans, n, c->samples.as<int16_t>(),
-                              h_heads ? c->heads.as<uint8_t>() : nullptr, c->pts.as<int16_t>(), c->head_out.as<uint8_t>(),
-                              c->cost.as<double>(), c->elen.as<double>(), c->parent.as<int32_t>(), c->stats.as<int64_t>(),
-                              c->scratch2.p, 0, st));
+    if (c->nlayers > 0)
+        RRTK_TRY(rrtk_plan2_batch_layers(cfg, c->layers.as<uint32_t>(), c->W, c->H, c->nlayers, c->plans.as<rrtk_plan_desc>(), nplans, n,
+                                         c->samples.as<int16_t>(), h_heads ? c->heads.as<uint8_t>() : nullptr, c->pts.as<int16_t>(),
+                                         c->head_out.as<uint8_t>(), c->cost.as<double>(), c->elen.as<double>(), c->parent.as<int32_t>(),
+                                         c->stats.as<int64_t>(), c->scratch2.p, 0, st));
+    else
+        RRTK_TRY(rrtk_plan2_batch(cfg, c->bits.as<uint32_t>(), c->W, c->H, c->plans.as<rrtk_plan_desc>(), nplans, n, c->samples.as<int16_t>(),
+                                  h_heads ? c->heads.as<uint8_t>() : nullptr, c->pts.as<int16_t>(), c->head_out.as<uint8_t>(),
+                                  c->cost.as<double>(), c->elen.as<double>(), c->parent.as<int32_t>(), c->stats.as<int64_t>(),
+                                  c->scratch2.p, 0, st));
     RRTK_CUDA(cudaMemcpyAsync(h_pts, c->pts.p, rows * 4, cudaMemcpyDeviceToHost, st));
     RRTK_CUDA(cudaMemcpyAsync(h_head, c->head_out.p, rows, cudaMemcpyDeviceToHost, st));
     RRTK_CUDA(cudaMemcpyAsync(h_cost, c->cost.p, rows * 8, cudaMemcpyDeviceToHost, st));
@@ -1636,8 +1791,13 @@ int rrtk_ctx_dubins_collision(rrtk_ctx *c, int world, const int32_t *h_q, int64_
     RRTK_TRY(c->a.reserve((size_t)nq * 24));
     RRTK_TRY(c->b.reserve((size_t)nq));
     RRTK_CUDA(cudaMemcpyAsync(c->a.p, h_q, (size_t)nq * 24, cudaMemcpyHostToDevice, c->stream));
-    RRTK_TRY(rrtk_dubins_collision(c->bits.as<uint32_t>() + (size_t)world * grid_words(c->W, c->H), c->W, c->H, c->a.as<int32_t>(), nullptr,
-                                   nq, nheadings, rho, ds, c->b.as<uint8_t>(), c->stream));
+    const size_t wpg = grid_words(c->W, c->H);
+    if (c->nlayers > 0)
+        RRTK_TRY(rrtk_dubins_collision_layers(c->layers.as<uint32_t>() + (size_t)world * c->nlayers * wpg, c->W, c->H, c->nlayers,
+                                              c->a.as<int32_t>(), nullptr, nq, nheadings, rho, ds, c->b.as<uint8_t>(), c->stream));
+    else
+        RRTK_TRY(rrtk_dubins_collision(c->bits.as<uint32_t>() + (size_t)world * wpg, c->W, c->H, c->a.as<int32_t>(), nullptr, nq, nheadings,
+                                       rho, ds, c->b.as<uint8_t>(), c->stream));
     RRTK_CUDA(cudaMemcpyAsync(h_free, c->b.p, (size_t)nq, cudaMemcpyDeviceToHost, c->stream));
     RRTK_CUDA(cudaStreamSynchronize(c->stream));
     return RRTK_OK;

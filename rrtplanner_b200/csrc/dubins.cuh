@@ -322,16 +322,29 @@ __device__ __forceinline__ bool cell_blocked(const uint32_t *bits, int W, int H,
     return (__ldg(bits + word_index(cx, cy, TY)) >> (cy & 31)) & 1u;
 }
 
+// Heading layer of a pose with angle th on L layer grids (include/rrtk.h, rrtk_plan2_batch_layers): floor(th * (L / 2 pi) + 1/2)
+// mod L, non-negative.  The same double operations as the specification (oracle/body_oracle.c, body_layer).
+__device__ __forceinline__ int body_layer(double th, int L)
+{
+    const double f = floor(__dadd_rn(__dmul_rn(th, (double)L / DM_TWO_PI), 0.5));
+    const int l = (int)((long long)f % L);
+    return l < 0 ? l + L : l;
+}
+
 // warp-cooperative sampled collision test of the path w from (x0, y0, h0) to cell (x1, y1): points at arc length
 // k * ds, k = 0 .. floor(len / ds), one per lane, two rounds of 32 in flight together (their grid reads overlap),
 // plus the target cell.  All lanes must pass the same path.
+// LAYERS: bits is the first of L heading-layer grids lstride words apart; a pose tests the layer of its own angle, the target
+// cell the layer of heading h1 (the angle dubins_track gives a vertex heading).  Otherwise h1, lstride and L are not read.
 #ifndef RRTK_FREE_INLINE
 #define RRTK_FREE_INLINE __forceinline__
 #endif
 // Inlined by default; as a real call (-DRRTK_FREE_INLINE=__noinline__, measured: -4 %) it would have the register budget to
 // itself but pays for saving the plan loop's state around every test.
-__device__ RRTK_FREE_INLINE bool dubins_free_path(const uint32_t *bits, int W, int H, int TY, int x0, int y0, int h0, int x1, int y1,
-                                                 int NH, double rho, double ds, int word, double t, double p, double len, int lane)
+template <bool LAYERS>
+__device__ RRTK_FREE_INLINE bool dubins_free_path_t(const uint32_t *bits, int W, int H, int TY, int x0, int y0, int h0, int x1, int y1,
+                                                   int h1, int NH, double rho, double ds, int word, double t, double p, double len,
+                                                   int lane, size_t lstride, int L)
 {
     if (word < 0) return false;
     DubinsPath w;
@@ -343,21 +356,36 @@ __device__ RRTK_FREE_INLINE bool dubins_free_path(const uint32_t *bits, int W, i
         bool hit = false;
         if (ka <= ns) {
             const Pose a = dubins_point(tr, (double)ka * ds);
-            hit = cell_blocked(bits, W, H, TY, a.x, a.y);
+            hit = cell_blocked(LAYERS ? bits + (size_t)body_layer(a.th, L) * lstride : bits, W, H, TY, a.x, a.y);
         }
         if (kb <= ns) {
             const Pose b = dubins_point(tr, (double)kb * ds);
-            hit |= cell_blocked(bits, W, H, TY, b.x, b.y);
+            hit |= cell_blocked(LAYERS ? bits + (size_t)body_layer(b.th, L) * lstride : bits, W, H, TY, b.x, b.y);
         }
         if (__any_sync(RRTK_FULL, hit)) return false;
     }
-    return !((__ldg(bits + word_index(x1, y1, TY)) >> (y1 & 31)) & 1u);
+    const uint32_t *g1 = LAYERS ? bits + (size_t)body_layer((double)h1 * (DM_TWO_PI / (double)NH), L) * lstride : bits;
+    return !((__ldg(g1 + word_index(x1, y1, TY)) >> (y1 & 31)) & 1u);
+}
+
+__device__ RRTK_FREE_INLINE bool dubins_free_path(const uint32_t *bits, int W, int H, int TY, int x0, int y0, int h0, int x1, int y1,
+                                                 int NH, double rho, double ds, int word, double t, double p, double len, int lane)
+{
+    return dubins_free_path_t<false>(bits, W, H, TY, x0, y0, h0, x1, y1, 0, NH, rho, ds, word, t, p, len, lane, 0, 1);
 }
 
 __device__ __forceinline__ bool dubins_free_warp(const uint32_t *bits, int W, int H, int TY, int x0, int y0, int h0, int x1, int y1,
                                                  int NH, double rho, double ds, const DubinsPath &w, int lane)
 {
     return dubins_free_path(bits, W, H, TY, x0, y0, h0, x1, y1, NH, rho, ds, w.word, w.t, w.p, w.len, lane);
+}
+
+// dubins_free_warp on L heading-layer grids lstride words apart; h1 = the heading index of the target vertex
+__device__ __forceinline__ bool dubins_free_warp_layers(const uint32_t *bits, size_t lstride, int L, int W, int H, int TY, int x0, int y0,
+                                                        int h0, int x1, int y1, int h1, int NH, double rho, double ds, const DubinsPath &w,
+                                                        int lane)
+{
+    return dubins_free_path_t<true>(bits, W, H, TY, x0, y0, h0, x1, y1, h1, NH, rho, ds, w.word, w.t, w.p, w.len, lane, lstride, L);
 }
 
 }  // namespace rrtk

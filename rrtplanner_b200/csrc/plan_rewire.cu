@@ -35,6 +35,10 @@
 
 namespace rrtk {
 
+// Dubins model on heading-layer grids (rrtk_plan2_batch_layers): a pose tests the layer grid of its own heading.  Internal: the
+// public rrtk_model values are EUCLID and DUBINS.
+constexpr int kModelDubinsLayers = 2;
+
 enum { S2_J = 0, S2_VGOAL, S2_FOUND, S2_CHECKS, S2_ACCEPTED, S2_REWIRES, S2_PROPAGATED, S2_RING, S2_LEN_EVALS, S2_OVERFLOW, S2_ELL_ITERS, S2_FIRST_SOL };
 
 struct Plan2Params {
@@ -68,6 +72,7 @@ struct Plan2Params {
     const double *ttpq;     // (t, p, q)
     const uint8_t *tword;   // word
     int tR;
+    int nlayers;            // kModelDubinsLayers: heading-layer grids per world, words_per_grid apart
 };
 
 __host__ __device__ __forceinline__ size_t dubins_table_entries(int R, int NH) { return (size_t)(2 * R + 1) * (2 * R + 1) * NH * NH; }
@@ -119,11 +124,14 @@ struct Edge {
         w = tmp;
     }
     // warp-cooperative: is a -> b free (w = the path of path() for the same pair)
-    static __device__ __forceinline__ bool is_free(const Plan2Params &P, const uint32_t *bits, uint32_t pa, int ha, uint32_t pb,
+    static __device__ __forceinline__ bool is_free(const Plan2Params &P, const uint32_t *bits, uint32_t pa, int ha, uint32_t pb, int hb,
                                                    const DubinsPath &w, int lane)
     {
         if (MODEL == RRTK_MODEL_EUCLID)
             return warp_first_hit(GlobalGrid{bits}, P.TY, px(pa), py(pa), px(pb), py(pb), lane) < 0;
+        if (MODEL == kModelDubinsLayers)
+            return dubins_free_warp_layers(bits, P.words_per_grid, P.nlayers, P.W, P.H, P.TY, px(pa), py(pa), ha, px(pb), py(pb), hb, P.NH,
+                                           P.rho, P.ds, w, lane);
         return dubins_free_warp(bits, P.W, P.H, P.TY, px(pa), py(pa), ha, px(pb), py(pb), P.NH, P.rho, P.ds, w, lane);
     }
 };
@@ -143,6 +151,7 @@ template <int MODEL, int T, bool INF>
 __global__ void __launch_bounds__(T, RRTK_K8_BLOCK_THREADS / T) plan_rewire_kernel(Plan2Params P)
 {
     constexpr int NW = T / 32;
+    constexpr bool DUB = MODEL != RRTK_MODEL_EUCLID;
     constexpr int KS = 1024 / T;                 // radius-set slots per thread (the list holds at most 1024)
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int n = P.n, cap = P.ring_cap;
@@ -180,7 +189,7 @@ __global__ void __launch_bounds__(T, RRTK_K8_BLOCK_THREADS / T) plan_rewire_kern
     __shared__ double s_cb;                     // informed: budget c of the ellipse the next sample is drawn from (s_nsol > 0)
 
     const rrtk_plan_desc pd = P.plans[plan];
-    const uint32_t *bits = P.bits + (size_t)pd.world * P.words_per_grid;
+    const uint32_t *bits = P.bits + (size_t)pd.world * (MODEL == kModelDubinsLayers ? P.nlayers : 1) * P.words_per_grid;
     const short2 *samples = P.samples + (size_t)plan * n;
     const uint8_t *heads = P.heads ? P.heads + (size_t)plan * n : nullptr;
     short2 *o_pts = P.pts + (size_t)plan * (n + 1);
@@ -202,7 +211,7 @@ __global__ void __launch_bounds__(T, RRTK_K8_BLOCK_THREADS / T) plan_rewire_kern
         cost[v] = CUDART_INF; elen[v] = CUDART_INF; parent[v] = -1;
         if (INF && ell_c) ell_c[v] = CUDART_NAN;
     }
-    if (MODEL == RRTK_MODEL_DUBINS) {
+    if (DUB) {
         const double dth = DM_TWO_PI / (double)P.NH;
         for (int h = tid; h < P.NH; h += T) {
             double s, c;
@@ -213,8 +222,8 @@ __global__ void __launch_bounds__(T, RRTK_K8_BLOCK_THREADS / T) plan_rewire_kern
     if (tid < 10) s_stat[tid] = 0;
     if (tid == 0) { s_nsol = 0; s_first = -1; s_cb = 0.0; }
     __syncthreads();
-    const int start_h = MODEL == RRTK_MODEL_DUBINS ? pd.reserved[0] : 0;
-    const int goal_h = MODEL == RRTK_MODEL_DUBINS ? pd.reserved[1] : 0;
+    const int start_h = DUB ? pd.reserved[0] : 0;
+    const int goal_h = DUB ? pd.reserved[1] : 0;
     if (tid == 0) {
         spts[0] = pack_xy(pd.start_x, pd.start_y); shead[0] = (uint8_t)start_h;
         o_pts[0] = make_short2((short)pd.start_x, (short)pd.start_y); o_head[0] = (uint8_t)start_h;
@@ -240,7 +249,7 @@ __global__ void __launch_bounds__(T, RRTK_K8_BLOCK_THREADS / T) plan_rewire_kern
     const bool both = P.rewire != 0;           // edge lengths in both directions per member
     // Dubins: a length costs ~1.5 k instructions, so phase B2 first drops the members no new vertex could improve;
     // Euclid: a length is one square root, so all of them are simply measured
-    const bool prune = both && MODEL == RRTK_MODEL_DUBINS;
+    const bool prune = both && DUB;
 
     for (int it = 0; it < n; ++it) {
         const short2 sm = samples[it];
@@ -252,7 +261,7 @@ __global__ void __launch_bounds__(T, RRTK_K8_BLOCK_THREADS / T) plan_rewire_kern
             if (tid == 0 && ell_c) ell_c[j] = c;                                                                     // rrt.py:701
             ++ell_iters;
         }
-        const int qh = (MODEL == RRTK_MODEL_DUBINS && heads) ? heads[it] : 0;
+        const int qh = (DUB && heads) ? heads[it] : 0;
         const uint32_t pnew = pack_xy(qx, qy);
 
         // ---- A: scan ---------------------------------------------------------------------------------
@@ -301,10 +310,10 @@ __global__ void __launch_bounds__(T, RRTK_K8_BLOCK_THREADS / T) plan_rewire_kern
             const int hn = shead[vnear];
             DubinsPath w0;
             const double l0 = Edge<MODEL>::length(P, tab, pn, hn, pnew, qh, w0);
-            if (MODEL == RRTK_MODEL_DUBINS && w0.t != w0.t)      // memoised length: fetch the path's (t, p, q)
+            if (DUB && w0.t != w0.t)      // memoised length: fetch the path's (t, p, q)
                 Edge<MODEL>::path(P, tab, pn, hn, pnew, qh, w0.word, w0);
             w0.len = l0;
-            const bool ok = Edge<MODEL>::is_free(P, bits, pn, hn, pnew, w0, lane);
+            const bool ok = Edge<MODEL>::is_free(P, bits, pn, hn, pnew, qh, w0, lane);
             if (lane == 0) {
                 ++my_checks; ++my_lens;
                 s_accept = ok && !dup_any && j != n && !overflow;
@@ -436,7 +445,7 @@ __global__ void __launch_bounds__(T, RRTK_K8_BLOCK_THREADS / T) plan_rewire_kern
             DubinsPath w;
             w.word = 0;
             Edge<MODEL>::path(P, tab, pv, shead[vn], pnew, qh, word1[i], w);
-            const bool ok = Edge<MODEL>::is_free(P, bits, pv, shead[vn], pnew, w, lane);
+            const bool ok = Edge<MODEL>::is_free(P, bits, pv, shead[vn], pnew, qh, w, lane);
             if (lane == 0) {
                 ++my_checks;
                 if (ok) atomicMin(&s_bestrank, r);
@@ -491,7 +500,7 @@ __global__ void __launch_bounds__(T, RRTK_K8_BLOCK_THREADS / T) plan_rewire_kern
                 DubinsPath w;
                 w.word = 0;
                 Edge<MODEL>::path(P, tab, pnew, qh, pv, shead[vn], word2[i], w);
-                const bool ok = Edge<MODEL>::is_free(P, bits, pnew, qh, pv, w, lane);
+                const bool ok = Edge<MODEL>::is_free(P, bits, pnew, qh, pv, shead[vn], w, lane);
                 __syncwarp();                        // every lane has read flag[i] before lane 0 rewrites it
                 if (lane == 0) { ++my_checks; flag[i] = ok ? 2 : 0; }
             }
@@ -595,7 +604,7 @@ __global__ void __launch_bounds__(T, RRTK_K8_BLOCK_THREADS / T) plan_rewire_kern
         DubinsPath w;
         w.word = 0;
         Edge<MODEL>::path(P, tab, spts[v], shead[v], pgoal, goal_h, (int)(int8_t)first[v], w);
-        const bool ok = Edge<MODEL>::is_free(P, bits, spts[v], shead[v], pgoal, w, lane);
+        const bool ok = Edge<MODEL>::is_free(P, bits, spts[v], shead[v], pgoal, goal_h, w, lane);
         if (lane == 0) {
             ++my_checks;
             if (ok) atomicMin(&s_best, (unsigned long long)__double_as_longlong(cg));
@@ -692,8 +701,9 @@ int plan2_footprint(int n, int threads, int optin, int sm_smem, int *smem_bytes,
     return RRTK_OK;
 }
 
-int plan2_launch(const rrtk_plan2_cfg &cfg, const uint32_t *d_bits, int W, int H, const rrtk_plan_desc *d_plans, int nplans, int n,
-                 const int16_t *d_samples, const uint8_t *d_heads, int16_t *d_pts, uint8_t *d_head, double *d_cost, double *d_elen,
+// nlayers > 0: DUBINS on nlayers heading-layer grids per world (rrtk_plan2_batch_layers); 0: one grid per world
+int plan2_launch(const rrtk_plan2_cfg &cfg, const uint32_t *d_bits, int W, int H, int nlayers, const rrtk_plan_desc *d_plans, int nplans,
+                 int n, const int16_t *d_samples, const uint8_t *d_heads, int16_t *d_pts, uint8_t *d_head, double *d_cost, double *d_elen,
                  int32_t *d_parent, int64_t *d_stats, void *d_scratch, int threads, int optin, cudaStream_t st)
 {
     Plan2Params P;
@@ -728,6 +738,7 @@ int plan2_launch(const rrtk_plan2_cfg &cfg, const uint32_t *d_bits, int W, int H
         P.tword = reinterpret_cast<const uint8_t *>(P.ttpq + 3 * N);
         P.tR = cfg.table_radius;
     }
+    P.nlayers = nlayers;
     P.ring_cap = plan2_ring_cap(n);
     const size_t smem = plan2_smem(n, P.ring_cap);
     if (smem + 1024 > (size_t)optin) {
@@ -739,6 +750,8 @@ int plan2_launch(const rrtk_plan2_cfg &cfg, const uint32_t *d_bits, int W, int H
         set_error("rrtk_plan2_batch: threads must be 0, 128 or 256");
         return RRTK_ERR_INVALID;
     }
+    if (nlayers > 0)
+        return T == 128 ? plan2_launch_t<kModelDubinsLayers, 128>(P, nplans, smem, st) : plan2_launch_t<kModelDubinsLayers, 256>(P, nplans, smem, st);
     if (cfg.model == RRTK_MODEL_EUCLID)
         return T == 128 ? plan2_launch_t<RRTK_MODEL_EUCLID, 128>(P, nplans, smem, st) : plan2_launch_t<RRTK_MODEL_EUCLID, 256>(P, nplans, smem, st);
     return T == 128 ? plan2_launch_t<RRTK_MODEL_DUBINS, 128>(P, nplans, smem, st) : plan2_launch_t<RRTK_MODEL_DUBINS, 256>(P, nplans, smem, st);
@@ -765,8 +778,10 @@ __global__ void dubins_paths_kernel(const int *q, long long nq, int NH, double r
     if (len) len[i] = w.len;
 }
 
-// one warp per query: sampled collision test, and optionally the sampled poses (cap per query)
-__global__ void dubins_walk_kernel(const uint32_t *bits, size_t words_per_grid, int W, int H, const int *q, const int *world,
+// one warp per query: sampled collision test, and optionally the sampled poses (cap per query).  LAYERS: each world has nlayers
+// heading-layer grids (rrtk_dubins_collision_layers).
+template <bool LAYERS>
+__global__ void dubins_walk_kernel(const uint32_t *bits, size_t words_per_grid, int W, int H, int nlayers, const int *q, const int *world,
                                    long long nq, int NH, double rho, double ds, uint8_t *free_out, int cap, double *xyth, int *count)
 {
     __shared__ double2 tab[256];
@@ -784,8 +799,10 @@ __global__ void dubins_walk_kernel(const uint32_t *bits, size_t words_per_grid, 
     DubinsPath w;
     dubins_shortest(e[3] - e[0], e[4] - e[1], e[2], e[5], NH, rho, tab, w);
     if (free_out) {
-        const uint32_t *g = bits + (size_t)(world ? world[i] : 0) * words_per_grid;
-        const bool ok = dubins_free_warp(g, W, H, tiles_y(H), e[0], e[1], e[2], e[3], e[4], NH, rho, ds, w, lane);
+        const uint32_t *g = bits + (size_t)(world ? world[i] : 0) * (LAYERS ? nlayers : 1) * words_per_grid;
+        const bool ok = LAYERS ? dubins_free_warp_layers(g, words_per_grid, nlayers, W, H, tiles_y(H), e[0], e[1], e[2], e[3], e[4], e[5], NH,
+                                                         rho, ds, w, lane)
+                               : dubins_free_warp(g, W, H, tiles_y(H), e[0], e[1], e[2], e[3], e[4], NH, rho, ds, w, lane);
         if (lane == 0) free_out[i] = ok ? 1 : 0;
     }
     if (xyth) {
@@ -846,11 +863,17 @@ int dubins_paths_launch(const int32_t *d_q, int64_t nq, int NH, double rho, int3
     return RRTK_OK;
 }
 
-int dubins_walk_launch(const uint32_t *d_bits, int W, int H, const int32_t *d_q, const int32_t *d_world, int64_t nq, int NH, double rho,
-                       double ds, uint8_t *d_free, int cap, double *d_xyth, int32_t *d_count, cudaStream_t st)
+// nlayers > 0: the worlds of d_bits are heading-layer grids, nlayers per world (rrtk_dubins_collision_layers)
+int dubins_walk_launch(const uint32_t *d_bits, int W, int H, int nlayers, const int32_t *d_q, const int32_t *d_world, int64_t nq, int NH,
+                       double rho, double ds, uint8_t *d_free, int cap, double *d_xyth, int32_t *d_count, cudaStream_t st)
 {
-    dubins_walk_kernel<<<(unsigned)((nq + 3) / 4), 128, 0, st>>>(d_bits, grid_words(W, H), W, H, d_q, d_world, nq, NH, rho, ds, d_free,
-                                                              cap, d_xyth, d_count);
+    const unsigned blocks = (unsigned)((nq + 3) / 4);
+    if (nlayers > 0)
+        dubins_walk_kernel<true><<<blocks, 128, 0, st>>>(d_bits, grid_words(W, H), W, H, nlayers, d_q, d_world, nq, NH, rho, ds, d_free, cap,
+                                                         d_xyth, d_count);
+    else
+        dubins_walk_kernel<false><<<blocks, 128, 0, st>>>(d_bits, grid_words(W, H), W, H, 0, d_q, d_world, nq, NH, rho, ds, d_free, cap,
+                                                          d_xyth, d_count);
     RRTK_CUDA(cudaGetLastError());
     return RRTK_OK;
 }

@@ -11,9 +11,12 @@ oracle/rewire_oracle.c (parity UNPINNED: it is this project's own definition).
 Model: a configuration is ``(x, y, h)`` -- an integer grid cell and a heading index ``h`` in ``[0, nheadings)``,
 heading angle ``h * 2 pi / nheadings`` measured from the +x axis towards +y.  Edges are shortest Dubins paths
 (turning radius ``rho`` cells) checked against the grid at points every ``ds`` cells of arc length.  ``robot_radius``
-(keyword-only) plans for a disc-shaped vehicle on the configuration-space grid, as for the planners of rrt.py; the footprint
-does not depend on the heading.  Nearest and
-rewire-radius queries are Euclidean on ``(x, y)`` exactly as in the reference's planners.
+(keyword-only) plans for a disc-shaped vehicle on the configuration-space grid, as for the planners of rrt.py; that footprint
+does not depend on the heading.  ``body`` (keyword-only, e.g. ``body.car_body(...)``) plans for a vehicle whose footprint turns
+with it: one stencil per heading layer, one configuration-space grid per layer (csrc/body.cu), and every sampled pose of an
+edge tests the layer of its own angle (``body.body_layer``), the edge's end cell the layer of the end heading.  Samples are
+drawn from the projection, the cells some heading leaves free.  Nearest and rewire-radius queries are Euclidean on ``(x, y)``
+exactly as in the reference's planners.
 """
 from __future__ import annotations
 
@@ -23,6 +26,7 @@ import networkx as nx
 import numpy as np
 
 from . import _lib
+from .body import body_runs, inflate_body_host
 from .rrt import RRT, _UNFILLED, _as_point
 
 __all__ = ["dubins_path", "dubins_length", "dubins_collisionfree", "dubins_points", "RRTDubins", "RRTStarDubins", "DUBINS_WORDS"]
@@ -60,12 +64,18 @@ def dubins_length(q0, q1, rho: float, nheadings: int = 16):
     return dubins_path(q0, q1, rho, nheadings)[2]
 
 
-def dubins_collisionfree(og, q0, q1, rho: float, nheadings: int = 16, ds: float = 1.0):
+def dubins_collisionfree(og, q0, q1, rho: float, nheadings: int = 16, ds: float = 1.0, body=None):
     """True iff the shortest Dubins path q0 -> q1 stays on free cells of ``og`` (points every ``ds`` cells, rounded to
-    the nearest cell, end cell included; leaving the grid counts as a collision)."""
+    the nearest cell, end cell included; leaving the grid counts as a collision).  ``body``: (nlayers, S, S) stencils of a body
+    with a heading (module ``body``); each pose then tests the heading layer of its own angle, the end cell that of q1's heading."""
     og = np.asarray(og)
     ctx = _lib.shared_context()
-    ctx.set_grids((og != 0).astype(np.uint8)[None])
+    if body is not None:
+        runs, layer_runs = body_runs(body)
+        ctx.set_body_grids((og != 0).astype(np.uint8)[None], runs, layer_runs)
+        RRT._cf_cache = None                 # the shared context no longer holds the grid RRT.collisionfree cached
+    else:
+        ctx.set_grids((og != 0).astype(np.uint8)[None])
     free = ctx.dubins_collision(_queries(q0, q1), nheadings, rho, ds)
     return bool(free[0]) if np.asarray(q0).ndim == 1 else free
 
@@ -87,7 +97,11 @@ class RRTDubins(RRT):
     _STAR = False
 
     def __init__(self, og: np.ndarray, n: int, rho: float, nheadings: int = 16, ds: float = 1.0, costfn: callable = None,
-                 pbar: bool = True, seed: int = 0, *, robot_radius=None):
+                 pbar: bool = True, seed: int = 0, *, robot_radius=None, body=None):
+        if body is not None and robot_radius is not None:
+            raise ValueError("pass either body or robot_radius, not both (a disc is a body whose stencils are all the same disc)")
+        self.body = None if body is None else np.asarray(body) != 0
+        self._body_runs = None if body is None else body_runs(body)
         super().__init__(og, n, costfn=costfn, pbar=pbar, seed=seed, robot_radius=robot_radius)
         if not (0 < rho <= 16384 and 0.05 <= ds <= 16384):
             raise ValueError("need 0 < rho <= 16384 and 0.05 <= ds <= 16384 (cells)")
@@ -96,6 +110,36 @@ class RRTDubins(RRT):
         self.rho, self.nheadings, self.ds = float(rho), int(nheadings), float(ds)
         self.r_rewire = 0.0
         self.rewire = False
+        if self.body is not None:
+            self.free = self._body_free(og)
+
+    def _body_free(self, og) -> np.ndarray:
+        """Free cells of the body's projection of ``og`` (the cells some heading leaves free), computed on the device."""
+        og = np.asarray(og)
+        if og.ndim != 2:
+            raise ValueError("og must be a 2-D occupancy grid")
+        _, proj = inflate_body_host(og, *self._body_runs)
+        return np.argwhere(proj[0] == 0)
+
+    def _device(self) -> "_lib.Context":
+        if self.body is None:
+            return super()._device()
+        if self._ctx is None:
+            self._ctx = _lib.Context()
+            self._dirty = True
+        if self._dirty:
+            og = np.asarray(self.og)
+            if og.ndim != 2:
+                raise ValueError("og must be a 2-D occupancy grid")
+            self._ctx.set_body_grids((og != 0).astype(np.uint8)[None], *self._body_runs)
+            self._dirty = False
+        return self._ctx
+
+    def set_og(self, og_new: np.ndarray):
+        """New occupancy grid; with a body its heading layers and projection are rebuilt."""
+        super().set_og(og_new)
+        if self.body is not None:
+            self.free = self._body_free(og_new)
 
     def sample_all_free(self):
         """A uniformly random free configuration: cell as RRT.sample_all_free (rrt.py:231-240), then a heading."""
@@ -103,7 +147,7 @@ class RRTDubins(RRT):
         return np.array([cell[0], cell[1], self.rand_gen.integers(0, self.nheadings)])
 
     def collisionfree(self, og, a, b) -> bool:  # noqa: D102 -- configurations instead of points
-        return dubins_collisionfree(og, a, b, self.rho, self.nheadings, self.ds)
+        return dubins_collisionfree(og, a, b, self.rho, self.nheadings, self.ds, body=self.body)
 
     def _sampler_overridden(self) -> bool:
         return type(self).sample_all_free is not RRTDubins.sample_all_free
@@ -178,7 +222,8 @@ class RRTStarDubins(RRTDubins):
     _STAR = True
 
     def __init__(self, og: np.ndarray, n: int, r_rewire: float, rho: float, nheadings: int = 16, ds: float = 1.0,
-                 costfn: callable = None, pbar: bool = True, seed: int = 0, *, rewire: bool = True, robot_radius=None):
-        super().__init__(og, n, rho, nheadings=nheadings, ds=ds, costfn=costfn, pbar=pbar, seed=seed, robot_radius=robot_radius)
+                 costfn: callable = None, pbar: bool = True, seed: int = 0, *, rewire: bool = True, robot_radius=None, body=None):
+        super().__init__(og, n, rho, nheadings=nheadings, ds=ds, costfn=costfn, pbar=pbar, seed=seed, robot_radius=robot_radius,
+                         body=body)
         self.r_rewire = r_rewire
         self.rewire = bool(rewire)
