@@ -243,6 +243,27 @@ int rrtk_sample_streams_carry(const uint32_t *d_bits, const int32_t *d_rowcum, i
                               const rrtk_plan_desc *d_plans, int nplans, uint64_t *d_state, uint32_t *d_carry,
                               int n, int16_t *d_samples, void *stream);
 
+/* Weighted sample streams: cells drawn from a per-cell weight map instead of uniformly over the free cells.  A weight map is
+ * (W, H) uint8, w[x*H + y] (the layout of the occupancy grids), one per world.  The effective weight of a cell is its weight
+ * where the bit grid leaves it free, else 0; T = the sum over the world.  Sample i of a plan is, exactly,
+ *     cum = cumsum(effective weights, row-major, int64);  k = integers(0, T);  cell = searchsorted(cum, k, side="right")
+ * with the plan's PCG64 generator as numpy draws integers(0, T) in every regime (T == 1: 0 without touching the generator;
+ * T < 2^32: 32-bit Lemire on buffered halves; T == 2^32: the raw halves; T > 2^32: 64-bit Lemire on next64).  With every
+ * weight 1 the stream is that of rrtk_sample_streams, byte for byte.
+ *   rrtk_weight_index  builds the index of nworlds worlds (d_bits = their tiled bit grids, d_weights = nworlds weight maps) in
+ *                      d_index, rrtk_weight_index_bytes(nworlds, W, H) bytes.  The layout is private except that its first
+ *                      nworlds int64 entries are the totals T, so a caller can check for T == 0 with one small copy.  The
+ *                      index is valid for these bit grids and weights only.  d_weights needs no particular alignment.
+ *   rrtk_sample_streams_weighted  n samples per plan from the index (same d_bits / d_weights / nworlds); d_state as for
+ *                      rrtk_sample_streams; with d_carry (optional, has_uint32 / uinteger per plan) d_state and d_carry advance
+ *                      in place as in rrtk_sample_streams_carry, without it d_state is only read.  A world with T == 0 has
+ *                      nothing to draw: its plans get in-grid cells that mean nothing (callers check the totals first). */
+size_t rrtk_weight_index_bytes(int nworlds, int W, int H);
+int rrtk_weight_index(const uint32_t *d_bits, const uint8_t *d_weights, int nworlds, int W, int H, void *d_index, void *stream);
+int rrtk_sample_streams_weighted(const uint32_t *d_bits, const uint8_t *d_weights, const void *d_index, int nworlds, int W, int H,
+                                 const rrtk_plan_desc *d_plans, int nplans, uint64_t *d_state, uint32_t *d_carry, int n,
+                                 int16_t *d_samples, void *stream);
+
 /* The unit-disc stream of the ellipse phase of RRTStarInformed.plan (rrt.py:240, 579-587, 694-701), from the same
  * generator: the reference draws free[choice(nfree)] in iterations 0 .. f (f = the first solution iteration) and then
  * unitball() = two uniform(0, 1) draws per iteration.  Per plan p (world d_plans[p].world, nfree = d_rowcum[world*(W+1)+W]):
@@ -506,12 +527,21 @@ int rrtk_ctx_plan_worlds(rrtk_ctx *ctx, int kind, const uint8_t *h_og, int nworl
  *                   after the extraction): h_path / h_xy / h_len hold the kept tree vertices, h_path_cost the pruned cost.
  *                   Needs RRTK_OUT_PATHS and path_cap <= RRTK_SHORTCUT_MAX_CAP (RRTK_ERR_INVALID / RRTK_ERR_CAPACITY before any
  *                   device work).  Trees and statistics are unchanged.  rrtk_ctx_plan2_worlds does not read this flag: straight
- *                   shortcuts would break the heading constraints of Dubins paths. */
+ *                   shortcuts would break the heading constraints of Dubins paths.
+ *   RRTK_SEED_WEIGHTS  seed mode draws each plan's cells from the weight maps of rrtk_ctx_set_sample_weights (one per world of
+ *                   this call: same nworlds, W and H): per chunk the index is built on the chunk's grids and
+ *                   rrtk_sample_streams_weighted replaces the uniform sampler.  Needs h_state and weights set, and cannot be
+ *                   combined with RRTK_SEED_BALLS (RRTK_ERR_INVALID otherwise, before any device work).  A world whose free
+ *                   cells carry no weight (T == 0) makes the call fail with RRTK_ERR_INVALID naming it, found on the device and
+ *                   reported when the call returns.  rrtk_ctx_plan2_worlds takes the flag too. */
 #define RRTK_IN_BITS 1
 #define RRTK_OUT_TREES 2
 #define RRTK_OUT_PATHS 4
 #define RRTK_SEED_BALLS 8
 #define RRTK_OUT_SHORTCUT 16
+#define RRTK_SEED_WEIGHTS 32
+/* copy nworlds (W, H) uint8 weight maps to the device for RRTK_SEED_WEIGHTS; h_weights NULL or nworlds 0 clears them */
+int rrtk_ctx_set_sample_weights(rrtk_ctx *ctx, const uint8_t *h_weights, int nworlds, int W, int H);
 int rrtk_ctx_plan_worlds2(rrtk_ctx *ctx, int kind, const void *h_grids, int nworlds, int W, int H,
                           const rrtk_plan_desc *h_plans, int nplans, int n, double r_rewire, double r_goal,
                           const int16_t *h_samples, const uint64_t *h_state, const double *h_balls, int flags,

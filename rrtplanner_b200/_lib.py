@@ -20,7 +20,7 @@ STAT_COUNT = len(STAT_NAMES)
 
 MODEL_EUCLID, MODEL_DUBINS = 0, 1
 # flags of rrtk_ctx_plan_worlds2 / rrtk_ctx_plan2_worlds
-IN_BITS, OUT_TREES, OUT_PATHS, SEED_BALLS, OUT_SHORTCUT = 1, 2, 4, 8, 16
+IN_BITS, OUT_TREES, OUT_PATHS, SEED_BALLS, OUT_SHORTCUT, SEED_WEIGHTS = 1, 2, 4, 8, 16, 32
 SHORTCUT_MAX_CAP = 4096            # RRTK_SHORTCUT_MAX_CAP: longest path row rrtk_shortcut_paths takes
 STAT2_NAMES = ("j", "vgoal", "found", "checks", "accepted", "rewires", "propagated", "ring_members", "len_evals", "overflow",
                "ell_iters", "first_solution_iter")
@@ -89,6 +89,9 @@ SIGNATURES = {
     "rrtk_argsort_scratch_bytes": (_sz, [_i]),
     "rrtk_sample_streams": (_i, [_vp, _vp, _i, _i, _vp, _i, _vp, _i, _vp, _vp]),
     "rrtk_sample_streams_carry": (_i, [_vp, _vp, _i, _i, _vp, _i, _vp, _vp, _i, _vp, _vp]),
+    "rrtk_weight_index_bytes": (_sz, [_i, _i, _i]),
+    "rrtk_weight_index": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp]),
+    "rrtk_sample_streams_weighted": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp, _i, _vp, _vp, _i, _vp, _vp]),
     "rrtk_ball_streams": (_i, [_vp, _i, _vp, _i, _i, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp]),
     "rrtk_plan_batch": (_i, [_i, _vp, _i, _i, _vp, _i, _i, _d, _d, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp]),
     "rrtk_plan_kernel": (C.c_char_p, [_i, _i, _i, _i, _i]),
@@ -101,6 +104,7 @@ SIGNATURES = {
     "rrtk_ctx_set_grids": (_i, [_vp, _vp, _i, _i, _i, _vp]),
     "rrtk_ctx_inflate": (_i, [_vp, _vp, _i, _i, _i, _vp, _i, _vp]),
     "rrtk_ctx_inflate_disc": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _i, _vp]),
+    "rrtk_ctx_set_sample_weights": (_i, [_vp, _vp, _i, _i, _i]),
     "rrtk_ctx_set_body_grids": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _i, _vp]),
     "rrtk_ctx_plan": (_i, [_vp, _i, _vp, _i, _i, _d, _d, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "rrtk_ctx_plan_worlds": (_i, [_vp, _i, _vp, _i, _i, _i, _vp, _i, _i, _d, _d, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i]),
@@ -188,6 +192,22 @@ def unpack_grids_host(bits, W: int, H: int) -> np.ndarray:
     return cells.transpose(0, 1, 3, 2, 4).reshape(b.shape[0], TX * 32, TY * 32)[:, :W, :H].copy()
 
 
+def sample_weights_array(weights, shape) -> np.ndarray:
+    """A weight map argument as a C-contiguous uint8 array of ``shape`` ((W, H) or (nworlds, W, H)); a single (W, H) map is
+    broadcast to every world.  Anything but uint8 is rejected (floats, other integer types, values outside [0, 255]): weights are
+    never quantised silently."""
+    w = np.asarray(weights)
+    if w.dtype != np.uint8:
+        raise TypeError(f"sample_weights must be a uint8 array (got {w.dtype}); weights are whole numbers in [0, 255]")
+    shape = tuple(int(v) for v in shape)
+    if w.shape != shape:
+        if len(shape) == 3 and w.shape == shape[1:]:
+            w = np.broadcast_to(w, shape)
+        else:
+            raise ValueError(f"sample_weights has shape {w.shape}, the grids need {shape}" + (f" or {shape[1:]}" if len(shape) == 3 else ""))
+    return np.ascontiguousarray(w)
+
+
 def check(rc: int, what: str = ""):
     if rc == 0:
         return
@@ -266,6 +286,25 @@ class Context:
         self.shape, self.nworlds, self.nlayers = (W, H), nw, layer_runs.shape[0] - 1
         return nfree
 
+    def set_sample_weights(self, weights, shape=None) -> None:
+        """Weight maps for RRTK_SEED_WEIGHTS (rrtk_ctx_set_sample_weights): (nworlds, W, H) uint8, or None to clear them.  ``shape``
+        (nworlds, W, H), if given, is the shape the maps must have (a single (W, H) map is then used for every world)."""
+        if weights is None:
+            check(lib().rrtk_ctx_set_sample_weights(self._h, None, 0, 0, 0), "rrtk_ctx_set_sample_weights")
+            return
+        w = sample_weights_array(weights, np.shape(weights) if shape is None else shape)
+        if w.ndim != 3:
+            raise ValueError("sample weights must have shape (nworlds, W, H)")
+        check(lib().rrtk_ctx_set_sample_weights(self._h, ptr(w), *w.shape), "rrtk_ctx_set_sample_weights")
+
+    def _weights_flag(self, sample_weights, nworlds, W, H) -> int:
+        """``sample_weights`` of the pipelined calls: None (uniform), True (the maps set_sample_weights holds) or maps to set now."""
+        if sample_weights is None or sample_weights is False:
+            return 0
+        if sample_weights is not True:
+            self.set_sample_weights(sample_weights, (nworlds, W, H))
+        return SEED_WEIGHTS
+
     # -- plans ---------------------------------------------------------------------------------
     def plan(self, kind, desc, n, r_rewire=0.0, r_goal=0.0, samples=None, states=None, balls=None, out=None):
         """``out``: optional preallocated (pts, cost, parent, stats, ell) host arrays (e.g. pinned)."""
@@ -319,13 +358,16 @@ class Context:
         return pts, cost, parent, stats, ell
 
     def plan_worlds2(self, kind, grids, W, H, desc, n, r_rewire=0.0, r_goal=0.0, samples=None, states=None, balls=None,
-                     bits=False, trees=False, paths=True, path_cap=256, out=None, chunk=0, seed_balls=False, shortcut=False):
+                     bits=False, trees=False, paths=True, path_cap=256, out=None, chunk=0, seed_balls=False, shortcut=False,
+                     sample_weights=None):
         """rrtk_ctx_plan_worlds2: ``grids`` is (nworlds, W, H) uint8, or with ``bits=True`` the (nworlds, words) uint32 tiled
         bit grids of pack_grids_host.  Returns a dict with ``stats`` and, as requested, the trees (``pts``, ``cost``,
         ``parent``, ``ell``) and / or the path records (``path``, ``xy``, ``len``, ``path_cost``).  ``out``: optional dict of
         preallocated (e.g. pinned) host arrays under the same names.  ``seed_balls`` (informed, with ``states``, no ``balls``):
         the ellipse phase draws from each plan's own generator, as a seeded RRTStarInformed object does (RRTK_SEED_BALLS).
-        ``shortcut`` (with ``paths``): the path records come back pruned by line of sight (RRTK_OUT_SHORTCUT, see shortcut())."""
+        ``shortcut`` (with ``paths``): the path records come back pruned by line of sight (RRTK_OUT_SHORTCUT, see shortcut()).
+        ``sample_weights`` (seed mode): each plan draws its cells from its world's weight map (RRTK_SEED_WEIGHTS): (nworlds, W, H)
+        or (W, H) uint8 maps, uploaded by this call, or True for the maps ``set_sample_weights`` already holds."""
         grids = np.ascontiguousarray(grids, dtype=np.uint32 if bits else np.uint8)
         nw = grids.shape[0]
         nplans = desc.shape[0]
@@ -337,6 +379,7 @@ class Context:
             return out[name]
         buf("stats", (nplans, STAT_COUNT), np.int64)
         flags = (1 if bits else 0) | (2 if trees else 0) | (4 if paths else 0) | (SEED_BALLS if seed_balls else 0) | (OUT_SHORTCUT if shortcut else 0)
+        flags |= self._weights_flag(sample_weights, nw, W, H)
         if trees:
             buf("pts", (nplans, n + 1, 2), np.int16); buf("cost", (nplans, n + 1), np.float64); buf("parent", (nplans, n + 1), np.int32)
             if kind == KIND_INFORMED:
@@ -432,11 +475,11 @@ class Context:
         return pts, head, cost, elen, parent, stats
 
     def plan2_worlds(self, cfg, grids, W, H, desc, n, samples=None, states=None, heads=None, bits=False, trees=False, paths=True,
-                     path_cap=256, out=None, chunk=0, balls=None, seed_balls=False):
+                     path_cap=256, out=None, chunk=0, balls=None, seed_balls=False, sample_weights=None):
         """rrtk_ctx_plan2_worlds: K8 plans with their worlds in one pipelined call.  ``grids`` as for plan_worlds2.  Returns a
         dict with ``stats`` and, as requested, the trees (``pts``, ``head``, ``cost``, ``elen``, ``parent``) and / or the path
         records (``path``, ``xy``, ``path_head``, ``len``, ``path_cost``); informed plans (``cfg["informed"]``, ``balls`` as for
-        plan2) also return ``ell``.  ``seed_balls`` as for plan_worlds2 (informed, with ``states``, no ``balls``)."""
+        plan2) also return ``ell``.  ``seed_balls`` and ``sample_weights`` as for plan_worlds2."""
         grids = np.ascontiguousarray(grids, dtype=np.uint32 if bits else np.uint8)
         nw = grids.shape[0]
         nplans = desc.shape[0]
@@ -454,6 +497,7 @@ class Context:
                 assert balls.shape == (nplans, n, 2), balls.shape
             cfg["balls"], cfg["ell_c"] = (0 if balls is None else balls.ctypes.data), buf("ell", (nplans, n + 1), np.float64).ctypes.data
         flags = (1 if bits else 0) | (2 if trees else 0) | (4 if paths else 0) | (SEED_BALLS if seed_balls else 0)
+        flags |= self._weights_flag(sample_weights, nw, W, H)
         if trees:
             buf("pts", (nplans, n + 1, 2), np.int16); buf("head", (nplans, n + 1), np.uint8); buf("cost", (nplans, n + 1), np.float64)
             buf("elen", (nplans, n + 1), np.float64); buf("parent", (nplans, n + 1), np.int32)

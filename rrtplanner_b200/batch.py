@@ -15,6 +15,7 @@ Two layers:
 """
 from __future__ import annotations
 
+import re
 from dataclasses import dataclass
 from typing import Optional, Sequence
 
@@ -175,7 +176,7 @@ class BatchResult:
 
 
 def plan_batch(kind, ogs, n, starts, goals, world_ids=None, r_rewire=0.0, r_goal=0.0, samples=None, seeds=None,
-               balls=None, rots=None, ctx: Optional[_lib.Context] = None, robot_radius=None) -> BatchResult:
+               balls=None, rots=None, ctx: Optional[_lib.Context] = None, robot_radius=None, sample_weights=None) -> BatchResult:
     """End-to-end batched plan() from host arrays through ``rrtk_ctx_plan_worlds``.
 
     ogs: (nworlds, W, H) array, non-zero = obstacle.  Either ``samples`` (P, n, 2) -- the explicit
@@ -199,6 +200,11 @@ def plan_batch(kind, ogs, n, starts, goals, world_ids=None, r_rewire=0.0, r_goal
     that radius in its world (``rrtk_inflate_disc``), i.e. it is what the planner class built with ``robot_radius`` computes.
     Each distinct (world, floor(radius^2)) pair is inflated once on the device, the packed grids come back once (1 bit per
     cell) and the plans run through ``rrtk_ctx_plan_worlds2`` on them.
+
+    ``sample_weights`` (``"standard"`` / ``"star"`` with ``seeds``): uint8 weight maps, (nworlds, W, H) like ``ogs`` or one (W, H)
+    map for every world.  Plan p then draws its cells by weight from its world's map, masked by the grid it plans on (with
+    ``robot_radius``, the configuration-space grid of its radius), i.e. it is what the planner class built with
+    ``sample_weights=sample_weights[world_ids[p]]`` computes.  The streams are drawn on the device (RRTK_SEED_WEIGHTS).
     """
     k = KINDS[kind] if isinstance(kind, str) else int(kind)
     seed_balls = isinstance(balls, str)
@@ -215,12 +221,21 @@ def plan_batch(kind, ogs, n, starts, goals, world_ids=None, r_rewire=0.0, r_goal
     ogs = np.asarray(ogs)
     if ogs.ndim == 2:
         ogs = ogs[None]
+    weights = None
+    if sample_weights is not None:
+        if k not in (_lib.KIND_STANDARD, _lib.KIND_STAR):
+            raise ValueError("sample_weights is for 'standard' and 'star' batches: the ellipse phase of a seeded informed batch "
+                             "(balls='seed') replays uniform free-space draws, so weighted informed batches are not supported")
+        if seeds is None or samples is not None:
+            raise ValueError("sample_weights weight the seeded streams: pass seeds, not samples")
+        weights = _lib.sample_weights_array(sample_weights, ogs.shape)
     starts = np.asarray(starts).reshape(-1, 2)
     nplans = starts.shape[0]
     if seed_balls and len(seeds) != nplans:
         raise ValueError("balls='seed' needs one seed per plan")
     if world_ids is None:
         world_ids = np.arange(nplans) % ogs.shape[0]
+    caller_worlds = np.asarray(world_ids).reshape(nplans)
     r2 = None
     if robot_radius is not None:
         r2 = _lib.disc_r2(robot_radius)
@@ -238,6 +253,8 @@ def plan_batch(kind, ogs, n, starts, goals, world_ids=None, r_rewire=0.0, r_goal
             pairs, world_ids = np.unique(np.stack([np.asarray(world_ids, dtype=np.int64).reshape(nplans), r2.astype(np.int64)], axis=1),
                                          axis=0, return_inverse=True)
             grids = ctx.inflate_disc(og_u8, pairs[:, 0], pairs[:, 1])
+            if weights is not None:
+                weights = weights[pairs[:, 0]]                    # each grid samples by the map of its source world
         desc = make_desc(np.asarray(world_ids).reshape(nplans), starts, goals, rots)
         states = None if seeds is None else seed_states(seeds)
         order = np.argsort(desc["world"], kind="stable")          # the pipelined call wants plans grouped by world
@@ -245,14 +262,21 @@ def plan_batch(kind, ogs, n, starts, goals, world_ids=None, r_rewire=0.0, r_goal
         if sorted_:
             order = np.arange(nplans)
         take = lambda a: None if a is None else np.asarray(a)[order]          # noqa: E731
-        if seed_balls or r2 is not None:
+        if seed_balls or r2 is not None or weights is not None:
             d = desc[order]
             stats = np.empty((nplans, _lib.STAT_COUNT), dtype=np.int64)
             try:
                 o = ctx.plan_worlds2(k, grids, og_u8.shape[1], og_u8.shape[2], d, n, r_rewire, r_goal, samples=take(samples),
                                      states=take(states), balls=None if seed_balls else take(balls), bits=r2 is not None,
-                                     trees=True, paths=False, seed_balls=seed_balls, out={"stats": stats})
+                                     trees=True, paths=False, seed_balls=seed_balls, out={"stats": stats}, sample_weights=weights)
             except ValueError as e:
+                # the call names a grid and a plan of the world-sorted batch: report the caller's plan and world instead
+                empty = re.search(r"world \d+ of plan (\d+) has no weight", str(e))
+                if empty:
+                    p = int(order[int(empty.group(1))])
+                    radius = "" if r2 is None else f" at robot_radius r2 = {int(r2[p])}"
+                    raise ValueError(f"plan {p}: sample_weights put no weight on a free cell of world {int(caller_worlds[p])}{radius}: "
+                                     "nothing to sample") from None
                 bad = (stats[:, 5] >= 0) & ~np.isfinite(d["rot"]).all(axis=1)
                 if "start == goal" not in str(e) or not bad.any():
                     raise
@@ -328,6 +352,7 @@ class DeviceBatch:
         self.L = _lib.lib()
         self.words = int(self.L.rrtk_grid_words(W, H))
         self.og = self.bits = self.rowcum = None
+        self.weights = None                         # set_sample_weights: (nworlds, W, H) uint8 on the device
         self.desc = self.samples = self.balls = None
         self.state_out = self.carry_out = None     # seed_informed: the generators after plan()
         self.nplans = 0
@@ -350,6 +375,7 @@ class DeviceBatch:
         t = self.torch
         assert og_u8.dtype == t.uint8 and og_u8.is_cuda and tuple(og_u8.shape[1:]) == (self.W, self.H)
         self.og = og_u8.contiguous()
+        self.weights = None                          # weight maps belong to the worlds they were given for
         nw = self.og.shape[0]
         self.bits = self._empty((nw, self.words), t.int32)
         self.rowcum = self._empty((nw, self.W + 1), t.int32)
@@ -402,6 +428,31 @@ class DeviceBatch:
         self.bits = bits
         return self
 
+    def set_sample_weights(self, weights):
+        """Weight maps for ``seed_samples``: a uint8 torch tensor or numpy array, (nworlds, W, H) or one (W, H) map for every
+        world.  ``seed_samples`` then draws each plan's cells by weight from its world's map, masked by ``bits`` as it is at that
+        call (so the weights follow ``inflate_disc`` / ``inflate_body``).  ``set_worlds_*`` clears them; None clears them too.
+        Returns self."""
+        t = self.torch
+        if weights is None:
+            self.weights = None
+            return self
+        shape = (int(self.bits.shape[0]), self.W, self.H)
+        if isinstance(weights, t.Tensor):
+            if weights.dtype != t.uint8:
+                raise TypeError(f"sample weights must be uint8 (got {weights.dtype}); weights are whole numbers in [0, 255]")
+            if tuple(weights.shape) == shape[1:]:
+                weights = weights.expand(shape)
+            if tuple(weights.shape) != shape:
+                raise ValueError(f"sample weights have shape {tuple(weights.shape)}, the worlds need {shape} or {shape[1:]}")
+            self.weights = weights.to(self.dev).contiguous()
+        else:
+            self.weights = t.from_numpy(_lib.sample_weights_array(weights, shape)).to(self.dev)
+        return self
+
+    def _plan_worlds(self) -> np.ndarray:
+        return np.unique(self.desc.view(self.torch.int32)[:, 0].cpu().numpy())
+
     def nfree(self) -> np.ndarray:
         return self.rowcum[:, self.W].cpu().numpy()
 
@@ -435,8 +486,10 @@ class DeviceBatch:
         return self
 
     def seed_samples(self, seeds: Sequence[int]):
-        """Sample streams on the device from numpy-compatible PCG64 (rrt.py:85,231-240)."""
+        """Sample streams on the device from numpy-compatible PCG64 (rrt.py:85,231-240); weighted after set_sample_weights."""
         t = self.torch
+        if self.weights is not None:
+            return self._seed_weighted(seeds)
         self._require_free_cells()
         st = t.from_numpy(seed_states(seeds).view(np.int64)).to(self.dev)
         self.samples = self._empty((self.nplans, self.n, 2), t.int16)
@@ -444,6 +497,26 @@ class DeviceBatch:
             _lib.check(self.L.rrtk_sample_streams(self._p(self.bits), self._p(self.rowcum), self.W, self.H, self._p(self.desc),
                                                   self.nplans, self._p(st), self.n, self._p(self.samples), self._stream()),
                        "sample_streams")
+        return self
+
+    def _seed_weighted(self, seeds: Sequence[int]):
+        """seed_samples with weight maps: the index of the current ``bits`` (rrtk_weight_index), its totals checked on the host
+        (a world whose free cells weigh nothing has nothing to draw), then rrtk_sample_streams_weighted."""
+        t = self.torch
+        nw = int(self.bits.shape[0])
+        index = self._empty((int(self.L.rrtk_weight_index_bytes(nw, self.W, self.H)),), t.uint8)
+        st = t.from_numpy(seed_states(seeds).view(np.int64)).to(self.dev)
+        self.samples = self._empty((self.nplans, self.n, 2), t.int16)
+        with t.cuda.device(self.dev):
+            _lib.check(self.L.rrtk_weight_index(self._p(self.bits), self._p(self.weights), nw, self.W, self.H, self._p(index), self._stream()),
+                       "weight_index")
+            tot = index[: 8 * nw].view(t.int64).cpu().numpy()
+            empty = [w for w in self._plan_worlds() if tot[w] <= 0]
+            if empty:
+                raise ValueError("world %d has no weight on its free cells: nothing to sample" % int(empty[0]))
+            _lib.check(self.L.rrtk_sample_streams_weighted(self._p(self.bits), self._p(self.weights), self._p(index), nw, self.W, self.H,
+                                                           self._p(self.desc), self.nplans, self._p(st), None, self.n, self._p(self.samples),
+                                                           self._stream()), "sample_streams_weighted")
         return self
 
     def _words(self, a, cols, dtype, name):
@@ -478,6 +551,9 @@ class DeviceBatch:
         t = self.torch
         if not self._is_informed():
             raise ValueError("seed_informed is for informed batches")
+        if self.weights is not None:
+            raise ValueError("seed_informed replays uniform free-space draws (rrtk_ball_streams): weighted informed batches are "
+                             "not supported (clear the weights with set_sample_weights(None))")
         self._require_free_cells()
         P, n = self.nplans, self.n
         st = self._words(states, 4, t.int64, "states")

@@ -53,6 +53,10 @@ int argsort_launch(const int64_t *, int, int32_t *, void *, size_t, cudaStream_t
 size_t argsort_scratch(int);
 int sample_streams_launch(const uint32_t *, const int32_t *, int, int, const rrtk_plan_desc *, int, const uint64_t *, int,
                           int16_t *, int, cudaStream_t, uint64_t * = nullptr, uint32_t * = nullptr);
+size_t weight_index_bytes(int, int, int);
+int weight_index_launch(const uint32_t *, const uint8_t *, int, int, int, void *, cudaStream_t);
+int weighted_streams_launch(const uint32_t *, const uint8_t *, const void *, int, int, int, const rrtk_plan_desc *, int, uint64_t *, uint32_t *,
+                            int, int16_t *, int, cudaStream_t);
 int ball_streams_launch(const int32_t *, int, const rrtk_plan_desc *, int, int, const uint64_t *, const uint32_t *, const int64_t *, int,
                         double *, uint64_t *, uint32_t *, cudaStream_t);
 int plan_launch(int, const uint32_t *, int, int, const rrtk_plan_desc *, int, int, double, double, const int16_t *,
@@ -154,6 +158,7 @@ struct PipeSlot {
     DevBuf og, bits, rowcum, plans, samples, state, balls, pts, cost, parent, stats, ell;
     DevBuf path, xy, len, pcost;                // path records (RRTK_OUT_PATHS)
     DevBuf heads, head_out, elen, scratch2, phead;   // K8 chunks (rrtk_ctx_plan2_worlds)
+    DevBuf windex;                              // RRTK_SEED_WEIGHTS: weight index of the chunk's worlds
     std::vector<rrtk_plan_desc> desc;
 };
 constexpr int kPipeSlots = 5;
@@ -176,6 +181,10 @@ struct rrtk_ctx {
     cudaStream_t pipe_prep = nullptr, pipe_post = nullptr;
     int32_t *pin_nfree = nullptr;               // pinned: free cells per world of a pipelined call (seed mode checks them)
     size_t pin_nfree_cap = 0;
+    DevBuf weights;                             // rrtk_ctx_set_sample_weights: w_nworlds (w_W, w_H) uint8 maps (w_nworlds 0: none)
+    int w_nworlds = 0, w_W = 0, w_H = 0;
+    int64_t *pin_wtot = nullptr;                // pinned: weight totals per world of a pipelined RRTK_SEED_WEIGHTS call
+    size_t pin_wtot_cap = 0;
 };
 
 // ---- host checks of the plan entries ---------------------------------------------------------------
@@ -237,6 +246,19 @@ static int require_free_cells(const int32_t *nfree, int nworlds, const rrtk_plan
         const int w = h_plans[p].world;
         if (w >= 0 && w < nworlds && nfree[w] <= 0) {
             set_error("%s: world %d of plan %d has no free cell to sample", who, w, p);
+            return RRTK_ERR_INVALID;
+        }
+    }
+    return RRTK_OK;
+}
+
+// RRTK_SEED_WEIGHTS draws integers(0, T): a world whose free cells carry no weight has nothing to draw (numpy raises)
+static int require_weight(const int64_t *tot, int nworlds, const rrtk_plan_desc *h_plans, int nplans, const char *who)
+{
+    for (int p = 0; p < nplans; ++p) {
+        const int w = h_plans[p].world;
+        if (w >= 0 && w < nworlds && tot[w] <= 0) {
+            set_error("%s: world %d of plan %d has no weight on its free cells (sample weights total 0)", who, w, p);
             return RRTK_ERR_INVALID;
         }
     }
@@ -306,6 +328,7 @@ struct PipeCall {
     const int16_t *samples;                     // exactly one of samples / state (seed mode)
     const uint64_t *state;
     const double *balls;                        // host unit-disc draws of informed plans, or NULL
+    const uint8_t *weights;                     // RRTK_SEED_WEIGHTS: the context's device weight maps, one per world, or NULL
     bool in_bits, trees, paths, seed_balls;
     bool ell;                                   // the plan kernel writes ellipse budgets into the slot's ell buffer
     int first_col;                              // stats column of the first-solution iteration (RRTK_SEED_BALLS)
@@ -334,13 +357,14 @@ static int pipe_slot_init(rrtk_ctx *c, PipeSlot &s)
     return RRTK_OK;
 }
 
-static int pipe_nfree_reserve(rrtk_ctx *c, size_t nworlds)
+template <class T>
+static int pin_reserve(T *&p, size_t &cap, size_t count)
 {
-    if (nworlds <= c->pin_nfree_cap) return RRTK_OK;
-    if (c->pin_nfree) cudaFreeHost(c->pin_nfree);
-    c->pin_nfree = nullptr; c->pin_nfree_cap = 0;
-    RRTK_CUDA(cudaHostAlloc(reinterpret_cast<void **>(&c->pin_nfree), nworlds * sizeof(int32_t), cudaHostAllocDefault));
-    c->pin_nfree_cap = nworlds;
+    if (count <= cap) return RRTK_OK;
+    if (p) cudaFreeHost(p);
+    p = nullptr; cap = 0;
+    RRTK_CUDA(cudaHostAlloc(reinterpret_cast<void **>(&p), count * sizeof(T), cudaHostAllocDefault));
+    cap = count;
     return RRTK_OK;
 }
 
@@ -398,7 +422,8 @@ static int pipe_run(rrtk_ctx *c, const PipeCall &a, int first_chunk, int chunk_p
         if (rc != RRTK_OK && status == RRTK_OK) status = rc;
         return rc == RRTK_OK;
     };
-    if (a.state) RRTK_TRY(pipe_nfree_reserve(c, (size_t)a.nworlds));
+    if (a.state && !a.weights) RRTK_TRY(pin_reserve(c->pin_nfree, c->pin_nfree_cap, (size_t)a.nworlds));
+    if (a.weights) RRTK_TRY(pin_reserve(c->pin_wtot, c->pin_wtot_cap, (size_t)a.nworlds));
     const bool balls = a.balls || a.seed_balls;                                   // the plan kernel reads unit-disc draws
     const size_t nslots = starts.size() - 1 < (size_t)kPipeSlots ? starts.size() - 1 : (size_t)kPipeSlots;
     for (size_t k = 0; k < nslots && status == RRTK_OK; ++k) {
@@ -412,6 +437,7 @@ static int pipe_run(rrtk_ctx *c, const PipeCall &a, int first_chunk, int chunk_p
         if (ok && !a.in_bits) ok = rrtk_ok(s.og.reserve(cells * max_nw));
         if (ok && balls) ok = rrtk_ok(s.balls.reserve(max_m * n * 16));
         if (ok && a.ell) ok = rrtk_ok(s.ell.reserve(rows1 * max_m * 8));
+        if (ok && a.weights) ok = rrtk_ok(s.windex.reserve(weight_index_bytes((int)max_nw, W, H)));
         if (ok && a.paths)
             ok = rrtk_ok(s.path.reserve(max_m * a.path_cap * 4)) && rrtk_ok(s.xy.reserve(max_m * a.path_cap * 4)) &&
                  rrtk_ok(s.len.reserve(max_m * 4)) && rrtk_ok(s.pcost.reserve(max_m * 8));
@@ -449,6 +475,14 @@ static int pipe_run(rrtk_ctx *c, const PipeCall &a, int first_chunk, int chunk_p
         if (!cuda_ok(cudaMemcpyAsync(s.plans.p, s.desc.data(), sizeof(rrtk_plan_desc) * m, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync(plans)")) break;
         if (a.samples) {
             if (!cuda_ok(cudaMemcpyAsync(s.samples.p, a.samples + (size_t)p0 * n * 2, (size_t)m * n * 4, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync(samples)")) break;
+        } else if (a.weights) {
+            // the index of the chunk's worlds on their grids, its totals down for the check after the drain, then the weighted sampler
+            const uint8_t *wmaps = a.weights + cells * w0;
+            if (!rrtk_ok(weight_index_launch(s.bits.as<uint32_t>(), wmaps, nw, W, H, s.windex.p, st))) break;
+            if (!cuda_ok(cudaMemcpyAsync(c->pin_wtot + w0, s.windex.p, (size_t)nw * 8, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(weight totals)")) break;
+            if (!cuda_ok(cudaMemcpyAsync(s.state.p, a.state + (size_t)p0 * 4, (size_t)m * 32, cudaMemcpyHostToDevice, st), "cudaMemcpyAsync(state)")) break;
+            if (!rrtk_ok(weighted_streams_launch(s.bits.as<uint32_t>(), wmaps, s.windex.p, nw, W, H, s.plans.as<rrtk_plan_desc>(), m,
+                                                 s.state.as<uint64_t>(), nullptr, n, s.samples.as<int16_t>(), di->optin, st))) break;
         } else {
             if (!rrtk_ok(free_rows_launch(s.bits.as<uint32_t>(), nw, W, H, s.rowcum.as<int32_t>(), st))) break;
             if (!cuda_ok(cudaMemcpy2DAsync(c->pin_nfree + w0, 4, s.rowcum.as<int32_t>() + W, (size_t)(W + 1) * 4, 4, nw, cudaMemcpyDeviceToHost, st),
@@ -514,7 +548,8 @@ static int pipe_run(rrtk_ctx *c, const PipeCall &a, int first_chunk, int chunk_p
     }
     for (cudaEvent_t e : tev) cudaEventDestroy(e);
     // seed mode: the free-cell counts came down with the chunks, so a world without a free cell is found only now
-    if (status == RRTK_OK && a.state) status = require_free_cells(c->pin_nfree, a.nworlds, a.plans, a.nplans, a.who);
+    if (status == RRTK_OK && a.state && !a.weights) status = require_free_cells(c->pin_nfree, a.nworlds, a.plans, a.nplans, a.who);
+    if (status == RRTK_OK && a.weights) status = require_weight(c->pin_wtot, a.nworlds, a.plans, a.nplans, a.who);
     if (status == RRTK_OK && a.seed_balls) status = pipe_require_rotations(a.plans, a.stats, a.nplans, a.first_col, a.who);
     return status;
 }
@@ -773,6 +808,32 @@ int rrtk_sample_streams_carry(const uint32_t *d_bits, const int32_t *d_rowcum, i
                                  d_state, d_carry);
 }
 
+size_t rrtk_weight_index_bytes(int nworlds, int W, int H)
+{
+    if (nworlds < 0 || W < 1 || H < 1) return 0;
+    return weight_index_bytes(nworlds, W, H);
+}
+
+int rrtk_weight_index(const uint32_t *d_bits, const uint8_t *d_weights, int nworlds, int W, int H, void *d_index, void *stream)
+{
+    RRTK_REQUIRE(nworlds >= 0 && (nworlds == 0 || (d_bits && d_weights && d_index)), "rrtk_weight_index: null pointer or negative count");
+    RRTK_TRY(check_grid_dims(W, H, 16384));
+    return weight_index_launch(d_bits, d_weights, nworlds, W, H, d_index, (cudaStream_t)stream);
+}
+
+int rrtk_sample_streams_weighted(const uint32_t *d_bits, const uint8_t *d_weights, const void *d_index, int nworlds, int W, int H,
+                                 const rrtk_plan_desc *d_plans, int nplans, uint64_t *d_state, uint32_t *d_carry, int n, int16_t *d_samples,
+                                 void *stream)
+{
+    RRTK_REQUIRE(d_bits && d_weights && d_index && d_plans && d_state && d_samples && nworlds >= 1 && nplans >= 0 && n >= 0,
+                 "rrtk_sample_streams_weighted: bad argument");
+    RRTK_TRY(check_grid_dims(W, H, 16384));
+    DevInfo *d;
+    RRTK_TRY(dev_info(&d));
+    return weighted_streams_launch(d_bits, d_weights, d_index, nworlds, W, H, d_plans, nplans, d_state, d_carry, n, d_samples, d->optin,
+                                   (cudaStream_t)stream);
+}
+
 int rrtk_ball_streams(const int32_t *d_rowcum, int W, const rrtk_plan_desc *d_plans, int nplans, int n, const uint64_t *d_state,
                       const uint32_t *d_carry, const int64_t *d_first, int first_stride, double *d_balls, uint64_t *d_state_out,
                       uint32_t *d_carry_out, void *stream)
@@ -905,6 +966,7 @@ int rrtk_destroy(rrtk_ctx *c)
         if (p.done) cudaEventDestroy(p.done);
     }
     if (c->pin_nfree) cudaFreeHost(c->pin_nfree);
+    if (c->pin_wtot) cudaFreeHost(c->pin_wtot);
     if (c->pipe_prep) cudaStreamDestroy(c->pipe_prep);
     if (c->pipe_post) cudaStreamDestroy(c->pipe_post);
     if (c->stream) cudaStreamDestroy(c->stream);
@@ -922,6 +984,41 @@ static int ctx_index_worlds(rrtk_ctx *c, int nworlds, int W, int H, int32_t *h_n
     RRTK_CUDA(cudaStreamSynchronize(c->stream));
     if (h_nfree) memcpy(h_nfree, c->nfree.data(), (size_t)nworlds * 4);
     c->W = W; c->H = H; c->nworlds = nworlds;
+    return RRTK_OK;
+}
+
+int rrtk_ctx_set_sample_weights(rrtk_ctx *c, const uint8_t *h_weights, int nworlds, int W, int H)
+{
+    RRTK_REQUIRE(c && nworlds >= 0, "rrtk_ctx_set_sample_weights: null context or negative count");
+    if (!h_weights || nworlds == 0) {
+        c->weights.release();
+        c->w_nworlds = c->w_W = c->w_H = 0;
+        return RRTK_OK;
+    }
+    RRTK_TRY(check_grid_dims(W, H, 16384));
+    c->w_nworlds = 0;
+    const size_t bytes = (size_t)nworlds * W * H;
+    RRTK_TRY(c->weights.reserve(bytes));
+    RRTK_CUDA(cudaMemcpyAsync(c->weights.p, h_weights, bytes, cudaMemcpyHostToDevice, c->stream));
+    RRTK_CUDA(cudaStreamSynchronize(c->stream));
+    c->w_nworlds = nworlds; c->w_W = W; c->w_H = H;
+    return RRTK_OK;
+}
+
+// RRTK_SEED_WEIGHTS of a pipelined call: the context's weight maps, checked against the call (NULL without the flag)
+static int pipe_weights(const rrtk_ctx *c, int flags, const uint64_t *h_state, int nworlds, int W, int H, const char *who, const uint8_t **out)
+{
+    *out = nullptr;
+    if (!(flags & RRTK_SEED_WEIGHTS)) return RRTK_OK;
+    if (!h_state) { set_error("%s: RRTK_SEED_WEIGHTS needs seed mode (h_state)", who); return RRTK_ERR_INVALID; }
+    if (flags & RRTK_SEED_BALLS) { set_error("%s: RRTK_SEED_WEIGHTS cannot be combined with RRTK_SEED_BALLS (the ellipse phase replays uniform draws)", who); return RRTK_ERR_INVALID; }
+    if (c->w_nworlds == 0) { set_error("%s: RRTK_SEED_WEIGHTS without weights (rrtk_ctx_set_sample_weights)", who); return RRTK_ERR_INVALID; }
+    if (c->w_nworlds != nworlds || c->w_W != W || c->w_H != H) {
+        set_error("%s: the sample weights are %d maps of (%d, %d), the call has %d worlds of (%d, %d)", who, c->w_nworlds, c->w_W, c->w_H,
+                  nworlds, W, H);
+        return RRTK_ERR_INVALID;
+    }
+    *out = static_cast<const uint8_t *>(c->weights.p);
     return RRTK_OK;
 }
 
@@ -1132,6 +1229,8 @@ int rrtk_ctx_plan_worlds2(rrtk_ctx *c, int kind, const void *h_grids, int nworld
     RRTK_REQUIRE(kind != RRTK_INFORMED || !out_trees || h_ell_c, "rrtk_ctx_plan_worlds2: informed trees need h_ell_c");
     RRTK_REQUIRE(nworlds >= 1 && nplans >= 0 && n >= 1 && n <= 65534, "rrtk_ctx_plan_worlds2: need nworlds >= 1, nplans >= 0, 1 <= n <= 65534");
     RRTK_TRY(check_grid_dims(W, H, 16384));
+    const uint8_t *weights;
+    RRTK_TRY(pipe_weights(c, flags, h_state, nworlds, W, H, "rrtk_ctx_plan_worlds2", &weights));
     if (nplans == 0) return RRTK_OK;
     RRTK_TRY(check_plan_descs(h_plans, nplans, nworlds, W, H, "rrtk_ctx_plan_worlds2", 0));
     RRTK_TRY(check_samples(h_samples, nplans, n, W, H));
@@ -1157,7 +1256,7 @@ int rrtk_ctx_plan_worlds2(rrtk_ctx *c, int kind, const void *h_grids, int nworld
     a.who = "rrtk_ctx_plan_worlds2";
     a.grids = h_grids; a.nworlds = nworlds; a.W = W; a.H = H;
     a.plans = h_plans; a.nplans = nplans; a.n = n;
-    a.samples = h_samples; a.state = h_state; a.balls = informed ? h_balls : nullptr;
+    a.samples = h_samples; a.state = h_state; a.balls = informed ? h_balls : nullptr; a.weights = weights;
     a.in_bits = in_bits; a.trees = out_trees; a.paths = out_paths; a.seed_balls = seed_balls;
     a.ell = informed; a.first_col = RRTK_STAT_FIRST_SOL_ITER;
     a.pts = h_pts; a.cost = h_cost; a.parent = h_parent;
@@ -1718,6 +1817,8 @@ int rrtk_ctx_plan2_worlds(rrtk_ctx *c, const rrtk_plan2_cfg *cfg, const void *h_
     RRTK_REQUIRE((h_samples != nullptr) != (h_state != nullptr), "rrtk_ctx_plan2_worlds: pass exactly one of h_samples / h_state");
     RRTK_REQUIRE(nworlds >= 1 && nplans >= 0 && n >= 1 && n <= 65534, "rrtk_ctx_plan2_worlds: need nworlds >= 1, nplans >= 0, 1 <= n <= 65534");
     RRTK_TRY(check_grid_dims(W, H, 16384));
+    const uint8_t *weights;
+    RRTK_TRY(pipe_weights(c, flags, h_state, nworlds, W, H, "rrtk_ctx_plan2_worlds", &weights));
     if (nplans == 0) return RRTK_OK;
     const bool dub = cfg->model == RRTK_MODEL_DUBINS;
     RRTK_TRY(check_plan_descs(h_plans, nplans, nworlds, W, H, "rrtk_ctx_plan2_worlds", dub ? cfg->nheadings : 0));
@@ -1737,6 +1838,7 @@ int rrtk_ctx_plan2_worlds(rrtk_ctx *c, const rrtk_plan2_cfg *cfg, const void *h_
     a.grids = h_grids; a.nworlds = nworlds; a.W = W; a.H = H;
     a.plans = h_plans; a.nplans = nplans; a.n = n;
     a.samples = h_samples; a.state = h_state; a.balls = cfg->informed ? cfg->balls : nullptr;     // host arrays in this form of the call
+    a.weights = weights;
     a.in_bits = in_bits; a.trees = out_trees; a.paths = out_paths; a.seed_balls = seed_balls;
     a.ell_c = cfg->informed ? cfg->ell_c : nullptr; a.ell = a.ell_c != nullptr; a.first_col = RRTK_STAT2_FIRST_SOL;
     a.pts = h_pts; a.cost = h_cost; a.parent = h_parent;

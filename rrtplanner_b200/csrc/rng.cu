@@ -60,6 +60,23 @@ struct Pcg64 {
         }
         return (uint32_t)(m >> 32);
     }
+    // Generator.integers(0, bound) for any bound >= 1 (a weighted stream's total): 32-bit Lemire below 2^32, the raw
+    // buffered 32-bit half at exactly 2^32, 64-bit Lemire on next64 above (which leaves the buffered half alone)
+    __device__ __forceinline__ unsigned long long bounded(unsigned long long bound)
+    {
+        if (bound < 0x100000000ull) return bounded((uint32_t)bound);
+        if (bound == 0x100000000ull) return next32();
+        unsigned long long v = next64();
+        unsigned long long left = v * bound;
+        if (left < bound) {
+            const unsigned long long thr = (0ull - bound) % bound;
+            while (left < thr) {
+                v = next64();
+                left = v * bound;
+            }
+        }
+        return __umul64hi(v, bound);
+    }
 };
 
 // rowcum may live in shared memory (the parallel kernel stages it) or in global memory
@@ -139,163 +156,418 @@ __device__ __forceinline__ void pcg_jump(Pcg64 &g, unsigned long long delta) { p
 constexpr int kSampleThreads = RRTK_SAMPLE_THREADS;
 constexpr int kRawSlack = 62;          // raw 32-bit values generated beyond n; more rejections than that -> sequential path
 
+// 32-bit words of the raw window of the parallel sampler: n + kRawSlack raw 32-bit values for 32-bit ranks; for 64-bit ranks
+// also n + kRawSlack / 2 raw next64 outputs (64-bit Lemire), i.e. 2 n + kRawSlack words.  Plus 4 words of slack.
+__host__ __device__ __forceinline__ int raw_window_words(int n, int rank_words) { return n * rank_words + kRawSlack + 4; }   // n <= 65534
+
+// ---- the select step: where a bounded draw lands ------------------------------------------------------------------
+// A sampler draws n ranks from integers(0, bound) and maps each rank to a cell.  The generator, the rejection compaction
+// and the sequential fallback below are shared; the select policy supplies the bound of a world, what the parallel kernel
+// stages in shared memory for it, and the rank -> cell map.
+//   bound_t / rank_t   integer types of the bound and of a rank
+//   stage_words(W)     32-bit words of shared memory the parallel kernel stages per plan
+//   bound(world, W)    the plan's bound (a bound <= 1 draws 0 without touching the generator, as numpy does)
+//   stage(world, W, s, tid)          fill the staged words (block-wide; read after the kernel's barriers)
+//   unstaged(world, W)               the same words in global memory, for the sequential kernel (which stages nothing)
+//   cell(world, W, H, s, k)          rank k -> cell; s = the staged words or their global copy
+
+// Uniform: free[integers(0, nfree)], rank = index into the row-major list of free cells (rowcum + bit grid).
+struct UniformSelect {
+    using bound_t = uint32_t;
+    using rank_t = uint32_t;
+    const uint32_t *bits;
+    const int *rowcum;
+    static size_t stage_words(int W) { return (size_t)W + 1; }
+    __device__ __forceinline__ uint32_t bound(int world, int W) const { return (uint32_t)__ldg(rowcum + (size_t)world * (W + 1) + W); }
+    __device__ __forceinline__ void stage(int world, int W, uint32_t *s, int tid) const
+    {
+        const int *rc = rowcum + (size_t)world * (W + 1);
+        for (int x = tid; x <= W; x += kSampleThreads) s[x] = (uint32_t)__ldg(rc + x);
+    }
+    __device__ __forceinline__ const uint32_t *unstaged(int world, int W) const
+    {
+        return reinterpret_cast<const uint32_t *>(rowcum + (size_t)world * (W + 1));
+    }
+    __device__ __forceinline__ short2 cell(int world, int W, int H, const uint32_t *s, uint32_t k) const
+    {
+        return rank_to_cell(bits + (size_t)world * grid_words(W, H), reinterpret_cast<const int *>(s), W, tiles_y(H), (int)k);
+    }
+};
+
+// Weighted: the effective weight of a cell is its uint8 weight where the grid is free, else 0; rank k of integers(0, T),
+// T = the world's total, lands on the cell whose exclusive prefix of effective weights (row-major) is <= k < prefix + weight
+// (np.searchsorted(cumsum, k, side="right")).  The index (rrtk_weight_index) holds, after the nworlds totals, per world
+// the W + 1 int64 prefixes of the row totals and per row the uint32 prefix at each 32-cell chunk (one bit-grid word).
+struct WeightIndex {
+    long long *tot;                    // nworlds totals T
+    long long *rows;                   // world w: rows + w * (W + 1), rows[x] = weight of rows < x
+    uint32_t *chunks;                  // world w, row x: chunks + (w * W + x) * TY, entry t = weight of cells y < 32 t of the row
+    __host__ __device__ WeightIndex(void *base, int nworlds, int W, int H)
+    {
+        tot = reinterpret_cast<long long *>(base);
+        rows = tot + nworlds;
+        chunks = reinterpret_cast<uint32_t *>(rows + (size_t)nworlds * (W + 1));
+        (void)H;
+    }
+    static size_t bytes(int nworlds, int W, int H)
+    {
+        return 8 * ((size_t)nworlds + (size_t)nworlds * (W + 1)) + 4 * (size_t)nworlds * W * tiles_y(H);
+    }
+};
+
+struct WeightedSelect {
+    using bound_t = unsigned long long;
+    using rank_t = unsigned long long;
+    const uint32_t *bits;
+    const uint8_t *weights;
+    const long long *tot, *rows;
+    const uint32_t *chunks;
+    static size_t stage_words(int) { return 0; }
+    __device__ __forceinline__ unsigned long long bound(int world, int) const { return (unsigned long long)__ldg(tot + world); }
+    __device__ __forceinline__ void stage(int, int, uint32_t *, int) const {}
+    __device__ __forceinline__ const uint32_t *unstaged(int, int) const { return nullptr; }
+    __device__ __forceinline__ short2 cell(int world, int W, int H, const uint32_t *, unsigned long long k) const
+    {
+        const int TY = tiles_y(H);
+        const long long *rp = rows + (size_t)world * (W + 1);
+        int lo = 0, hi = W;                                   // largest x with rp[x] <= k (rp[W] = T > k)
+        while (hi - lo > 1) {
+            const int mid = (lo + hi) >> 1;
+            if ((unsigned long long)__ldg(rp + mid) <= k) lo = mid; else hi = mid;
+        }
+        uint32_t rem = (uint32_t)(k - (unsigned long long)__ldg(rp + lo));
+        const uint32_t *cp = chunks + ((size_t)world * W + lo) * TY;
+        int a = 0, b = TY;                                    // largest chunk t with cp[t] <= rem
+        while (b - a > 1) {
+            const int mid = (a + b) >> 1;
+            if (__ldg(cp + mid) <= rem) a = mid; else b = mid;
+        }
+        rem -= __ldg(cp + a);
+        const uint32_t occ = __ldg(bits + (size_t)world * grid_words(W, H) + word_index(lo, a << 5, TY));
+        const uint8_t *wr = weights + ((size_t)world * W + lo) * H;
+        int y = a << 5;
+        const int last = min(H, y + 32) - 1;
+        for (; y < last; ++y) {                               // at most 32 masked bytes; the last one takes what is left
+            const uint32_t e = ((occ >> (y & 31)) & 1u) ? 0u : (uint32_t)__ldg(wr + y);
+            if (rem < e) break;
+            rem -= e;
+        }
+        return make_short2((short)lo, (short)y);
+    }
+};
+
+// Lemire's 32-bit threshold (2^32 - bound) mod bound; for bound = 2^32 it is 0 and the rank is the raw value itself
+__device__ __forceinline__ uint32_t lemire32_threshold(uint32_t bound) { return (0xffffffffu - (bound - 1u)) % bound; }
+__device__ __forceinline__ uint32_t lemire32_threshold(unsigned long long bound) { return (uint32_t)((0x100000000ull - bound) % bound); }
+__device__ __forceinline__ bool needs_next64(uint32_t) { return false; }
+__device__ __forceinline__ bool needs_next64(unsigned long long bound) { return bound > 0x100000000ull; }
+
+// 64-bit outputs k0 .. k1-1 of the generator, each thread its own slice [tid * per, ...) reached by jump-ahead
+template <class Store>
+__device__ __forceinline__ void raw_slices(const Pcg64 &g0, int n64, int tid, Store store)
+{
+    const int per = (n64 + kSampleThreads - 1) / kSampleThreads;      // outputs per thread
+    Pcg64 g = g0;
+    const int k0 = tid * per;
+    if (k0 < n64) {
+        pcg_jump(g, (unsigned long long)k0);
+        const int k1 = min(n64, k0 + per);
+        for (int k = k0; k < k1; ++k) store(k, g.next64());
+    }
+}
+
+// Lemire's rejection loop as a block compaction of the raw values s_raw[0 .. total): thread t owns raw indices
+// [t * span, (t + 1) * span); accept(raw, rank) says whether a raw value is kept and gives its rank.  Writes the first n ranks
+// and returns (block-uniformly) the raw values they used up, or -1 when the window held fewer than n accepted values.
+template <class Raw, class Rank, class Accept>
+__device__ __forceinline__ int compact_ranks(const Raw *s_raw, int total, int n, Rank *s_rank, Accept accept, int *s_warp, int *s_consumed,
+                                             int tid)
+{
+    const int lane = tid & 31, warp = tid >> 5;
+    const int span = (total + kSampleThreads - 1) / kSampleThreads;
+    const int r0 = tid * span, r1 = min(total, r0 + span);
+    Rank rank;
+    int acc = 0;
+    for (int r = r0; r < r1; ++r) acc += accept(s_raw[r], rank) ? 1 : 0;
+    int incl = acc;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int v = __shfl_up_sync(RRTK_FULL, incl, o);
+        if (lane >= o) incl += v;
+    }
+    if (lane == 31) s_warp[warp] = incl;
+    if (tid == 0) *s_consumed = -1;
+    __syncthreads();
+    int before = incl - acc;
+    for (int w = 0; w < warp; ++w) before += s_warp[w];
+    for (int r = r0; r < r1; ++r) {
+        if (accept(s_raw[r], rank)) {
+            if (before < n) s_rank[before] = rank;
+            if (before == n - 1) *s_consumed = r + 1;
+            ++before;
+        }
+    }
+    __syncthreads();
+    return *s_consumed;
+}
+
+__device__ __forceinline__ void store_state(unsigned long long *state_out, int plan, const Pcg64 &g)
+{
+    state_out[4 * plan] = g.hi; state_out[4 * plan + 1] = g.lo; state_out[4 * plan + 2] = g.inc_hi; state_out[4 * plan + 3] = g.inc_lo;
+}
+
 // one block per plan: the generator's raw outputs in parallel slices, Lemire's rejection as a compaction, then
 // ranks -> cells in parallel.  The sequential generator remains as the fallback for a stream with more than kRawSlack
-// rejections (probability ~ (n * nfree / 2^32)^62 / 62!).
+// rejections (probability ~ (n * bound / 2^32)^62 / 62!).  state_out / carry (optional) receive the generator after the
+// n draws; state_out may alias state.
+template <class Sel>
 __global__ void __launch_bounds__(kSampleThreads)
-sample_stream_kernel(const uint32_t *__restrict__ bits, const int *__restrict__ rowcum, int W, int H,
-                     const rrtk_plan_desc *__restrict__ plans, const unsigned long long *__restrict__ state, int n,
+sample_stream_kernel(Sel sel, int W, int H, const rrtk_plan_desc *__restrict__ plans, const unsigned long long *__restrict__ state, int n,
                      short2 *__restrict__ samples, unsigned long long *__restrict__ state_out, uint32_t *__restrict__ carry)
 {
+    using Bound = typename Sel::bound_t;
+    using Rank = typename Sel::rank_t;
     extern __shared__ uint32_t s_mem[];
-    uint32_t *s_rank = s_mem;                    // n bounded draws
-    uint32_t *s_raw = s_mem + n;                 // raw 32-bit values in the order numpy's next_uint32 hands them out
-    int *s_rowcum = reinterpret_cast<int *>(s_mem + 2 * n + kRawSlack + 4);      // W + 1 row offsets of this plan's world
+    constexpr int kRankWords = (int)(sizeof(Rank) / 4);
+    Rank *s_rank = reinterpret_cast<Rank *>(s_mem);                     // n bounded draws
+    uint32_t *s_raw = s_mem + kRankWords * n;                           // raw values in the order numpy hands them out
+    uint32_t *s_stage = s_mem + kRankWords * n + raw_window_words(n, kRankWords);   // what the select step stages for this plan's world
     __shared__ int s_warp[kSampleThreads / 32];
     __shared__ int s_consumed;                   // raw values used up by the n draws (-1: not enough generated)
-    const int plan = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int plan = blockIdx.x, tid = threadIdx.x;
     const int world = plans[plan].world;
-    const int *rc = rowcum + (size_t)world * (W + 1);
-    const uint32_t nfree = (uint32_t)__ldg(rc + W);
-    for (int x = tid; x <= W; x += kSampleThreads) s_rowcum[x] = __ldg(rc + x);    // visible after the barriers below
+    const Bound bound = sel.bound(world, W);
+    sel.stage(world, W, s_stage, tid);           // visible after the barriers below
     Pcg64 g0;
     g0.hi = state[4 * plan]; g0.lo = state[4 * plan + 1];
     g0.inc_hi = state[4 * plan + 2]; g0.inc_lo = state[4 * plan + 3];
     g0.has32 = false; g0.buf32 = 0;
     if (carry) { g0.has32 = carry[2 * plan] != 0; g0.buf32 = carry[2 * plan + 1]; }   // numpy's has_uint32 / uinteger
     const int off = g0.has32 ? 1 : 0;
-    if (nfree <= 1u) {                           // numpy returns the single value without touching the generator
+    if (bound <= 1u) {                           // numpy returns the single value without touching the generator
         for (int i = tid; i < n; i += kSampleThreads) s_rank[i] = 0;
-        if (tid == 0) {
-            if (state_out) { state_out[4 * plan] = g0.hi; state_out[4 * plan + 1] = g0.lo; state_out[4 * plan + 2] = g0.inc_hi; state_out[4 * plan + 3] = g0.inc_lo; }
+        if (tid == 0 && state_out) store_state(state_out, plan, g0);
+        __syncthreads();
+    } else if (needs_next64(bound)) {            // 64-bit Lemire: one raw next64 per candidate, the buffered half untouched
+        unsigned long long *s_raw64 = reinterpret_cast<unsigned long long *>(s_raw);
+        const int nraw = n + kRawSlack / 2;
+        raw_slices(g0, nraw, tid, [&](int k, unsigned long long v) { s_raw64[k] = v; });
+        __syncthreads();
+        const unsigned long long thr = (0ull - (unsigned long long)bound) % (unsigned long long)bound;
+        const int consumed = compact_ranks(s_raw64, nraw, n, s_rank, [&](unsigned long long v, Rank &rank) {
+            rank = (Rank)__umul64hi(v, (unsigned long long)bound);
+            return v * (unsigned long long)bound >= thr;
+        }, s_warp, &s_consumed, tid);
+        if (consumed < 0) {
+            if (tid == 0) {
+                Pcg64 g = g0;
+                for (int i = 0; i < n; ++i) s_rank[i] = (Rank)g.bounded(bound);
+                if (state_out) store_state(state_out, plan, g);
+            }
+        } else if (tid == 0 && state_out) {
+            Pcg64 g = g0;
+            pcg_jump(g, (unsigned long long)consumed);
+            store_state(state_out, plan, g);
         }
         __syncthreads();
     } else {
         const int nraw = n + kRawSlack;                                   // raw values wanted: indices 0 .. nraw-1
         const int n64 = (nraw - off + 1) >> 1;                            // 64-bit outputs that cover them
-        const int per = (n64 + kSampleThreads - 1) / kSampleThreads;      // outputs per thread
-        {
-            Pcg64 g = g0;
-            const int k0 = tid * per;
-            if (k0 < n64) {
-                pcg_jump(g, (unsigned long long)k0);
-                const int k1 = min(n64, k0 + per);
-                for (int k = k0; k < k1; ++k) {
-                    const unsigned long long v = g.next64();
-                    s_raw[off + 2 * k] = (uint32_t)v;
-                    s_raw[off + 2 * k + 1] = (uint32_t)(v >> 32);
-                }
-            }
-            if (tid == 0 && off) s_raw[0] = g0.buf32;
-        }
+        raw_slices(g0, n64, tid, [&](int k, unsigned long long v) {
+            s_raw[off + 2 * k] = (uint32_t)v;
+            s_raw[off + 2 * k + 1] = (uint32_t)(v >> 32);
+        });
+        if (tid == 0 && off) s_raw[0] = g0.buf32;
         __syncthreads();
-        // compaction: thread t owns raw indices [t * span, (t + 1) * span)
-        const int total = off + 2 * n64;                                  // raw values available (>= nraw)
-        const int span = (total + kSampleThreads - 1) / kSampleThreads;
-        const uint32_t thr = (0xffffffffu - (nfree - 1u)) % nfree;        // Lemire's threshold
-        const int r0 = tid * span, r1 = min(total, r0 + span);
-        int acc = 0;
-        for (int r = r0; r < r1; ++r) acc += ((uint32_t)((unsigned long long)s_raw[r] * nfree) >= thr) ? 1 : 0;
-        int incl = acc;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const int v = __shfl_up_sync(RRTK_FULL, incl, o);
-            if (lane >= o) incl += v;
-        }
-        if (lane == 31) s_warp[warp] = incl;
-        if (tid == 0) s_consumed = -1;
-        __syncthreads();
-        int before = incl - acc;
-        for (int w = 0; w < warp; ++w) before += s_warp[w];
-        for (int r = r0; r < r1; ++r) {
-            const unsigned long long m = (unsigned long long)s_raw[r] * nfree;
-            if ((uint32_t)m >= thr) {
-                if (before < n) s_rank[before] = (uint32_t)(m >> 32);
-                if (before == n - 1) s_consumed = r + 1;
-                ++before;
-            }
-        }
-        __syncthreads();
-        if (s_consumed < 0) {                    // not enough accepted values in the window: the plain sequential generator
+        const uint32_t thr = lemire32_threshold(bound);
+        const int consumed = compact_ranks(s_raw, off + 2 * n64, n, s_rank, [&](uint32_t v, Rank &rank) {
+            const unsigned long long m = (unsigned long long)v * bound;
+            rank = (Rank)(m >> 32);
+            return (uint32_t)m >= thr;
+        }, s_warp, &s_consumed, tid);
+        if (consumed < 0) {                      // not enough accepted values in the window: the plain sequential generator
             if (tid == 0) {
                 Pcg64 g = g0;
-                for (int i = 0; i < n; ++i) s_rank[i] = g.bounded(nfree);
-                if (state_out) { state_out[4 * plan] = g.hi; state_out[4 * plan + 1] = g.lo; state_out[4 * plan + 2] = g.inc_hi; state_out[4 * plan + 3] = g.inc_lo; }
+                for (int i = 0; i < n; ++i) s_rank[i] = g.bounded(bound);
+                if (state_out) store_state(state_out, plan, g);
                 if (carry) { carry[2 * plan] = g.has32 ? 1u : 0u; carry[2 * plan + 1] = g.buf32; }
             }
         } else if (tid == 0 && (state_out || carry)) {
             // the generator as the next plan() of the same planner object finds it (rrt.py:85: one rand_gen per object)
-            const int used = s_consumed - off;                            // raw values taken from fresh 64-bit outputs
+            const int used = consumed - off;                              // raw values taken from fresh 64-bit outputs
             const int out64 = (used + 1) >> 1;
             Pcg64 g = g0;
             pcg_jump(g, (unsigned long long)out64);
-            if (state_out) { state_out[4 * plan] = g.hi; state_out[4 * plan + 1] = g.lo; state_out[4 * plan + 2] = g.inc_hi; state_out[4 * plan + 3] = g.inc_lo; }
+            if (state_out) store_state(state_out, plan, g);
             if (carry) {
-                const bool half = used > 0 ? (used & 1) != 0 : g0.has32 && s_consumed == 0;
+                const bool half = used > 0 ? (used & 1) != 0 : g0.has32 && consumed == 0;
                 carry[2 * plan] = half ? 1u : 0u;
-                carry[2 * plan + 1] = half ? s_raw[s_consumed] : (used > 0 ? s_raw[s_consumed - 1] : g0.buf32);
+                carry[2 * plan + 1] = half ? s_raw[consumed] : (used > 0 ? s_raw[consumed - 1] : g0.buf32);
             }
         }
         __syncthreads();
     }
-    const uint32_t *g = bits + (size_t)world * grid_words(W, H);
-    const int TY = tiles_y(H);
     short2 *out = samples + (size_t)plan * n;
-    for (int i = tid; i < n; i += kSampleThreads) out[i] = rank_to_cell(g, s_rowcum, W, TY, (int)s_rank[i]);
+    for (int i = tid; i < n; i += kSampleThreads) out[i] = sel.cell(world, W, H, s_stage, s_rank[i]);
 }
 
 // n too large for the raw window in shared memory: thread 0 runs the generator sequentially
-__global__ void sample_stream_seq_kernel(const uint32_t *__restrict__ bits, const int *__restrict__ rowcum, int W, int H,
-                                         const rrtk_plan_desc *__restrict__ plans, const unsigned long long *__restrict__ state, int n,
-                                         short2 *__restrict__ samples, unsigned long long *__restrict__ state_out, uint32_t *__restrict__ carry)
+template <class Sel>
+__global__ void sample_stream_seq_kernel(Sel sel, int W, int H, const rrtk_plan_desc *__restrict__ plans,
+                                         const unsigned long long *__restrict__ state, int n, short2 *__restrict__ samples,
+                                         unsigned long long *__restrict__ state_out, uint32_t *__restrict__ carry)
 {
-    extern __shared__ uint32_t s_rank[];
+    using Rank = typename Sel::rank_t;
+    extern __shared__ uint32_t s_mem[];
+    Rank *s_rank = reinterpret_cast<Rank *>(s_mem);
     const int plan = blockIdx.x;
     const int world = plans[plan].world;
-    const int *rc = rowcum + (size_t)world * (W + 1);
-    const uint32_t nfree = (uint32_t)__ldg(rc + W);
+    const typename Sel::bound_t bound = sel.bound(world, W);
     if (threadIdx.x == 0) {
         Pcg64 g;
         g.hi = state[4 * plan]; g.lo = state[4 * plan + 1];
         g.inc_hi = state[4 * plan + 2]; g.inc_lo = state[4 * plan + 3];
         g.has32 = false; g.buf32 = 0;
         if (carry) { g.has32 = carry[2 * plan] != 0; g.buf32 = carry[2 * plan + 1]; }
-        for (int i = 0; i < n; ++i) s_rank[i] = nfree ? g.bounded(nfree) : 0;
-        if (state_out) {
-            state_out[4 * plan] = g.hi; state_out[4 * plan + 1] = g.lo;
-            state_out[4 * plan + 2] = g.inc_hi; state_out[4 * plan + 3] = g.inc_lo;
-        }
+        for (int i = 0; i < n; ++i) s_rank[i] = bound ? g.bounded(bound) : 0;
+        if (state_out) store_state(state_out, plan, g);
         if (carry) { carry[2 * plan] = g.has32 ? 1u : 0u; carry[2 * plan + 1] = g.buf32; }
     }
     __syncthreads();
-    const uint32_t *g = bits + (size_t)world * grid_words(W, H);
-    const int TY = tiles_y(H);
     short2 *out = samples + (size_t)plan * n;
-    for (int i = threadIdx.x; i < n; i += blockDim.x) out[i] = rank_to_cell(g, rc, W, TY, (int)s_rank[i]);
+    const uint32_t *rows = sel.unstaged(world, W);
+    for (int i = threadIdx.x; i < n; i += blockDim.x) out[i] = sel.cell(world, W, H, rows, s_rank[i]);
 }
 
-int sample_streams_launch(const uint32_t *d_bits, const int32_t *d_rowcum, int W, int H, const rrtk_plan_desc *d_plans,
-                          int nplans, const uint64_t *d_state, int n, int16_t *d_samples, int optin, cudaStream_t st,
-                          uint64_t *d_state_out, uint32_t *d_carry)
+template <class Sel>
+static int sample_launch(const Sel &sel, int W, int H, const rrtk_plan_desc *d_plans, int nplans, const uint64_t *d_state, int n,
+                         int16_t *d_samples, int optin, cudaStream_t st, uint64_t *d_state_out, uint32_t *d_carry)
 {
     if (nplans == 0 || n == 0) return RRTK_OK;
-    const size_t smem = ((size_t)2 * n + kRawSlack + 4 + W + 1) * 4;      // bounded draws + raw 32-bit values + row offsets
-    const size_t smem_seq = (size_t)n * 4;
+    const size_t rank_words = sizeof(typename Sel::rank_t) / 4;
+    const size_t smem = (n * rank_words + (size_t)raw_window_words(n, (int)rank_words) + Sel::stage_words(W)) * 4;   // draws + raw values + staged words
+    const size_t smem_seq = (size_t)n * rank_words * 4;
     const unsigned long long *st64 = reinterpret_cast<const unsigned long long *>(d_state);
+    unsigned long long *out64 = reinterpret_cast<unsigned long long *>(d_state_out);
+    short2 *out = reinterpret_cast<short2 *>(d_samples);
     if (smem <= (size_t)optin) {
-        RRTK_CUDA(cudaFuncSetAttribute(sample_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        sample_stream_kernel<<<nplans, kSampleThreads, smem, st>>>(d_bits, d_rowcum, W, H, d_plans, st64, n, reinterpret_cast<short2 *>(d_samples),
-                                                                  reinterpret_cast<unsigned long long *>(d_state_out), d_carry);
+        RRTK_CUDA(cudaFuncSetAttribute(sample_stream_kernel<Sel>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        sample_stream_kernel<Sel><<<nplans, kSampleThreads, smem, st>>>(sel, W, H, d_plans, st64, n, out, out64, d_carry);
     } else if (smem_seq <= (size_t)optin) {
-        RRTK_CUDA(cudaFuncSetAttribute(sample_stream_seq_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_seq));
-        sample_stream_seq_kernel<<<nplans, 128, smem_seq, st>>>(d_bits, d_rowcum, W, H, d_plans, st64, n, reinterpret_cast<short2 *>(d_samples),
-                                                               reinterpret_cast<unsigned long long *>(d_state_out), d_carry);
+        RRTK_CUDA(cudaFuncSetAttribute(sample_stream_seq_kernel<Sel>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_seq));
+        sample_stream_seq_kernel<Sel><<<nplans, 128, smem_seq, st>>>(sel, W, H, d_plans, st64, n, out, out64, d_carry);
     } else {
         set_error("sample stream of n=%d does not fit shared memory", n);
         return RRTK_ERR_CAPACITY;
     }
     RRTK_CUDA(cudaGetLastError());
     return RRTK_OK;
+}
+
+int sample_streams_launch(const uint32_t *d_bits, const int32_t *d_rowcum, int W, int H, const rrtk_plan_desc *d_plans,
+                          int nplans, const uint64_t *d_state, int n, int16_t *d_samples, int optin, cudaStream_t st,
+                          uint64_t *d_state_out, uint32_t *d_carry)
+{
+    return sample_launch(UniformSelect{d_bits, d_rowcum}, W, H, d_plans, nplans, d_state, n, d_samples, optin, st, d_state_out, d_carry);
+}
+
+// ---- weighted sampling: the index and the stream ------------------------------------------------------------------
+size_t weight_index_bytes(int nworlds, int W, int H) { return WeightIndex::bytes(nworlds, W, H); }
+
+// one warp per (world, row): lane t sums the effective weights of chunk t (+32, ...) -- the grid word is the mask -- then a
+// warp scan writes the chunk prefixes and the row total (into rows[x + 1], made a prefix by weight_rows_kernel)
+constexpr int kIndexWarps = 8;
+__global__ void __launch_bounds__(kIndexWarps * 32)
+weight_chunks_kernel(const uint32_t *__restrict__ bits, const uint8_t *__restrict__ weights, int nworlds, int W, int H, bool words4,
+                     WeightIndex ix)
+{
+    const int lane = threadIdx.x & 31;
+    const long long r = (long long)blockIdx.x * kIndexWarps + (threadIdx.x >> 5);
+    if (r >= (long long)nworlds * W) return;
+    const int world = (int)(r / W), x = (int)(r % W);
+    const int TY = tiles_y(H);
+    const uint32_t *g = bits + (size_t)world * grid_words(W, H);
+    const uint8_t *wr = weights + (size_t)r * H;
+    uint32_t *cp = ix.chunks + (size_t)r * TY;
+    uint32_t carry = 0;
+    for (int t0 = 0; t0 < TY; t0 += 32) {
+        const int t = t0 + lane;
+        uint32_t sum = 0;
+        if (t < TY) {
+            const uint32_t occ = __ldg(g + word_index(x, t << 5, TY));
+            const int y0 = t << 5, len = min(32, H - y0);
+            if (words4) {                         // every row starts 4-byte aligned: four cells per load
+                const uint32_t *w4 = reinterpret_cast<const uint32_t *>(wr + y0);
+                for (int j = 0; j < (len >> 2); ++j) {
+                    const uint32_t v = __ldg(w4 + j), m = occ >> (4 * j);
+#pragma unroll
+                    for (int b = 0; b < 4; ++b) sum += ((m >> b) & 1u) ? 0u : ((v >> (8 * b)) & 0xffu);
+                }
+            } else {
+                for (int j = 0; j < len; ++j) sum += ((occ >> j) & 1u) ? 0u : (uint32_t)__ldg(wr + y0 + j);
+            }
+        }
+        uint32_t incl = sum;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const uint32_t v = __shfl_up_sync(RRTK_FULL, incl, o);
+            if (lane >= o) incl += v;
+        }
+        if (t < TY) cp[t] = carry + incl - sum;
+        carry += __shfl_sync(RRTK_FULL, incl, 31);
+    }
+    if (lane == 0) ix.rows[(size_t)world * (W + 1) + x + 1] = carry;
+}
+
+// one block per world: rows[0] = 0 and the row totals in rows[1 .. W] become inclusive prefixes; tot[world] = rows[W]
+constexpr int kRowThreads = 1024;
+__global__ void __launch_bounds__(kRowThreads) weight_rows_kernel(int W, WeightIndex ix)
+{
+    __shared__ long long s_warp[kRowThreads / 32];
+    const int world = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    long long *rp = ix.rows + (size_t)world * (W + 1);
+    const int per = (W + kRowThreads - 1) / kRowThreads;
+    const int x0 = 1 + tid * per, x1 = min(W + 1, x0 + per);
+    long long acc = 0;
+    for (int x = x0; x < x1; ++x) acc += rp[x];
+    long long incl = acc;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const long long v = __shfl_up_sync(RRTK_FULL, incl, o);
+        if (lane >= o) incl += v;
+    }
+    if (lane == 31) s_warp[warp] = incl;
+    __syncthreads();
+    long long run = incl - acc;
+    for (int w = 0; w < warp; ++w) run += s_warp[w];
+    for (int x = x0; x < x1; ++x) { run += rp[x]; rp[x] = run; }
+    if (tid == 0) rp[0] = 0;
+    if (x0 <= W && W < x1) ix.tot[world] = run;
+    if (W == 0 && tid == 0) ix.tot[world] = 0;
+}
+
+int weight_index_launch(const uint32_t *d_bits, const uint8_t *d_weights, int nworlds, int W, int H, void *d_index, cudaStream_t st)
+{
+    if (nworlds == 0) return RRTK_OK;
+    WeightIndex ix(d_index, nworlds, W, H);
+    const long long warps = (long long)nworlds * W;
+    // the weights may start anywhere (a view into a caller's buffer): whole words only when the base and every row are aligned
+    const bool words4 = (H & 3) == 0 && (reinterpret_cast<uintptr_t>(d_weights) & 3) == 0;
+    weight_chunks_kernel<<<(unsigned)((warps + kIndexWarps - 1) / kIndexWarps), kIndexWarps * 32, 0, st>>>(d_bits, d_weights, nworlds, W, H,
+                                                                                                          words4, ix);
+    RRTK_CUDA(cudaGetLastError());
+    weight_rows_kernel<<<nworlds, kRowThreads, 0, st>>>(W, ix);
+    RRTK_CUDA(cudaGetLastError());
+    return RRTK_OK;
+}
+
+int weighted_streams_launch(const uint32_t *d_bits, const uint8_t *d_weights, const void *d_index, int nworlds, int W, int H,
+                            const rrtk_plan_desc *d_plans, int nplans, uint64_t *d_state, uint32_t *d_carry, int n, int16_t *d_samples,
+                            int optin, cudaStream_t st)
+{
+    WeightIndex ix(const_cast<void *>(d_index), nworlds, W, H);
+    const WeightedSelect sel{d_bits, d_weights, ix.tot, ix.rows, ix.chunks};
+    return sample_launch(sel, W, H, d_plans, nplans, d_state, n, d_samples, optin, st, d_carry ? d_state : nullptr, d_carry);
 }
 
 // ---- the ellipse-phase unit-disc stream of RRTStarInformed.plan (rrt.py:579-587, 694-701) -------------------------

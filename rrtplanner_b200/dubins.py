@@ -97,12 +97,12 @@ class RRTDubins(RRT):
     _STAR = False
 
     def __init__(self, og: np.ndarray, n: int, rho: float, nheadings: int = 16, ds: float = 1.0, costfn: callable = None,
-                 pbar: bool = True, seed: int = 0, *, robot_radius=None, body=None):
+                 pbar: bool = True, seed: int = 0, *, robot_radius=None, body=None, sample_weights=None):
         if body is not None and robot_radius is not None:
             raise ValueError("pass either body or robot_radius, not both (a disc is a body whose stencils are all the same disc)")
         self.body = None if body is None else np.asarray(body) != 0
         self._body_runs = None if body is None else body_runs(body)
-        super().__init__(og, n, costfn=costfn, pbar=pbar, seed=seed, robot_radius=robot_radius)
+        super().__init__(og, n, costfn=costfn, pbar=pbar, seed=seed, robot_radius=robot_radius, sample_weights=sample_weights)
         if not (0 < rho <= 16384 and 0.05 <= ds <= 16384):
             raise ValueError("need 0 < rho <= 16384 and 0.05 <= ds <= 16384 (cells)")
         if not (1 <= int(nheadings) <= 255):
@@ -110,11 +110,11 @@ class RRTDubins(RRT):
         self.rho, self.nheadings, self.ds = float(rho), int(nheadings), float(ds)
         self.r_rewire = 0.0
         self.rewire = False
-        if self.body is not None:
-            self.free = self._body_free(og)
 
-    def _body_free(self, og) -> np.ndarray:
-        """Free cells of the body's projection of ``og`` (the cells some heading leaves free), computed on the device."""
+    def _free_cells(self, og) -> np.ndarray:
+        """With a body: free cells of its projection of ``og`` (the cells some heading leaves free), computed on the device."""
+        if self.body is None:
+            return super()._free_cells(og)
         og = np.asarray(og)
         if og.ndim != 2:
             raise ValueError("og must be a 2-D occupancy grid")
@@ -135,15 +135,10 @@ class RRTDubins(RRT):
             self._dirty = False
         return self._ctx
 
-    def set_og(self, og_new: np.ndarray):
-        """New occupancy grid; with a body its heading layers and projection are rebuilt."""
-        super().set_og(og_new)
-        if self.body is not None:
-            self.free = self._body_free(og_new)
-
     def sample_all_free(self):
-        """A uniformly random free configuration: cell as RRT.sample_all_free (rrt.py:231-240), then a heading."""
-        cell = self.free[self.rand_gen.choice(self.free.shape[0])]
+        """A uniformly random free configuration: cell as RRT.sample_all_free (rrt.py:231-240, weighted with ``sample_weights``),
+        then a heading."""
+        cell = RRT.sample_all_free(self)
         return np.array([cell[0], cell[1], self.rand_gen.integers(0, self.nheadings)])
 
     def collisionfree(self, og, a, b) -> bool:  # noqa: D102 -- configurations instead of points
@@ -222,8 +217,9 @@ class RRTStarDubins(RRTDubins):
     _STAR = True
 
     def __init__(self, og: np.ndarray, n: int, r_rewire: float, rho: float, nheadings: int = 16, ds: float = 1.0,
-                 costfn: callable = None, pbar: bool = True, seed: int = 0, *, rewire: bool = True, robot_radius=None, body=None):
+                 costfn: callable = None, pbar: bool = True, seed: int = 0, *, rewire: bool = True, robot_radius=None, body=None,
+                 sample_weights=None):
         super().__init__(og, n, rho, nheadings=nheadings, ds=ds, costfn=costfn, pbar=pbar, seed=seed, robot_radius=robot_radius,
-                         body=body)
+                         body=body, sample_weights=sample_weights)
         self.r_rewire = r_rewire
         self.rewire = bool(rewire)

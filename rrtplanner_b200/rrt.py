@@ -25,6 +25,11 @@ section 0):
   object; ``self.free``, the device grid, ``go2goal`` and ``shortcut_path`` use the inflated grid, ``set_og`` inflates again,
   the static ``collisionfree`` is unchanged.  A start or goal inside the inflated obstacles behaves as an occupied one does:
   no growth from the root, or the goal is not found.  ``None`` (default) and radii below 1 (r2 = 0) leave the grid as it is.
+* ``sample_weights`` (keyword-only, not in the reference): a (W, H) uint8 map that biases the free-space samples.  A cell's
+  effective weight is its weight where the planning grid (the configuration-space grid with ``robot_radius``) leaves it free,
+  else 0, and each sample is ``free[searchsorted(cumsum(effective weights), integers(0, T), side="right")]`` with T their sum,
+  drawn from the planner's generator (all weights 1 gives the uniform stream exactly).  ``sample_all_free`` and the plans draw
+  this way; ``set_og`` masks the weights again.  A subclass that overrides ``sample_all_free`` cannot also take weights.
 * points must be integer arrays inside the grid (the reference's Numba kernel rejects float
   points with a TypingError and reads out of bounds for outside points); grids up to
   16384 x 16384, n <= 65534.
@@ -84,20 +89,28 @@ class RRT(object):
 
     _KIND = None
 
-    def __init__(self, og: np.ndarray, n: int, costfn: callable = None, pbar: bool = True, seed: int = 0, *, robot_radius=None):
+    def __init__(self, og: np.ndarray, n: int, costfn: callable = None, pbar: bool = True, seed: int = 0, *, robot_radius=None,
+                 sample_weights=None):
         if costfn is not None:
             raise NotImplementedError(
                 "custom cost functions are Python callables and cannot run on the device; "
                 "rrtplanner_b200 has no CPU fallback (pass costfn=None)")
         self.pbar = pbar
         self.n = n
+        if sample_weights is not None:
+            if self._sampler_overridden():
+                raise TypeError(f"{type(self).__name__} overrides sample_all_free, so sample_weights would be ambiguous: "
+                                "weight the overriding sampler itself, or drop the override")
+            sample_weights = _lib.sample_weights_array(sample_weights, np.shape(og))
+        self.sample_weights = sample_weights
         self.robot_radius = robot_radius
         if robot_radius is not None and np.ndim(robot_radius) != 0:
             raise ValueError("robot_radius must be a number (cells)")
         self._r2 = None if robot_radius is None else int(_lib.disc_r2(robot_radius))
         self._ctx = None
         self._cspace = self._inflate(og)
-        self.free = np.argwhere((og if self._cspace is None else self._cspace) == 0)
+        self.free = self._free_cells(og)
+        self._weigh()
         self.og = og
 
         def costfn(vcosts, points, v, x):
@@ -135,6 +148,27 @@ class RRT(object):
             self._dirty = True
         bits = self._ctx.inflate_disc((og != 0).astype(np.uint8)[None], [0], [self._r2])
         return _lib.unpack_grids_host(bits, *og.shape)[0]
+
+    def _free_cells(self, og) -> np.ndarray:
+        """Free cells of the planning grid of ``og``, row-major (rrt.py:64)."""
+        return np.argwhere((og if self._cspace is None else self._cspace) == 0)
+
+    def _weigh(self):
+        """Cumulative effective weights over ``self.free`` (None without weights).  Cells the grid blocks or that weigh 0 never
+        end a searchsorted step, so the cumulative sum over the free cells picks the same cells as the one over the whole grid."""
+        self._wcum = None
+        if self.sample_weights is None:
+            return
+        cum = np.cumsum(self.sample_weights[self.free[:, 0], self.free[:, 1]].astype(np.int64))
+        if not cum.size or cum[-1] == 0:
+            raise ValueError("sample_weights put no weight on a free cell of the planning grid: nothing to sample")
+        self._wcum = cum
+
+    def _draw_free(self, rng: np.random.Generator, count: int) -> np.ndarray:
+        """``count`` free cells from ``rng`` as the stock sampler draws them: uniform (integers(0, nfree)), or weighted."""
+        if self._wcum is None:
+            return self.free[rng.integers(0, self.free.shape[0], size=count)]
+        return self.free[np.searchsorted(self._wcum, rng.integers(0, int(self._wcum[-1]), size=count), side="right")]
 
     # ---- graph helpers (host, rrt.py:87-129) -----------------------------------------------------
     def route2gv(self, T: nx.DiGraph, gv) -> List[int]:
@@ -215,7 +249,9 @@ class RRT(object):
         return bool(ctx.collision(np.concatenate([a, b])[None])[0])
 
     def sample_all_free(self):
-        """A uniformly random free cell (rrt.py:231-240)."""
+        """A uniformly random free cell (rrt.py:231-240); with ``sample_weights`` a free cell drawn by weight."""
+        if self._wcum is not None:
+            return self.free[np.searchsorted(self._wcum, self.rand_gen.integers(0, int(self._wcum[-1])), side="right")]
         return self.free[self.rand_gen.choice(self.free.shape[0])]
 
     def plan(self, xstart: np.ndarray, xgoal: np.ndarray):
@@ -224,9 +260,12 @@ class RRT(object):
 
     def set_og(self, og_new: np.ndarray):
         """New occupancy grid: refresh free space (rrt.py:261-272) and the device copy."""
+        if self.sample_weights is not None and self.sample_weights.shape != np.shape(og_new):
+            raise ValueError(f"sample_weights has shape {self.sample_weights.shape}, the new grid {np.shape(og_new)}")
         self.og = og_new
         self._cspace = self._inflate(og_new)
-        self.free = np.argwhere((og_new if self._cspace is None else self._cspace) == 0)
+        self.free = self._free_cells(og_new)
+        self._weigh()
         self._dirty = True
 
     def set_n(self, n: int):
@@ -309,8 +348,7 @@ class RRT(object):
         reference's loop does (rrt.py:420,501)."""
         if type(self).sample_all_free is not RRT.sample_all_free and self._sampler_overridden():
             return self._as_samples([np.asarray(self.sample_all_free()) for _ in range(count)])
-        idx = self.rand_gen.integers(0, self.free.shape[0], size=count)
-        return self.free[idx]
+        return self._draw_free(self.rand_gen, count)
 
     def _desc(self, xstart, xgoal, rot=None):
         d = np.zeros(1, dtype=_lib.PLAN_DESC)
@@ -354,8 +392,9 @@ class RRTStandard(RRT):
 
     _KIND = _lib.KIND_STANDARD
 
-    def __init__(self, og: np.ndarray, n: int, costfn: callable = None, pbar=True, seed: int = 0, *, robot_radius=None):
-        super().__init__(og, n, costfn=costfn, pbar=pbar, seed=seed, robot_radius=robot_radius)
+    def __init__(self, og: np.ndarray, n: int, costfn: callable = None, pbar=True, seed: int = 0, *, robot_radius=None,
+                 sample_weights=None):
+        super().__init__(og, n, costfn=costfn, pbar=pbar, seed=seed, robot_radius=robot_radius, sample_weights=sample_weights)
 
     def plan(self, xstart: np.ndarray, xgoal: np.ndarray) -> Tuple[nx.DiGraph, int]:
         self._check_hooks()
@@ -381,8 +420,8 @@ class RRTStar(RRT):
     _KIND = _lib.KIND_STAR
 
     def __init__(self, og: np.ndarray, n: int, r_rewire: float, costfn: callable = None, pbar=True, seed: int = 0, *,
-                 rewire: str = "reference", robot_radius=None):
-        super().__init__(og, n, costfn=costfn, pbar=pbar, seed=seed, robot_radius=robot_radius)
+                 rewire: str = "reference", robot_radius=None, sample_weights=None):
+        super().__init__(og, n, costfn=costfn, pbar=pbar, seed=seed, robot_radius=robot_radius, sample_weights=sample_weights)
         self.r_rewire = r_rewire
         if rewire not in ("reference", "rrtstar"):
             raise ValueError("rewire must be 'reference' or 'rrtstar'")
@@ -408,7 +447,7 @@ class RRTStar(RRT):
 
 
 class RRTStarInformed(RRT):
-    """Informed RRT* (rrt.py:562-758).
+    """Informed RRT* (rrt.py:562-758).  ``sample_weights`` weight the free-space phase only; the ellipse phase is the reference's.
 
     ``rewire`` (keyword-only, not in the reference) as for :class:`RRTStar`: ``"reference"`` keeps the reference's rewire
     block, which never fires; ``"rrtstar"`` runs the loop with the rewire that fires (kernel K8 with the informed sampling
@@ -418,8 +457,8 @@ class RRTStarInformed(RRT):
     _KIND = _lib.KIND_INFORMED
 
     def __init__(self, og: np.ndarray, n: int, r_rewire: float, r_goal: float, costfn: callable = None,
-                 pbar: bool = True, seed: int = 0, *, rewire: str = "reference", robot_radius=None):
-        super().__init__(og, n, costfn=costfn, pbar=pbar, seed=seed, robot_radius=robot_radius)
+                 pbar: bool = True, seed: int = 0, *, rewire: str = "reference", robot_radius=None, sample_weights=None):
+        super().__init__(og, n, costfn=costfn, pbar=pbar, seed=seed, robot_radius=robot_radius, sample_weights=sample_weights)
         self.r_rewire = r_rewire
         self.r_goal = r_goal
         self.ellipses = {}
@@ -532,12 +571,11 @@ class RRTStarInformed(RRT):
                     if 0 <= f < drawn:
                         first = f
         else:
-            nfree = self.free.shape[0]
             probe_gen = copy.deepcopy(self.rand_gen)
-            samples = self.free[probe_gen.integers(0, nfree, size=n)].astype(np.int16)[None]
+            samples = self._draw_free(probe_gen, n).astype(np.int16)[None]
             first = self._launch(ctx, desc, samples)[5]
             # advance the real generator by exactly the free-space draws the reference consumes
-            self.rand_gen.integers(0, nfree, size=n if first < 0 else first + 1)
+            self._draw_free(self.rand_gen, n if first < 0 else first + 1)
         balls = np.zeros((1, n, 2))
         if first >= 0:
             rot = self.rotation_to_world_frame(xstart, xgoal)    # LinAlgError if xstart == xgoal, as the reference
